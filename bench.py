@@ -31,6 +31,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 SEED = 1234
 N_QUAD = 100
@@ -225,6 +226,20 @@ def i8crt_executed_ops(M, rows, chunk=16384):
     return total
 
 
+LEAF_NAMES = ('Z', 'raw_lengthscale', 'raw_outputscale', 'm', 'L_raw', 'log_var_noise', 'theta')
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes out_dir/<name>.npy (float64) for each array, so that two builds can be compared output for output."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def load_json(path):
     try:
         return json.load(open(path))
@@ -350,10 +365,10 @@ def run_ours(args):
                 if x is not None:
                     x.grad = None
             # sync_ell=False: ONE collective per step (the global ELL rides in the packed all-reduce of the backward)
-            ELL, KLD, _, _, _ = Fn.elbo_terms(eng, xb, yb, sc, *leaves, None, check_status=True, sync_ell=False)
-            loss = -(ELL - KLD)
+            terms = Fn.elbo_terms(eng, xb, yb, sc, *leaves, None, check_status=True, sync_ell=False)
+            loss = -(terms[0] - terms[1])
             loss.backward()
-            return loss
+            return loss, terms
         return eng, leaves, step_fn
 
     def dist_parity():
@@ -369,7 +384,7 @@ def run_ours(args):
         got = [None if x is None else x.grad.clone() for x in leaves]
         ell_global = float((sc * eng.last_ell_sum).item())
         with Fn.local_only():
-            loss = step_fn(xg, yg, sc)
+            loss, _ = step_fn(xg, yg, sc)
         errs = [float((a - x.grad).norm() / x.grad.norm()) for a, x in zip(got, leaves) if x is not None]
         kl = float(eng.kl.item())
         errs.append(abs((-(ell_global - kl)) - float(loss.item())) / abs(float(loss.item())))
@@ -379,8 +394,9 @@ def run_ours(args):
                 'what': 'all-reduced ELBO and gradients (Z, lengthscale, outputscale, m, L_S, noise, flow) of a row-sharded '
                         'global minibatch vs one rank evaluating it alone; max L2-relative error over tensors and ranks'}
 
-    def measure(compute, sample_clocks):
-        """W warm-up + K timed ELBO fwd+bwd steps of the device arm in one compute mode."""
+    def measure(compute, sample_clocks, keep_outputs=False):
+        """W warm-up + K timed ELBO fwd+bwd steps of the device arm in one compute mode.  keep_outputs: also return, as
+        float64 host arrays, what the last timed step gave its caller (loss, the elbo_terms outputs, every gradient)."""
         eng, leaves, step_fn = make_step(compute)
         clocks = ClockSampler(local)
         if sample_clocks and rank == 0 and not args.no_clocks:
@@ -415,13 +431,18 @@ def run_ours(args):
         ev0.record()
         for s in range(args.warmup, steps_total):
             flush.fill_(s & 0xFF)                       # L2 flush between timed iterations
-            loss = step_fn(*dev_batch(s))
+            loss, terms = step_fn(*dev_batch(s))
         ev1.record()
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         ms = ev0.elapsed_time(ev1)
+        outputs = None
+        if keep_outputs:
+            outputs = dict(zip(('loss', 'ell', 'kld', 'ell_rows', 'mu', 'v'), (loss,) + tuple(terms)))
+            outputs.update(('grad_' + n, x.grad) for n, x in zip(LEAF_NAMES, leaves) if x is not None)
+            outputs = {k: t.detach().double().cpu().numpy() for k, t in outputs.items()}
         gemm_ms, gemm_n = (C.c_double * 3)(), (C.c_long * 3)()
         lib.tgp_gemm_timing(0, gemm_ms, gemm_n)
         launches = lib.tgp_launch_count() - launches0
@@ -456,7 +477,7 @@ def run_ours(args):
             tn = torch.tensor([e0.elapsed_time(e1), e1.elapsed_time(e2)], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(tn, op=dist.ReduceOp.MAX)
-        return dict(ms_total=ms, value=global_batch * args.steps / (ms * 1e-3), loss=loss_global,
+        return dict(ms_total=ms, value=global_batch * args.steps / (ms * 1e-3), loss=loss_global, outputs=outputs,
                     gemm_ms=list(gemm_ms), gemm_n=list(gemm_n), launches=int(launches), clocks=clk,
                     test_nll_rows_per_s=global_batch * args.steps / (float(tn[0].item()) * 1e-3),
                     test_nll_cached_rows_per_s=global_batch * args.steps / (float(tn[1].item()) * 1e-3))
@@ -468,7 +489,7 @@ def run_ours(args):
     other = None
     if not args.no_other_mode:
         measure(second, False)                      # discarded: absorbs the cold start of a fresh box
-    head = measure(args.compute, True)
+    head = measure(args.compute, True, keep_outputs=bool(args.dump_outputs))
     if not args.no_other_mode:
         other = measure(second, False)
     ms_total, value, final_loss, launches, clk = head['ms_total'], head['value'], head['loss'], head['launches'], head['clocks']
@@ -481,6 +502,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, head['outputs'])
     # ---- roofline of the dominant kernel -----------------------------------------------------------------------------
     peaks = load_json(os.path.join(ROOT, 'MEASURED_PEAKS.json'))
     extra = load_json(os.path.join(ROOT, 'profiles', 'r02_measured_peaks_extra.json'))     # scripts/measure_peaks.py on this pool
@@ -673,7 +696,13 @@ def main():
     ap.add_argument('--no-gemm-timing', action='store_true', help='(diagnostic) do not instrument GEMM launches with events')
     ap.add_argument('--no-clocks', action='store_true', help='(diagnostic) do not sample nvidia-smi during the timed region')
     ap.add_argument('--no-overlap', action='store_true', help='(diagnostic) K_xz generation on the main stream (TGP_OPT_OVERLAP_KGEN = 0)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step of the headline mode returned (loss, ELL, KLD, per-row ell, mu, v '
+                         'and every gradient) as DIR/<name>.npy, float64; inputs are seeded, so runs with the same '
+                         'arguments can be compared')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -1,11 +1,12 @@
 """Generate `tests/golden/*.npz` by running the UNMODIFIED reference under `oracle/ref_shims` (O1).
 
-Run in the build container only (`python oracle/make_golden.py`); `/root/reference` does not exist on the GPU box.
+Run where the original project is checked out (`TGP_REFERENCE_ROOT=<checkout> python oracle/make_golden.py`).
 Each fixture stores the inputs, every parameter, a JSON description of the flow, and the reference's outputs:
 ELBO / ELL / KLD, q(f) marginals, every gradient of ELBO, test log-likelihood and predictive moments.
 `tests/test_oracle_golden.py` replays them through `oracle/tgp_oracle.py` (O2); `tests/test_gpu_parity.py`
 replays them through the CUDA path.
 """
+import hashlib
 import json
 import os
 import sys
@@ -15,7 +16,8 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
-from oracle.ref_loader import load_reference  # noqa: E402
+from oracle.ref_loader import REFERENCE_ROOT, load_reference  # noqa: E402
+from tests.golden_util import variational_grid  # noqa: E402
 
 dsp = load_reference()
 import dsp.config as cg  # noqa: E402
@@ -27,7 +29,7 @@ from dsp.flows import (SAL, StepTanhL, ArcSL, BoxCoxL, InverseBoxCoxL, build_cha
                        StepSAL, StepArcSL, StepBoxCoxL, StepInverseBoxCoxL, StepAllL)
 
 OUT = os.path.join(os.path.dirname(HERE), 'tests', 'golden')
-UCI = os.path.join(os.environ.get('TGP_REFERENCE_ROOT', '/root/reference'), 'code', 'datasets', 'regression', 'uci')
+UCI = os.path.join(REFERENCE_ROOT or '', 'code', 'datasets', 'regression', 'uci')
 
 
 def load_uci(name, seed=1):
@@ -94,13 +96,12 @@ def randomise(model, seed, nnet_scale=0.2):
 def randomise_big(model, seed):
     """P1 state for the BASELINE-size fixtures.  Same distributions as `randomise`, except that the M x M variational
     factor is drawn from a 17-level grid (0.5 I + 0.05 * k/8, k in -8..8, strictly lower part only; the upper triangle,
-    which the reference masks away at use, is zero) so that the stored parameter compresses to < 1 byte per entry."""
+    which the reference masks away at use, is zero); the fixture stores the grid's seed instead of the M x M parameter.
+    Returns that seed."""
     randomise(model, seed)
-    g = torch.Generator().manual_seed(seed + 1000)
-    M = model.M
     with torch.no_grad():
-        q = torch.randint(-8, 9, (1, M, M), generator=g).double() / 8.0
-        model.q_U.chol_variational_covar.copy_((0.5 * torch.eye(M).unsqueeze(0) + 0.05 * q).tril())
+        model.q_U.chol_variational_covar.copy_(torch.from_numpy(variational_grid(model.M, seed + 1000)))
+    return seed + 1000
 
 
 def flow_to_spec(flow, store, X=None, prefix='fl'):
@@ -211,10 +212,11 @@ def projection_basis(M, k=6):
     return (((i * 2654435761 + (c + 1) * 40503 + i * c * 97) % 1024).astype(np.float64) / 1024.0) - 0.5
 
 
-def record(name, model, X, Y, Xte, Yte, y_std, likelihood, id_flow=False, extra=None, big=False, tape=None):
+def record(name, model, X, Y, Xte, Yte, y_std, likelihood, id_flow=False, extra=None, big=False, tape=None, grid_seed=None):
     """big=True (fixtures at the BASELINE sizes M = 1024 / 2048): the M x M gradient of chol_variational_covar is stored
     as checksums — G R, G^T R for the fixed basis R above, its diagonal and Frobenius norm — instead of 8-32 MB of
-    incompressible doubles (the parameter itself is low-entropy by construction, see randomise_big)."""
+    incompressible doubles, and the parameter itself as the seed `grid_seed` of randomise_big plus its SHA-256
+    (tests/golden_util regenerates it)."""
     if ONLY and name not in ONLY:
         return
     store = {}
@@ -228,7 +230,13 @@ def record(name, model, X, Y, Xte, Yte, y_std, likelihood, id_flow=False, extra=
     store['ELBO'], store['ELL'], store['KLD'] = E.item(), ELL.item(), KLD.item()
     names = []
     for n, prm in model.named_parameters():
-        store['param:' + n] = prm.detach().numpy().copy()
+        if big and n.endswith('chol_variational_covar'):
+            p = prm.detach().numpy()
+            assert np.array_equal(p, variational_grid(p.shape[1], grid_seed))
+            store['paramgrid:' + n] = np.array([grid_seed, p.shape[1]], dtype=np.int64)
+            store['paramsha256:' + n] = np.array(hashlib.sha256(np.ascontiguousarray(p).tobytes()).hexdigest())
+        else:
+            store['param:' + n] = prm.detach().numpy().copy()
         gr = (torch.zeros_like(prm) if prm.grad is None else prm.grad).numpy().copy()
         if big and n.endswith('chol_variational_covar'):
             G = gr[0]
@@ -513,13 +521,15 @@ def main_big():
     SAL(1)); row counts the CPU oracle replays in seconds.  Z = distinct data rows, as in bench.py."""
     Xs, Ys = synthetic_regression(2048 + 256, 8, 1234)
     m = build('TGP', Xs, 1024, 5.0e6, StepTanhL(1, 3, add_f0=True), seed=40)
-    randomise_big(m, 41)
-    record('synth_reg_d8_m1024_p1', m, Xs[:2048], Ys[:2048], Xs[2048:], Ys[2048:], 1.3, 'gauss_nonlinear', big=True)
+    s = randomise_big(m, 41)
+    record('synth_reg_d8_m1024_p1', m, Xs[:2048], Ys[:2048], Xs[2048:], Ys[2048:], 1.3, 'gauss_nonlinear', big=True,
+           grid_seed=s)
     Xc, Yc = synthetic_classification(4096, 16, 4321)
     cg.quad_points = 100
     m = build('TGP', Xc, 2048, 1.0e6, SAL(1), likelihood=Bernoulli(), seed=42)
-    randomise_big(m, 43)
-    record('synth_clf_d16_m2048_p1', m, Xc[:1024], Yc[:1024], Xc[1024:1152], Yc[1024:1152], 1.0, 'bernoulli', big=True)
+    s = randomise_big(m, 43)
+    record('synth_clf_d16_m2048_p1', m, Xc[:1024], Yc[:1024], Xc[1024:1152], Yc[1024:1152], 1.0, 'bernoulli', big=True,
+           grid_seed=s)
 
 
 if __name__ == '__main__':

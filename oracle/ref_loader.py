@@ -1,8 +1,8 @@
-"""Import the UNMODIFIED reference (`/root/reference/code/dsp`) under `oracle/ref_shims` ("O1").
+"""Import the UNMODIFIED reference (`$TGP_REFERENCE_ROOT/code/dsp`) under `oracle/ref_shims` ("O1").
 
-TEST INFRASTRUCTURE ONLY.  Works only where `/root/reference` exists (the build container); it is used by
-`oracle/make_golden.py` to generate `tests/golden/*.npz` and by the `needs_reference` CPU tests.  Never
-imported by the product, the GPU tests, `smoke()` or `bench.py`.
+TEST INFRASTRUCTURE ONLY.  Works only where TGP_REFERENCE_ROOT names a checkout of the original TGP.pytorch project,
+which this repository does not contain; it is used by `oracle/make_golden.py` to generate `tests/golden/*.npz` and by
+the `needs_reference` CPU tests.  Never imported by the product, the GPU tests, `smoke()` or `bench.py`.
 
 What is patched, and nothing else (SURVEY.md §8c):
   * `sys.path`: shims first, then the reference's `code/` directory;
@@ -13,18 +13,19 @@ import os
 import sys
 import warnings
 
-REFERENCE_ROOT = os.environ.get('TGP_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('TGP_REFERENCE_ROOT')
 _SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'ref_shims')
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, 'code', 'dsp'))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, 'code', 'dsp'))
 
 
 def load_reference():
     """Returns the reference's `dsp` package (module object), CPU device, FP64 + 100 quadrature points."""
     if not reference_available():
-        raise RuntimeError('reference tree not found at %s' % REFERENCE_ROOT)
+        raise RuntimeError('reference tree not found: set TGP_REFERENCE_ROOT to a checkout of the original TGP.pytorch '
+                           '(got %r)' % REFERENCE_ROOT)
     warnings.filterwarnings('ignore')
     for p in (os.path.join(REFERENCE_ROOT, 'code'), _SHIMS):
         if p in sys.path:

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run with -m gpu on the B200 box)')
-    config.addinivalue_line('markers', 'needs_reference: needs /root/reference (build container only)')
+    config.addinivalue_line('markers', 'needs_reference: needs a checkout of the original TGP.pytorch named by TGP_REFERENCE_ROOT')
 
 
 def pytest_collection_modifyitems(config, items):
@@ -22,7 +22,7 @@ def pytest_collection_modifyitems(config, items):
         if 'gpu' in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason='no CUDA device'))
         if 'needs_reference' in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason='/root/reference not present'))
+            item.add_marker(pytest.mark.skip(reason='TGP_REFERENCE_ROOT does not name a TGP.pytorch checkout'))
 
 
 # ---- measured residuals -----------------------------------------------------------------------------------------

@@ -1,5 +1,6 @@
 """Load `tests/golden/*.npz` (written by oracle/make_golden.py) into oracle-style parameter dicts."""
 import glob
+import hashlib
 import json
 import os
 
@@ -61,10 +62,43 @@ def flow_grad_keys(spec, constrained=False):
     return keys
 
 
+def variational_grid(M, seed):
+    """(1, M, M) variational factor of the BASELINE-size fixtures (oracle/make_golden.randomise_big): 0.5 I + 0.05 k / 8 on
+    the lower triangle, k drawn uniformly from -8..8 by a torch CPU generator seeded with `seed`."""
+    g = torch.Generator().manual_seed(int(seed))
+    q = torch.randint(-8, 9, (1, M, M), generator=g).double() / 8.0
+    return (0.5 * torch.eye(M, dtype=torch.float64).unsqueeze(0) + 0.05 * q).tril().numpy()
+
+
+class _Arrays(dict):
+    """The arrays of one fixture; `.files` lists the keys, as on the NpzFile they were read from."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
+def _load_fixture(path):
+    """Reads a fixture; a parameter stored as `paramgrid:<name>` = (seed, M) is regenerated with `variational_grid` and
+    checked against the SHA-256 of the parameter the reference was run with (`paramsha256:<name>`)."""
+    with np.load(path, allow_pickle=False) as z:
+        arrays = _Arrays((k, z[k]) for k in z.files)
+    for key in [k for k in arrays if k.startswith('paramgrid:')]:
+        name = key[len('paramgrid:'):]
+        seed, M = (int(x) for x in arrays.pop(key))
+        a = variational_grid(M, seed)
+        want = str(arrays.pop('paramsha256:' + name))
+        if hashlib.sha256(a.tobytes()).hexdigest() != want:
+            raise RuntimeError('%s: %s regenerated from seed %d differs from the stored SHA-256 (torch CPU generator changed?)'
+                               % (os.path.basename(path), name, seed))
+        arrays['param:' + name] = a
+    return arrays
+
+
 class Golden:
     def __init__(self, name):
         self.name = name
-        self.z = np.load(os.path.join(GOLDEN_DIR, name + '.npz'), allow_pickle=False)
+        self.z = _load_fixture(os.path.join(GOLDEN_DIR, name + '.npz'))
         self.meta = json.loads(str(self.z['meta']))
 
     def t(self, key, dtype=torch.float64):

@@ -1,4 +1,4 @@
-"""Drop-in checks against the UNMODIFIED reference (build container only: needs /root/reference).
+"""Drop-in checks against the UNMODIFIED reference (needs TGP_REFERENCE_ROOT = a checkout of the original TGP.pytorch).
 
 1. Every name the reference's main.py / exp_utils.py import from the hot-path modules (main.py:26-37, exp_utils.py:7-8) exists
    in tgp.pytorch_b200.dsp with the same call signature; so do the methods the reference's trainer calls on the model.
