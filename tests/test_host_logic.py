@@ -202,6 +202,35 @@ def test_library_options_and_workspace_sizing_without_a_gpu():
         assert lib.tgp_set_option(_lib.OPT_ROW_CHUNK, 32768) == 0
 
 
+def test_workspace_sizes_follow_the_compute_mode_without_a_gpu():
+    """The step workspace holds the FP64 region plus the planes of the active mode only, so the FP64 mode's is the smallest
+    and each tensor-core mode adds an amount that depends on M alone; batch sizes grow with R across the row-chunk edges
+    (16384 rows for the tensor-core modes, 32768 for FP64); the single-call workspace holds all the regions."""
+    from tgp.pytorch_b200 import _lib
+    lib = _lib.load()
+    modes = (_lib.TGP_F64, _lib.TGP_F32, _lib.TGP_F64_I8)
+    m = _lib.TgpModel()
+    m.likelihood, m.n_quad = 1, 30
+    for M in (1, 100, 1024, 2048):
+        extra = set()
+        for D in (1, 8, 33):
+            m.M, m.D = M, D
+            step = {}
+            for dt in modes:
+                m.dtype = dt
+                step[dt] = lib.tgp_step_workspace_bytes(m)
+                batch = [lib.tgp_batch_workspace_bytes(m, R) for R in (1, 16383, 16384, 16385, 32768, 32769, 100000)]
+                assert batch[0] > 0 and batch == sorted(batch), (M, D, dt, batch)
+                lay = _lib.TgpReduceLayout()
+                assert lib.tgp_reduce_layout(m, lay) == 0
+                for R in (1, 4096):
+                    need = step[dt] + lib.tgp_batch_workspace_bytes(m, R) + 8 * (lay.total + lay.packed_total)
+                    assert lib.tgp_workspace_bytes(m, R) >= need, (M, D, dt, R)
+            assert 0 < step[_lib.TGP_F64] < step[_lib.TGP_F32] and step[_lib.TGP_F64] < step[_lib.TGP_F64_I8], (M, D, step)
+            extra.add((step[_lib.TGP_F32] - step[_lib.TGP_F64], step[_lib.TGP_F64_I8] - step[_lib.TGP_F64]))
+        assert len(extra) == 1, (M, extra)
+
+
 def test_split_csv_reader_standardises_like_the_reference(tmp_path):
     """data.load_split_csv: the airline-style on-disk format (header-less CSV + splits_idx pickle,
     regression_datasets.py:95-192) with the training-statistics standardisation of data.py:260-299."""

@@ -93,6 +93,22 @@ __device__ __forceinline__ T warp_max(T v) {
 
 __host__ __device__ inline long cdiv(long a, long b) { return (a + b - 1) / b; }
 
+// Carves typed views out of a caller-owned workspace in declaration order, each starting on a 256-byte ABSOLUTE address
+// (callers of the staged entry points may pass any alignment; cp.async, vector loads and TMA need 16 bytes).  With a NULL
+// base it only measures: `used` starts at 256, so bytes() covers a carve of the same pieces from a base of any alignment.
+// Every workspace size the library reports is bytes() of the layout function that the entry points carve with.
+struct Carve {
+    char* base;
+    size_t used;
+    explicit Carve(void* b) : base(static_cast<char*>(b)), used(b ? 0 : 256) {}
+    template <class T> T* take(size_t n) {
+        const uintptr_t b = reinterpret_cast<uintptr_t>(base), at = (b + used + 255) & ~uintptr_t(255);
+        used = at - b + n * sizeof(T);
+        return reinterpret_cast<T*>(at);
+    }
+    size_t bytes() const { return used; }
+};
+
 // cudaFuncSetAttribute is per DEVICE: one-time kernel configuration is tracked per (site, device), so that a second GPU
 // used from the same process gets its own opt-in to large dynamic shared memory.
 struct PerDeviceOnce {

@@ -39,26 +39,19 @@ struct StepPlanes {               // per step: residues of W = [Linv; C] (2M x M
     uint8_t *Wc;                   // planes [T][2M][ldk] of W~ = diag(2^c) W, per-column scale: backward-data operand, rebuilt per row
                                   // chunk (c = column exponents of that chunk's [Abar | Bbar]); reduction over its ROWS: the tensor
                                   // core reads it MN-major, no transposed copy
-    int *w_row_exp, *w_col_exp, *k_exp;
+    int *w_row_exp, *k_exp;
     long ldk;
 };
 
-inline size_t step_bytes(int M) {
-    const long ldk = pad16(M);
-    return (size_t)2 * M * M * sizeof(double) + (size_t)2 * T_ALL * 2L * M * ldk + (size_t)(3L * M + 64) * sizeof(int) + 1024;
-}
-
-inline StepPlanes carve_step(void* region, int M) {
+// the residue region of the step workspace, carved after its FP64 region
+inline StepPlanes step_planes(Carve& c, int M) {
     StepPlanes s;
     s.ldk = pad16(M);
-    char* p = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(region) + 255) & ~uintptr_t(255));
-    s.Wst = reinterpret_cast<double*>(p); p += (size_t)2 * M * M * sizeof(double);
-    s.W = reinterpret_cast<uint8_t*>(p); p += (size_t)T_ALL * 2L * M * s.ldk;
-    s.Wc = reinterpret_cast<uint8_t*>(p); p += (size_t)T_ALL * 2L * M * s.ldk;
-    p = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(p) + 15) & ~uintptr_t(15));
-    s.w_row_exp = reinterpret_cast<int*>(p); p += (size_t)2 * M * sizeof(int);
-    s.w_col_exp = reinterpret_cast<int*>(p); p += (size_t)M * sizeof(int);
-    s.k_exp = reinterpret_cast<int*>(p);
+    s.Wst = c.take<double>(2L * M * M);
+    s.W = c.take<uint8_t>(T_ALL * 2L * M * s.ldk);
+    s.Wc = c.take<uint8_t>(T_ALL * 2L * M * s.ldk);
+    s.w_row_exp = c.take<int>(2L * M);
+    s.k_exp = c.take<int>(1);
     return s;
 }
 
@@ -80,32 +73,20 @@ struct BatchView {
 // D <= 32: K_xz is generated straight into residue planes (i8::k_rbf_residues) and recomputed by the backward
 inline bool keeps_kxz(int D) { return D > 32; }
 
-inline size_t batch_bytes(int M, int D, long R) {
-    const long Rc = chunk_rows(R), ldk = pad16(M), ld2m = pad16(2L * M);
-    size_t b = 0;
-    b += (size_t)R * 2 * M * 8 + (keeps_kxz(D) ? (size_t)R * M * 8 : 0) + (size_t)Rc * M * 8;
-    b += (size_t)T_ALL * R * ldk;
-    b += (size_t)2 * T_ALL * Rc * ld2m + (size_t)T_ALL * Rc * ldk + (size_t)T_ALL * 2 * M * ldk;
-    b += (size_t)(3L * M + 64) * sizeof(int) + 4096;
-    return b;
-}
-
-inline BatchView carve_batch(void* ws, int M, int D, long R) {
+inline BatchView batch_view(Carve& c, int M, int D, long R) {
     BatchView b;
     b.Rc = chunk_rows(R); b.ldk = pad16(M); b.ld2m = pad16(2L * M);
-    char* p = reinterpret_cast<char*>(ws);
-    auto take = [&](size_t n) { char* q = p; p += (n + 255) / 256 * 256; return q; };
-    b.AB = reinterpret_cast<double*>(take((size_t)R * 2 * M * 8));
-    b.Kbuf = keeps_kxz(D) ? reinterpret_cast<double*>(take((size_t)R * M * 8)) : nullptr;
-    b.Kbar = reinterpret_cast<double*>(take((size_t)b.Rc * M * 8));
-    b.Kp = reinterpret_cast<uint8_t*>(take((size_t)T_ALL * R * b.ldk));
-    b.Op = reinterpret_cast<uint8_t*>(take((size_t)T_ALL * b.Rc * b.ld2m));
-    b.Pc = reinterpret_cast<uint8_t*>(take((size_t)T_ALL * b.Rc * b.ld2m));
-    b.Kbp = reinterpret_cast<uint8_t*>(take((size_t)T_ALL * b.Rc * b.ldk));
-    b.Gp = reinterpret_cast<uint8_t*>(take((size_t)T_ALL * 2 * M * b.ldk));
-    b.col_exp = reinterpret_cast<int*>(take((size_t)2 * M * sizeof(int)));
-    b.wc_exp = reinterpret_cast<int*>(take((size_t)M * sizeof(int)));
-    b.zero_exp = reinterpret_cast<int*>(take(sizeof(int)));
+    b.AB = c.take<double>(R * 2 * M);
+    b.Kbuf = keeps_kxz(D) ? c.take<double>(R * M) : nullptr;
+    b.Kbar = c.take<double>(b.Rc * M);
+    b.Kp = c.take<uint8_t>(T_ALL * R * b.ldk);
+    b.Op = c.take<uint8_t>(T_ALL * b.Rc * b.ld2m);
+    b.Pc = c.take<uint8_t>(T_ALL * b.Rc * b.ld2m);
+    b.Kbp = c.take<uint8_t>(T_ALL * b.Rc * b.ldk);
+    b.Gp = c.take<uint8_t>(T_ALL * 2 * M * b.ldk);
+    b.col_exp = c.take<int>(2L * M);
+    b.wc_exp = c.take<int>(M);
+    b.zero_exp = c.take<int>(1);
     return b;
 }
 
@@ -178,9 +159,8 @@ inline int rbf_residues(const double* X, const double* Zs, const double* ls, con
 }
 
 // per step, after run_prepare: residues of W scaled per row (forward operand; the backward-data operand is built per chunk)
-inline int make_step_planes(const StepView& v, void* region, cudaStream_t st) {
+inline int make_step_planes(const StepView& v, const StepPlanes& s, cudaStream_t st) {
     const int M = v.M;
-    StepPlanes s = carve_step(region, M);
     k_stack_w<<<2 * M, 256, 0, st>>>(v.Linv, v.Cm, v.Mp, M, s.Wst);
     TGP_TRY(check_launch("k_stack_w"));
     k_exp_of_scalar<<<1, 1, 0, st>>>(v.os, s.k_exp);
@@ -299,11 +279,9 @@ __global__ void __launch_bounds__(256) k_wt_residues(const double* __restrict__ 
     i8::emit_residues_rt(tab.T, xi, tab, r, rows, c, M, planes, ldp, plane_stride);
 }
 
-inline int qf_forward(const StepView& s, void* step_region, void* batch_ws, const double* X, long R, double* mu, double* v,
+inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, double* mu, double* v,
                       cudaStream_t st) {
     const int M = s.M, D = s.D;
-    StepPlanes sp = carve_step(step_region, M);
-    BatchView b = carve_batch(batch_ws, M, D, R);
     const int Tf = fwd_T(M), bits = fwd_bits_w(M);
     // K_xz (FP64 values + residue planes) of all rows in one launch.  It depends on Zs / ls / os only, not on the factorisation:
     // it is enqueued BEFORE the join with the factorisation, which may still be running on the library's high-priority stream
@@ -332,13 +310,10 @@ inline int qf_forward(const StepView& s, void* step_region, void* batch_ws, cons
     return 0;
 }
 
-inline int qf_backward(const StepView& s, void* step_region, void* batch_ws, const double* X, long R, const double* g_mu,
+inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
                        const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
                        cudaStream_t st) {
     const int M = s.M, D = s.D;
-    StepPlanes sp = carve_step(step_region, M);
-    BatchView b = carve_batch(batch_ws, M, D, R);
-    if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     TGP_TRY(fill_int(b.zero_exp, 1, 0, st));
     const double* const kval = b.Kbuf;            // NULL for D <= 32: k_kernel_grads recomputes the K_xz tile (same arithmetic)
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
@@ -396,47 +371,49 @@ inline int qf_backward(const StepView& s, void* step_region, void* batch_ws, con
 }
 
 // ---- test hook: C = A B^T through the residue pipeline ------------------------------------------------------------------
-// mn_major bit 0 / 1: A / B is passed TRANSPOSED ((K x Mr) / (K x N), row-major) and contracted over its rows
-inline size_t debug_bytes(long Mr, long N, long K, int T) {
+// mn_major bit 0 / 1: A / B is passed TRANSPOSED ((K x Mr) / (K x N), row-major) and contracted over its rows.  The scratch
+// holds the operand planes of either orientation: its size does not depend on mn_major.
+struct DebugScratch { uint8_t *Ap, *Bp, *Cp; int *ea, *eb; };
+inline DebugScratch debug_scratch(Carve& c, long Mr, long N, long K, int T) {
     const long ldk = pad16(K), ldn = pad16(N), ldm = pad16(Mr);
-    return (size_t)T * ((Mr > K ? Mr : K) * (ldk > ldm ? ldk : ldm) + (N > K ? N : K) * (ldk > ldn ? ldk : ldn) + Mr * ldn) +
-           (size_t)(Mr + N + 64) * sizeof(int) + 8192;
+    DebugScratch d;
+    d.Ap = c.take<uint8_t>((size_t)T * (K * ldm > Mr * ldk ? K * ldm : Mr * ldk));
+    d.Bp = c.take<uint8_t>((size_t)T * (K * ldn > N * ldk ? K * ldn : N * ldk));
+    d.Cp = c.take<uint8_t>((size_t)T * Mr * ldn);
+    d.ea = c.take<int>(Mr);
+    d.eb = c.take<int>(N);
+    return d;
 }
 
 inline int debug_matmul(long Mr, long N, long K, const double* A, long lda, const double* B, long ldb, double* C, long ldc, int T,
                         int tri_mode, int tri_rows, int lower_rows, int accumulate, int mn_major, void* scratch, cudaStream_t st) {
     const long ldk = pad16(K), ldn = pad16(N), ldm = pad16(Mr);
     const bool at = mn_major & 1, bt = mn_major & 2;
-    char* p = reinterpret_cast<char*>(scratch);
-    auto take = [&](size_t n) { char* q = p; p += (n + 255) / 256 * 256; return q; };
-    uint8_t* Ap = reinterpret_cast<uint8_t*>(take((size_t)T * (at ? K * ldm : Mr * ldk)));
-    uint8_t* Bp = reinterpret_cast<uint8_t*>(take((size_t)T * (bt ? K * ldn : N * ldk)));
-    uint8_t* Cp = reinterpret_cast<uint8_t*>(take((size_t)T * Mr * ldn));
-    int* ea = reinterpret_cast<int*>(take((size_t)Mr * sizeof(int)));
-    int* eb = reinterpret_cast<int*>(take((size_t)N * sizeof(int)));
+    Carve c(scratch);
+    const DebugScratch d = debug_scratch(c, Mr, N, K, T);
     const int bits = i8::crt_bits(T, K);
     if (at) {
-        TGP_TRY(exponents(A, lda, K, (int)Mr, nullptr, ea, st));
-        TGP_TRY(to_residues(A, lda, K, (int)Mr, 1, ea, bits, T, Ap, ldm, K * ldm, st));
+        TGP_TRY(exponents(A, lda, K, (int)Mr, nullptr, d.ea, st));
+        TGP_TRY(to_residues(A, lda, K, (int)Mr, 1, d.ea, bits, T, d.Ap, ldm, K * ldm, st));
     } else {
-        TGP_TRY(exponents(A, lda, Mr, (int)K, ea, nullptr, st));
-        TGP_TRY(to_residues(A, lda, Mr, (int)K, 0, ea, bits, T, Ap, ldk, Mr * ldk, st));
+        TGP_TRY(exponents(A, lda, Mr, (int)K, d.ea, nullptr, st));
+        TGP_TRY(to_residues(A, lda, Mr, (int)K, 0, d.ea, bits, T, d.Ap, ldk, Mr * ldk, st));
     }
     if (bt) {
-        TGP_TRY(exponents(B, ldb, K, (int)N, nullptr, eb, st));
-        TGP_TRY(to_residues(B, ldb, K, (int)N, 1, eb, bits, T, Bp, ldn, K * ldn, st));
+        TGP_TRY(exponents(B, ldb, K, (int)N, nullptr, d.eb, st));
+        TGP_TRY(to_residues(B, ldb, K, (int)N, 1, d.eb, bits, T, d.Bp, ldn, K * ldn, st));
     } else {
-        TGP_TRY(exponents(B, ldb, N, (int)K, eb, nullptr, st));
-        TGP_TRY(to_residues(B, ldb, N, (int)K, 0, eb, bits, T, Bp, ldk, N * ldk, st));
+        TGP_TRY(exponents(B, ldb, N, (int)K, d.eb, nullptr, st));
+        TGP_TRY(to_residues(B, ldb, N, (int)K, 0, d.eb, bits, T, d.Bp, ldk, N * ldk, st));
     }
     i8::Params q{};
     q.Mrows = (int)Mr; q.Ncols = (int)N; q.K = (int)K; q.T = T; q.tri_mode = tri_mode; q.tri_rows = tri_rows; q.lower_rows = lower_rows;
     q.mn_major = mn_major;
-    q.C = Cp; q.ldc = ldn; q.plane_stride_c = Mr * ldn;
-    const Planes PA = at ? Planes{Ap, K, Mr, ldm, K * ldm} : Planes{Ap, Mr, K, ldk, Mr * ldk};
-    const Planes PB = bt ? Planes{Bp, K, N, ldn, K * ldn} : Planes{Bp, N, K, ldk, N * ldk};
+    q.C = d.Cp; q.ldc = ldn; q.plane_stride_c = Mr * ldn;
+    const Planes PA = at ? Planes{d.Ap, K, Mr, ldm, K * ldm} : Planes{d.Ap, Mr, K, ldk, Mr * ldk};
+    const Planes PB = bt ? Planes{d.Bp, K, N, ldn, K * ldn} : Planes{d.Bp, N, K, ldk, N * ldk};
     TGP_TRY(i8::gemm_i8_mod(PA, PB, q, st));
-    return combine(Cp, ldn, Mr * ldn, Mr, (int)N, T, 2 * bits, ea, 0, eb, 1, C, ldc, accumulate, lower_rows, st);
+    return combine(d.Cp, ldn, Mr * ldn, Mr, (int)N, T, 2 * bits, d.ea, 0, d.eb, 1, C, ldc, accumulate, lower_rows, st);
 }
 
 }  // namespace crt

@@ -14,6 +14,11 @@ constexpr int MAX_THETA = 288;     // global flow scalars (largest shipped archi
 constexpr int MAX_ROWP = 16;       // per-row (input-dependent) flow parameters
 constexpr int ROW_THREADS = 128;   // 4 warps = 4 rows per CTA pass
 
+inline int row_grid(long R) {
+    const long blocks = cdiv(R, ROW_THREADS / 32);
+    return (int)(blocks < 148 * 16 ? blocks : 148 * 16);
+}
+
 // log(2*pi) with the reference's float32-rounded pi (code/dsp/config.py:71, utils.py:180) and exact 1/sqrt(pi)
 __device__ constexpr double LOG_2PI_F32PI = 1.8378770942368803;
 __device__ constexpr double INV_SQRT_PI = 0.5641895835477563;

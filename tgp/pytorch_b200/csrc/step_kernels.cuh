@@ -289,25 +289,21 @@ inline int pad_M(int M) {
     return mp;
 }
 
-inline size_t step_ws_doubles(int M, int D) {
-    const size_t Mp = pad_M(M);
-    return 64 + (size_t)((D + 7) / 8 * 8) + 8 + (size_t)M * D + 8 + 8 + (size_t)M + 8 +
-           (size_t)POTRF_NB * POTRF_NB + 9 * Mp * Mp;
-}
-
-inline StepView carve_step(void* ws, int M, int D) {
+// The FP64 region of the step workspace.  The Mp x Mp matrices are multiples of 256 bytes, so they are contiguous:
+// run_prepare zeroes L and Linv with one memset, and the region ends on a 256-byte boundary.
+inline StepView step_view(Carve& c, int M, int D) {
     StepView v;
     v.M = M; v.D = D; v.Mp = pad_M(M);
-    double* p = reinterpret_cast<double*>(ws);
     const size_t mm = (size_t)v.Mp * v.Mp;
-    v.ls = p; p += (D + 7) / 8 * 8;
-    v.os = p; p += 8;
-    v.kl3 = p; p += 8;
-    v.Zs = p; p += ((size_t)M * D + 7) / 8 * 8;
-    v.mvec = p; p += ((size_t)M + 7) / 8 * 8;
-    v.Dinv = p; p += POTRF_NB * POTRF_NB;
-    v.Kzz = p; p += mm; v.L = p; p += mm; v.Linv = p; p += mm; v.LS = p; p += mm; v.Cm = p; p += mm;
-    v.S0 = p; p += mm; v.S1 = p; p += mm; v.S2 = p; p += mm; v.S3 = p; p += mm;
+    v.ls = c.take<double>(D);
+    v.os = c.take<double>(1);
+    v.kl3 = c.take<double>(8);
+    v.Zs = c.take<double>((size_t)M * D);
+    v.mvec = c.take<double>(M);
+    v.Dinv = c.take<double>(POTRF_NB * POTRF_NB);
+    v.Kzz = c.take<double>(mm); v.L = c.take<double>(mm); v.Linv = c.take<double>(mm); v.LS = c.take<double>(mm);
+    v.Cm = c.take<double>(mm);
+    v.S0 = c.take<double>(mm); v.S1 = c.take<double>(mm); v.S2 = c.take<double>(mm); v.S3 = c.take<double>(mm);
     return v;
 }
 

@@ -24,46 +24,32 @@ struct BatchPlanes {
 
 inline long chunk_rows(long R) { return R < TC_ROW_CHUNK ? R : TC_ROW_CHUNK; }
 
-inline size_t step_plane_floats(int M) {
-    const long ldk = pad4(M), ld2m = pad4(2L * M);
-    return (size_t)(2 * (2L * M * ldk) + 2 * ((long)M * ld2m) + 2L * M + 64);
-}
-
-inline StepPlanes carve_step_planes(void* step_ws, int M, int D) {
-    // the planes follow the FP64 region of the step workspace
-    float* p = reinterpret_cast<float*>(reinterpret_cast<double*>(step_ws) + (step_ws_doubles(M, D) + 1) / 2 * 2);
+// the planes of the step workspace, carved after its FP64 region
+inline StepPlanes step_planes(Carve& c, int M) {
     StepPlanes s;
     s.ldk = pad4(M); s.ld2m = pad4(2L * M);
-    s.Whi = p; p += 2L * M * s.ldk;
-    s.Wlo = p; p += 2L * M * s.ldk;
-    s.Wthi = p; p += (long)M * s.ld2m;
-    s.Wtlo = p; p += (long)M * s.ld2m;
-    s.u = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(p) + 15) & ~uintptr_t(15));
+    s.Whi = c.take<float>(2L * M * s.ldk);
+    s.Wlo = c.take<float>(2L * M * s.ldk);
+    s.Wthi = c.take<float>((long)M * s.ld2m);
+    s.Wtlo = c.take<float>((long)M * s.ld2m);
+    s.u = c.take<double>(M);
     return s;
 }
 
-inline size_t batch_plane_floats(int M, long R) {
-    const long Rc = chunk_rows(R), ldk = pad4(M), ld2m = pad4(2L * M), ldt = pad4(Rc);
-    const long nch = (R + Rc - 1) / Rc;
-    return (size_t)(R * ld2m + 2 * R * ldk + 2 * nch * (long)M * ldt + 2 * Rc * ld2m + 2 * 2L * M * ldt + Rc * ldk + 64);
-}
-
-inline BatchPlanes carve_batch_planes(void* ws, int M, long R) {
+inline BatchPlanes batch_planes(Carve& c, int M, long R) {
     BatchPlanes b;
     b.Rc = chunk_rows(R); b.ldk = pad4(M); b.ld2m = pad4(2L * M); b.ldt = pad4(b.Rc);
-    float* p = reinterpret_cast<float*>(ws);
-    b.AB = p; p += R * b.ld2m;
     const long nch = (R + b.Rc - 1) / b.Rc;
-    b.Khi = p; p += R * b.ldk; b.Klo = p; p += R * b.ldk;
-    b.KThi = p; p += nch * (long)M * b.ldt; b.KTlo = p; p += nch * (long)M * b.ldt;
-    b.Phi = p; p += b.Rc * b.ld2m; b.Plo = p; p += b.Rc * b.ld2m;
-    b.PThi = p; p += 2L * M * b.ldt; b.PTlo = p; p += 2L * M * b.ldt;
-    b.Kbar = p;
+    b.AB = c.take<float>(R * b.ld2m);
+    b.Khi = c.take<float>(R * b.ldk); b.Klo = c.take<float>(R * b.ldk);
+    b.KThi = c.take<float>(nch * (long)M * b.ldt); b.KTlo = c.take<float>(nch * (long)M * b.ldt);
+    b.Phi = c.take<float>(b.Rc * b.ld2m); b.Plo = c.take<float>(b.Rc * b.ld2m);
+    b.PThi = c.take<float>(2L * M * b.ldt); b.PTlo = c.take<float>(2L * M * b.ldt);
+    b.Kbar = c.take<float>(b.Rc * b.ldk);
     return b;
 }
 
-inline int make_step_planes(const StepView& v, void* step_ws, cudaStream_t st) {
-    StepPlanes s = carve_step_planes(step_ws, v.M, v.D);
+inline int make_step_planes(const StepView& v, const StepPlanes& s, cudaStream_t st) {
     dim3 grid((unsigned)cdiv(v.M, 32), (unsigned)cdiv(v.M, 32));
     k_make_w_planes<<<grid, 256, 0, st>>>(v.Linv, v.Cm, v.Mp, v.M, s.Whi, s.Wlo, s.ldk, s.Wthi, s.Wtlo, s.ld2m);
     TGP_TRY(check_launch("k_make_w_planes"));
@@ -76,12 +62,12 @@ inline int row_grid128(long R) {
     return (int)(blocks < 148 * 16 ? blocks : 148 * 16);
 }
 
-// forward: K planes per chunk -> [A | B] = K [Linv; C]^T on tcgen05 -> row statistics
-inline int qf_forward(const StepView& s, void* step_ws, void* batch_ws, const double* X, long R, double* mu, double* v,
+// forward: K planes per chunk -> [A | B] = K [Linv; C]^T on tcgen05 -> row statistics.  The K generation reads u = L^-T m:
+// it joins the factorisation first.
+inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, double* mu, double* v,
                       cudaStream_t st) {
     const int M = s.M, D = s.D;
-    StepPlanes sp = carve_step_planes(step_ws, M, D);
-    BatchPlanes b = carve_batch_planes(batch_ws, M, R);
+    if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     if (g_fused_forward && D <= FUSED_MAX_D) {
         FusedFwdParams fp;
         fp.X = X; fp.Zs = s.Zs; fp.ls = s.ls; fp.os = s.os; fp.mvec = s.mvec;
@@ -89,7 +75,7 @@ inline int qf_forward(const StepView& s, void* step_ws, void* batch_ws, const do
         Operand W{sp.Whi, sp.Wlo, 2L * M, M, sp.ldk};
         return fwd_fused(W, fp, st);
     }
-    // mu = K_xz (L^-T m) is accumulated in FP64 by the K generation (u is ready: the caller has joined the factorisation)
+    // mu = K_xz (L^-T m) is accumulated in FP64 by the K generation
     cudaMemsetAsync(mu, 0, (size_t)R * sizeof(double), st);
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
@@ -110,12 +96,10 @@ inline int qf_forward(const StepView& s, void* step_ws, void* batch_ws, const do
 }
 
 // backward: ABbar planes (+transposes), K^T planes; Kbar = ABbar Wt^T; kernel gradients; Gbar / Cbar += ABbar^T K
-inline int qf_backward(const StepView& s, void* step_ws, void* batch_ws, const double* X, long R, const double* g_mu,
+inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
                        const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
                        cudaStream_t st) {
     const int M = s.M, D = s.D;
-    StepPlanes sp = carve_step_planes(step_ws, M, D);
-    BatchPlanes b = carve_batch_planes(batch_ws, M, R);
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
         {

@@ -6,6 +6,7 @@
 #include "step_kernels.cuh"
 #include "row_kernels.cuh"
 #include "backward_kernels.cuh"
+#include "f64_driver.cuh"
 #include "tc_driver.cuh"
 #include "flow_mlp.cuh"
 #include "crt_driver.cuh"
@@ -20,30 +21,7 @@ GemmTimer g_gemm_timer;
 namespace tc { int g_fused_forward = 0; }
 int g_overlap_kgen = 1;
 
-long g_row_chunk = 32768;             // rows per launch of the batch contractions (Kbar / Abar staging); measured at cfg4:
-                                      // 8192 -> 20.3 ms/step, 16384 -> 20.0, 32768 -> 19.6, 65536 -> 19.5
-
-// AB = [A | B] (R x 2M) and K (R x M) are kept from the forward for the backward; Kbar / Abar are per-chunk staging
-struct BatchView { double *AB, *Kbuf, *Kbar, *Abar; long Rc; };
-
-inline long chunk_rows(long R) { return R < g_row_chunk ? R : g_row_chunk; }
 inline long even(long x) { return (x + 1) / 2 * 2; }
-
-inline size_t batch_ws_doubles(int M, long R) {
-    const long Rc = chunk_rows(R);
-    return (size_t)even(R * 2 * M) + (size_t)even(R * M) + 2 * (size_t)even(Rc * M) + 16;
-}
-
-inline BatchView carve_batch(void* ws, int M, long R) {
-    BatchView b;
-    b.Rc = chunk_rows(R);
-    double* p = reinterpret_cast<double*>(ws);
-    b.AB = p; p += even(R * 2 * M);
-    b.Kbuf = p; p += even(R * M);
-    b.Kbar = p; p += even(b.Rc * M);
-    b.Abar = p;
-    return b;
-}
 
 inline TgpReduceLayout reduce_layout(const TgpModel* md) {
     TgpReduceLayout l;
@@ -122,20 +100,6 @@ inline void fill_flow(FlowDesc& fd, const TgpModel* md) {
     for (int i = 0; i < md->n_layers; ++i) fd.layers[i] = md->layers[i];
 }
 
-// The weight-gradient GEMMs have only (M/128)^2 output tiles but a reduction over thousands of rows: split the
-// reduction so that the live CTAs fill whole waves of the 148 SMs (36 lower tiles x 4 splits = 144 CTAs at M = 1024).
-inline int weight_splitk(int M, int rc, bool lower) {
-    const long tiles = gemm_tiles(M, M, lower);
-    const long max_split = rc / (8 * GBK) > 0 ? rc / (8 * GBK) : 1;
-    auto util = [&](long s) { const long c = tiles * s; return (double)c / (double)(cdiv(c, GEMM_SLOTS) * GEMM_SLOTS); };
-    double best_util = 0.0;
-    for (long s = 1; s <= max_split && s <= 64; ++s) best_util = util(s) > best_util ? util(s) : best_util;
-    int best = 1;
-    for (long s = 1; s <= max_split && s <= 64; ++s)           // smallest split that fills the waves (fewest atomics)
-        if (util(s) >= best_util - 0.03) { best = (int)s; break; }
-    return best;
-}
-
 // M x M x M products of the per-step chain have only (M/128)^2 output tiles: split their reduction (FP64 atomics into a
 // zeroed output) so that one launch fills the SMs instead of running 36-64 long CTAs.
 inline int gemm_small(GemmArgs g, cudaStream_t st) {
@@ -153,15 +117,14 @@ inline int gemm_small(GemmArgs g, cudaStream_t st) {
     return gemm_f64(g, st);
 }
 
-// the integer-residue step region follows the FP64 matrices and the FP32 planes of the step workspace
-inline size_t crt_step_offset(const TgpModel* md) {
-    const size_t b = step_ws_doubles(md->M, md->D) * sizeof(double) + tc::step_plane_floats(md->M) * sizeof(float);
-    return (b + 255) / 256 * 256;
-}
-
-inline int row_grid(long R) {
-    const long blocks = cdiv(R, ROW_THREADS / 32);
-    return (int)(blocks < 148 * 16 ? blocks : 148 * 16);
+// The step workspace: the FP64 region, then the planes of the active tensor-core mode (TGP_F64 has none)
+struct StepWorkspace { StepView f64; tc::StepPlanes tc; crt::StepPlanes crt; };
+inline StepWorkspace step_layout(Carve& c, const TgpModel* md) {
+    StepWorkspace w{};
+    w.f64 = step_view(c, md->M, md->D);
+    if (md->dtype == TGP_F32) w.tc = tc::step_planes(c, md->M);
+    if (md->dtype == TGP_F64_I8) w.crt = crt::step_planes(c, md->M);
+    return w;
 }
 }  // namespace tgp
 
@@ -174,14 +137,18 @@ int tgp_version(void) { return 100; }
 
 size_t tgp_step_workspace_bytes(const TgpModel* md) {
     if (validate(md)) return 0;
-    return crt_step_offset(md) + (md->dtype == TGP_F64_I8 ? crt::step_bytes(md->M) : 0);
+    Carve c(nullptr);
+    step_layout(c, md);
+    return c.bytes();
 }
 
 size_t tgp_batch_workspace_bytes(const TgpModel* md, long R) {
     if (validate(md) || R < 0) return 0;
-    if (md->dtype == TGP_F32) return tc::batch_plane_floats(md->M, R) * sizeof(float);
-    if (md->dtype == TGP_F64_I8) return crt::batch_bytes(md->M, md->D, R);
-    return batch_ws_doubles(md->M, R) * sizeof(double);
+    Carve c(nullptr);
+    if (md->dtype == TGP_F32) tc::batch_planes(c, md->M, R);
+    else if (md->dtype == TGP_F64_I8) crt::batch_view(c, md->M, md->D, R);
+    else f64::batch_view(c, md->M, R);
+    return c.bytes();
 }
 
 int tgp_reduce_layout(const TgpModel* md, TgpReduceLayout* out) {
@@ -212,12 +179,13 @@ int tgp_prepare(const TgpModel* md, const TgpParams* p, double jitter, void* ste
     if (!p || !step_ws || !kl_out || !status) return set_error(-1, "NULL argument to tgp_prepare");
     cudaStream_t st = (cudaStream_t)stream;
     if (join_factor(st)) return set_error(-100, "join with the previous factorisation failed");      // it may still use this workspace
-    StepView v = carve_step(step_ws, md->M, md->D);
-    TGP_TRY(run_prepare(v, (const double*)p->Z, (const double*)p->raw_lengthscale, (const double*)p->raw_outputscale,
+    Carve c(step_ws);
+    const StepWorkspace w = step_layout(c, md);
+    TGP_TRY(run_prepare(w.f64, (const double*)p->Z, (const double*)p->raw_lengthscale, (const double*)p->raw_outputscale,
                         (const double*)p->m, (const double*)p->L_raw, jitter, kl_out, status, md->dtype != TGP_F64, st, fork_factor));
     cudaStream_t fst = g_factor_stream;
-    if (md->dtype == TGP_F32) TGP_TRY(tc::make_step_planes(v, step_ws, fst));
-    if (md->dtype == TGP_F64_I8) TGP_TRY(crt::make_step_planes(v, reinterpret_cast<char*>(step_ws) + crt_step_offset(md), fst));
+    if (md->dtype == TGP_F32) TGP_TRY(tc::make_step_planes(w.f64, w.tc, fst));
+    if (md->dtype == TGP_F64_I8) TGP_TRY(crt::make_step_planes(w.f64, w.crt, fst));
     SideStream& ss = side_stream();
     ss.status_valid = false;
     if (!stream_is_capturing(st)) {          // the pivot status travels to pinned host memory behind the factorisation alone
@@ -240,6 +208,7 @@ int tgp_factor_status(int* status_out) {
     return 0;
 }
 
+// Each mode's qf_forward joins the factorisation as soon as it has enqueued the work that does not need it
 int tgp_qf_forward(const TgpModel* md, const void* step_ws, void* batch_ws, const void* X, long R, void* mu, void* v,
                    void* stream) {
     TGP_TRY(validate(md));
@@ -247,40 +216,13 @@ int tgp_qf_forward(const TgpModel* md, const void* step_ws, void* batch_ws, cons
     if (!step_ws || !batch_ws || !X || !mu || !v) return set_error(-1, "NULL argument to tgp_qf_forward");
     cudaStream_t st = (cudaStream_t)stream;
     const int M = md->M, D = md->D;
-    StepView s = carve_step(const_cast<void*>(step_ws), M, D);
-    if (md->dtype == TGP_F32) {
-        if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
-    }
-    if (md->dtype == TGP_F32)
-        return tc::qf_forward(s, const_cast<void*>(step_ws), batch_ws, (const double*)X, R, (double*)mu, (double*)v, st);
-    if (md->dtype == TGP_F64_I8)
-        return crt::qf_forward(s, reinterpret_cast<char*>(const_cast<void*>(step_ws)) + crt_step_offset(md), batch_ws, (const double*)X,
-                               R, (double*)mu, (double*)v, st);
-    BatchView b = carve_batch(batch_ws, M, R);
+    Carve cs(const_cast<void*>(step_ws)), cb(batch_ws);
+    const StepWorkspace w = step_layout(cs, md);
     const double* Xd = (const double*)X;
-    // K_xz of every chunk depends on the transformed parameters only: it is enqueued BEFORE the join with the factorisation
-    // (which may still be running on the library's high-priority stream, TGP_OPT_OVERLAP_KGEN) and runs under it
-    for (long r0 = 0; r0 < R; r0 += b.Rc) {
-        const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        TGP_TRY(launch_rbf(Xd + r0 * D, s.Zs, s.ls, s.os, rc, M, D, 0, b.Kbuf + r0 * M, M, rc, M, 0.0, st));
-    }
-    if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
-    for (long r0 = 0; r0 < R; r0 += b.Rc) {
-        const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        double* Kc = b.Kbuf + r0 * M;
-        // A = K L^-T   (Bop[n,k] = Linv[n,k], nonzero k <= n)
-        GemmArgs ga = make_gemm(rc, M, M, Kc, M, 0, s.Linv, s.Mp, 0, b.AB + r0 * 2 * M, 2 * M);
-        ga.b_tri = 1;
-        ga.tag = 1;
-        TGP_TRY(gemm_f64(ga, st));
-        // B = A L_S   (Bop[n,k] = L_S[k,n], nonzero k >= n) — the reference's two-contraction form, both triangular
-        GemmArgs gb = make_gemm(rc, M, M, b.AB + r0 * 2 * M, 2 * M, 0, s.LS, s.Mp, 1, b.AB + r0 * 2 * M + M, 2 * M);
-        gb.b_tri = 2;
-        gb.tag = 1;
-        TGP_TRY(gemm_f64(gb, st));
-    }
-    k_row_stats<<<row_grid(R), ROW_THREADS, 0, st>>>(b.AB, s.mvec, s.os, (int)R, M, (double*)mu, (double*)v);
-    return check_launch("k_row_stats");
+    if (md->dtype == TGP_F32) return tc::qf_forward(w.f64, w.tc, tc::batch_planes(cb, M, R), Xd, R, (double*)mu, (double*)v, st);
+    if (md->dtype == TGP_F64_I8)
+        return crt::qf_forward(w.f64, w.crt, crt::batch_view(cb, M, D, R), Xd, R, (double*)mu, (double*)v, st);
+    return f64::qf_forward(w.f64, f64::batch_view(cb, M, R), Xd, R, (double*)mu, (double*)v, st);
 }
 
 int tgp_ell_forward(const TgpModel* md, const TgpParams* p, const void* mu, const void* v, const void* Y,
@@ -317,53 +259,19 @@ int tgp_qf_backward(const TgpModel* md, const TgpParams* p, const void* step_ws,
         return set_error(-1, "NULL argument to tgp_qf_backward");
     cudaStream_t st = (cudaStream_t)stream;
     const int M = md->M, D = md->D;
-    StepView s = carve_step(const_cast<void*>(step_ws), M, D);
-    BatchView b = carve_batch(batch_ws, M, R);
+    Carve cs(const_cast<void*>(step_ws)), cb(batch_ws);
+    const StepWorkspace w = step_layout(cs, md);
     const TgpReduceLayout l = reduce_layout(md);
     const double* Xd = (const double*)X;
+    const double *gm = (const double*)g_mu, *gv = (const double*)g_v;
+    double *dm = reduce_buf + l.dm, *dos = reduce_buf + l.dos, *dZ = reduce_buf + l.dZ, *dls = reduce_buf + l.dls;
+    double *Gbar = reduce_buf + l.Gbar, *Cbar = reduce_buf + l.Cbar;
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
-    double* Gbar = reduce_buf + l.Gbar;
-    double* Cbar = reduce_buf + l.Cbar;
     if (md->dtype == TGP_F32)
-        return tc::qf_backward(s, const_cast<void*>(step_ws), batch_ws, Xd, R, (const double*)g_mu, (const double*)g_v,
-                               reduce_buf + l.dm, reduce_buf + l.dos, reduce_buf + l.dZ, reduce_buf + l.dls, Gbar, Cbar, st);
+        return tc::qf_backward(w.f64, w.tc, tc::batch_planes(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
     if (md->dtype == TGP_F64_I8)
-        return crt::qf_backward(s, reinterpret_cast<char*>(const_cast<void*>(step_ws)) + crt_step_offset(md), batch_ws, Xd, R,
-                                (const double*)g_mu, (const double*)g_v, reduce_buf + l.dm, reduce_buf + l.dos, reduce_buf + l.dZ,
-                                reduce_buf + l.dls, Gbar, Cbar, st);
-    // FP64 mode keeps the reference's two dependent triangular contractions (a = L^-1 k, b = L_S^T a):
-    //   Bbar = 2 g_v B;  Abar = g_mu m - 2 g_v A + Bbar L_S^T;  Kbar = Abar L^-1;
-    //   Gbar += tril(Abar^T K);  dL_S += tril(A^T Bbar)   (accumulated in the `Cbar` slot of the reduce buffer)
-    for (long r0 = 0; r0 < R; r0 += b.Rc) {
-        const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        double* ABc = b.AB + r0 * 2 * M;
-        {
-            dim3 grid((unsigned)cdiv(M, ABB_COLS), (unsigned)cdiv(rc, ABB_ROWS));
-            k_make_abbar<<<grid, ABB_COLS, 0, st>>>(ABc, b.Abar, (const double*)g_mu + r0, (const double*)g_v + r0, s.mvec,
-                                                    rc, M, reduce_buf + l.dm, reduce_buf + l.dos);
-            TGP_TRY(check_launch("k_make_abbar"));
-        }
-        // Abar += Bbar * L_S^T   (Bop[n,k] = L_S[n,k], nonzero k <= n)
-        GemmArgs g0 = make_gemm(rc, M, M, ABc + M, 2 * M, 0, s.LS, s.Mp, 0, b.Abar, M, 1.0, 1.0);
-        g0.b_tri = 1; g0.tag = 1;
-        TGP_TRY(gemm_f64(g0, st));
-        const double* Kc = b.Kbuf + r0 * M;          // K_xz of these rows, kept by the forward
-        // Kbar = Abar * Linv     (Bop[n,k] = Linv[k,n], nonzero k >= n)
-        GemmArgs g1 = make_gemm(rc, M, M, b.Abar, M, 0, s.Linv, s.Mp, 1, b.Kbar, M);
-        g1.b_tri = 2; g1.tag = 1;
-        TGP_TRY(gemm_f64(g1, st));
-        TGP_TRY(launch_kernel_grads(b.Kbar, M, Xd + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, reduce_buf + l.dZ,
-                                    reduce_buf + l.dls, reduce_buf + l.dos, st, Kc, M));
-        // Gbar += tril(Abar^T K)      (reduction over the rows of the chunk)
-        GemmArgs g3 = make_gemm(M, M, rc, b.Abar, M, 1, Kc, M, 1, Gbar, s.Mp, 1.0, 1.0);
-        g3.c_lower = 1; g3.splitk = weight_splitk(M, rc, true); g3.tag = 1;
-        TGP_TRY(gemm_f64(g3, st));
-        // dL_S += tril(A^T Bbar)
-        GemmArgs g4 = make_gemm(M, M, rc, ABc, 2 * M, 1, ABc + M, 2 * M, 1, Cbar, s.Mp, 1.0, 1.0);
-        g4.c_lower = 1; g4.splitk = weight_splitk(M, rc, true); g4.tag = 1;
-        TGP_TRY(gemm_f64(g4, st));
-    }
-    return 0;
+        return crt::qf_backward(w.f64, w.crt, crt::batch_view(cb, M, D, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
+    return f64::qf_backward(w.f64, f64::batch_view(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
 }
 
 int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, const double* reduce_buf, double gE,
@@ -377,7 +285,8 @@ int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, co
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     const int M = md->M, D = md->D, Mp = pad_M(md->M);
     const size_t mm = (size_t)Mp * Mp;
-    StepView s = carve_step(step_ws, M, D);
+    Carve c(step_ws);
+    const StepView s = step_layout(c, md).f64;
     const TgpReduceLayout l = reduce_layout(md);
     const double* Cbar = reduce_buf + l.Cbar;
     double* Gtot = s.Kzz;                          // K_zz's buffer is free after the factorisation
@@ -570,41 +479,49 @@ int tgp_flow_mlp_backward(const TgpMlp* m, const void* weights, const void* X, l
 }
 
 // ---- single-call interface ------------------------------------------------------------------------------------------
+namespace tgp {
+// Regions of the handle's workspace.  The step and batch regions are as large as the staged entry points' queries
+// report, so those entry points carve them again from their own base.
+struct HandleView {
+    void *step, *batch;
+    double *reduce, *packed;
+    double *kl;                                  // the KL term of the last factorisation
+    double *mu, *v, *g_mu, *g_v, *ell_rows;      // max_rows each
+};
+inline HandleView handle_view(Carve& c, const TgpModel* md, long max_rows) {
+    const TgpReduceLayout l = reduce_layout(md);
+    HandleView w;
+    w.step = c.take<char>(tgp_step_workspace_bytes(md));
+    w.batch = c.take<char>(tgp_batch_workspace_bytes(md, max_rows));
+    w.reduce = c.take<double>(l.total);
+    w.packed = c.take<double>(l.packed_total);
+    w.kl = c.take<double>(1);
+    w.mu = c.take<double>(max_rows);
+    w.v = c.take<double>(max_rows);
+    w.g_mu = c.take<double>(max_rows);
+    w.g_v = c.take<double>(max_rows);
+    w.ell_rows = c.take<double>(max_rows);
+    return w;
+}
+}  // namespace tgp
+
 struct TgpHandle {
     TgpModel model;
     long max_rows;
-    size_t need_bytes, bound_bytes;
-    // regions of the bound workspace
-    char* base;
-    size_t off_step, off_batch, off_reduce, off_packed, off_rows;
+    bool bound;
+    tgp::HandleView ws;          // regions of the bound workspace
     long last_R;                 // rows of the last forward (the backward must match)
     bool prepared;
 };
 
 namespace tgp {
-inline size_t align256(size_t x) { return (x + 255) / 256 * 256; }
-inline size_t row_region_bytes(long max_rows) { return align256((size_t)(max_rows + 16) * sizeof(double)); }
-inline void handle_layout(TgpHandle* h) {
-    const TgpModel* md = &h->model;
-    const TgpReduceLayout l = reduce_layout(md);
-    size_t o = 0;
-    h->off_step = o;   o += align256(tgp_step_workspace_bytes(md));
-    h->off_batch = o;  o += align256(tgp_batch_workspace_bytes(md, h->max_rows));
-    h->off_reduce = o; o += align256((size_t)l.total * sizeof(double));
-    h->off_packed = o; o += align256((size_t)l.packed_total * sizeof(double));
-    h->off_rows = o;   o += row_region_bytes(h->max_rows) * 5;   // mu, v, g_mu, g_v, [8 scratch doubles | ell_rows]
-    h->need_bytes = o;
-}
-inline double* row_region(TgpHandle* h, int i) {
-    return reinterpret_cast<double*>(h->base + h->off_rows + (size_t)i * row_region_bytes(h->max_rows));
-}
 __global__ void k_fwd_terms(const double* __restrict__ rb_ell, const double* __restrict__ kl, double scale, double* __restrict__ terms) {
     terms[0] = scale * rb_ell[0];
     terms[1] = kl[0];
 }
 inline int handle_ready(TgpHandle* h, const TgpBatch* b) {
     if (!h) return set_error(-1, "handle is NULL");
-    if (!h->base) return set_error(-1, "no workspace bound: call tgp_bind_workspace first");
+    if (!h->bound) return set_error(-1, "no workspace bound: call tgp_bind_workspace first");
     if (!b || b->R < 0 || b->R > h->max_rows) return set_error(-1, "batch rows exceed the max_rows the handle was created for");
     return 0;
 }
@@ -612,18 +529,16 @@ inline int handle_ready(TgpHandle* h, const TgpBatch* b) {
 
 size_t tgp_workspace_bytes(const TgpModel* md, long max_rows) {
     if (validate(md) || max_rows < 1) return 0;
-    TgpHandle h{};
-    h.model = *md; h.max_rows = max_rows;
-    handle_layout(&h);
-    return h.need_bytes;
+    Carve c(nullptr);
+    handle_view(c, md, max_rows);
+    return c.bytes();
 }
 
 int tgp_create(const TgpModel* md, long max_rows, TgpHandle** out) {
     TGP_TRY(validate(md));
     if (!out || max_rows < 1) return set_error(-1, "tgp_create: out is NULL or max_rows < 1");
     TgpHandle* h = new TgpHandle();
-    h->model = *md; h->max_rows = max_rows; h->base = nullptr; h->bound_bytes = 0; h->last_R = -1; h->prepared = false;
-    handle_layout(h);
+    h->model = *md; h->max_rows = max_rows; h->bound = false; h->last_R = -1; h->prepared = false;
     *out = h;
     return 0;
 }
@@ -632,10 +547,12 @@ void tgp_destroy(TgpHandle* h) { delete h; }
 
 int tgp_bind_workspace(TgpHandle* h, void* workspace, size_t bytes) {
     if (!h || !workspace) return set_error(-1, "NULL argument to tgp_bind_workspace");
-    handle_layout(h);            // the row-chunk option may have changed since tgp_create
-    if (bytes < h->need_bytes) return set_error(-1, "workspace smaller than tgp_workspace_bytes()");
+    // the size is asked for again: the row-chunk option may have changed since tgp_create
+    if (bytes < tgp_workspace_bytes(&h->model, h->max_rows)) return set_error(-1, "workspace smaller than tgp_workspace_bytes()");
     if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) return set_error(-2, "workspace must be 256-byte aligned");
-    h->base = reinterpret_cast<char*>(workspace); h->bound_bytes = bytes; h->prepared = false; h->last_R = -1;
+    Carve c(workspace);
+    h->ws = handle_view(c, &h->model, h->max_rows);
+    h->bound = true; h->prepared = false; h->last_R = -1;
     return 0;
 }
 
@@ -645,20 +562,17 @@ int tgp_elbo_fwd(TgpHandle* h, const TgpParams* p, const TgpBatch* b, double jit
     const TgpModel* md = &h->model;
     cudaStream_t st = (cudaStream_t)stream;
     const TgpReduceLayout l = reduce_layout(md);
-    double* rb = reinterpret_cast<double*>(h->base + h->off_reduce);
-    double* kl = row_region(h, 4);               // 8 scratch doubles at the head of the fifth row region
-    void* step_ws = h->base + h->off_step;
-    void* batch_ws = h->base + h->off_batch;
-    double* mu = out->mu ? (double*)out->mu : row_region(h, 0);
-    double* v = out->v ? (double*)out->v : row_region(h, 1);
-    double* rows = out->ell_rows ? (double*)out->ell_rows : row_region(h, 4) + 8;
-    cudaMemsetAsync(rb, 0, (size_t)l.total * sizeof(double), st);
-    TGP_TRY(tgp_prepare(md, p, jitter, step_ws, kl, out->status, stream));
+    const HandleView& w = h->ws;
+    double* mu = out->mu ? (double*)out->mu : w.mu;
+    double* v = out->v ? (double*)out->v : w.v;
+    double* rows = out->ell_rows ? (double*)out->ell_rows : w.ell_rows;
+    cudaMemsetAsync(w.reduce, 0, (size_t)l.total * sizeof(double), st);
+    TGP_TRY(tgp_prepare(md, p, jitter, w.step, w.kl, out->status, stream));
     h->prepared = true;
-    TGP_TRY(tgp_qf_forward(md, step_ws, batch_ws, b->X, b->R, mu, v, stream));
-    TGP_TRY(tgp_ell_forward(md, p, mu, v, b->Y, b->rowparams, b->R, b->scale, b->quad_t, b->quad_w, 1, rows, row_region(h, 2),
-                            row_region(h, 3), nullptr, rb, stream));
-    k_fwd_terms<<<1, 1, 0, st>>>(rb + l.ell_sum, kl, b->scale, out->terms);
+    TGP_TRY(tgp_qf_forward(md, w.step, w.batch, b->X, b->R, mu, v, stream));
+    TGP_TRY(tgp_ell_forward(md, p, mu, v, b->Y, b->rowparams, b->R, b->scale, b->quad_t, b->quad_w, 1, rows, w.g_mu, w.g_v,
+                            nullptr, w.reduce, stream));
+    k_fwd_terms<<<1, 1, 0, st>>>(w.reduce + l.ell_sum, w.kl, b->scale, out->terms);
     h->last_R = b->R;
     return check_launch("k_fwd_terms");
 }
@@ -672,17 +586,15 @@ int tgp_elbo_bwd(TgpHandle* h, const TgpParams* p, const TgpBatch* b, const doub
     if (md->n_rowparams > 0)
         return set_error(-1, "input-dependent flows: use the staged entry points (drowparams flows back to the caller's MLP)");
     const TgpReduceLayout l = reduce_layout(md);
-    double* rb = reinterpret_cast<double*>(h->base + h->off_reduce);
-    void* step_ws = h->base + h->off_step;
-    TGP_TRY(tgp_qf_backward(md, p, step_ws, h->base + h->off_batch, b->X, b->R, row_region(h, 2), row_region(h, 3), rb, stream));
+    const HandleView& w = h->ws;
+    TGP_TRY(tgp_qf_backward(md, p, w.step, w.batch, b->X, b->R, w.g_mu, w.g_v, w.reduce, stream));
     if (allreduce) {
-        double* packed = reinterpret_cast<double*>(h->base + h->off_packed);
-        TGP_TRY(tgp_reduce_pack(md, rb, packed, stream));
-        if (allreduce(packed, l.packed_total, user, stream) != 0) return set_error(-103, "the all-reduce callback failed");
-        TGP_TRY(tgp_reduce_unpack(md, packed, rb, stream));
+        TGP_TRY(tgp_reduce_pack(md, w.reduce, w.packed, stream));
+        if (allreduce(w.packed, l.packed_total, user, stream) != 0) return set_error(-103, "the all-reduce callback failed");
+        TGP_TRY(tgp_reduce_unpack(md, w.packed, w.reduce, stream));
     }
     h->last_R = -1;
-    return tgp_chain_backward(md, p, step_ws, rb, 0.0, 0.0, g_dev, g->dZ, g->draw_lengthscale, g->draw_outputscale, g->dm,
+    return tgp_chain_backward(md, p, w.step, w.reduce, 0.0, 0.0, g_dev, g->dZ, g->draw_lengthscale, g->draw_outputscale, g->dm,
                               g->dL_raw, g->dlog_var_noise, g->dtheta, stream);
 }
 
@@ -692,15 +604,15 @@ int tgp_test_nll_fwd(TgpHandle* h, const TgpParams* p, const TgpBatch* b, int re
     TGP_TRY(handle_ready(h, b));
     if (!p || !logp_rows || !m1 || !m2) return set_error(-1, "NULL argument to tgp_test_nll_fwd");
     const TgpModel* md = &h->model;
-    void* step_ws = h->base + h->off_step;
+    const HandleView& w = h->ws;
     if (refactor || !h->prepared) {
         if (!status) return set_error(-1, "status required when the factorisation is (re)computed");
-        TGP_TRY(tgp_prepare(md, p, 0.0, step_ws, row_region(h, 4), status, stream));
+        TGP_TRY(tgp_prepare(md, p, 0.0, w.step, w.kl, status, stream));
         h->prepared = true;
     }
-    double* mu = mu_out ? (double*)mu_out : row_region(h, 0);
-    double* v = v_out ? (double*)v_out : row_region(h, 1);
-    TGP_TRY(tgp_qf_forward(md, step_ws, h->base + h->off_batch, b->X, b->R, mu, v, stream));
+    double* mu = mu_out ? (double*)mu_out : w.mu;
+    double* v = v_out ? (double*)v_out : w.v;
+    TGP_TRY(tgp_qf_forward(md, w.step, w.batch, b->X, b->R, mu, v, stream));
     h->last_R = -1;
     return tgp_test_rows(md, p, mu, v, b->Y, b->rowparams, b->R, n_mc, y_std, b->quad_t, b->quad_w, bern_std, logp_rows, m1,
                          m2, stream);
@@ -760,7 +672,7 @@ int tgp_set_option(int key, int value) {
     if (key == TGP_OPT_OVERLAP_KGEN) { g_overlap_kgen = value != 0; return 0; }
     if (key == TGP_OPT_ROW_CHUNK) {
         if (value < 128) return set_error(-1, "row chunk must be >= 128");
-        g_row_chunk = value;
+        f64::g_row_chunk = value;
         return 0;
     }
     return set_error(-1, "unknown option");
@@ -798,7 +710,11 @@ int tgp_debug_gemm_tf32x3(int Mrows, int Ncols, int K, const float* Ahi, const f
     return tc::gemm_tf32x3(A, B, p, (cudaStream_t)stream);
 }
 
-size_t tgp_debug_gemm_crt_bytes(long M, long N, long K, int T) { return crt::debug_bytes(M, N, K, T); }
+size_t tgp_debug_gemm_crt_bytes(long M, long N, long K, int T) {
+    Carve c(nullptr);
+    crt::debug_scratch(c, M, N, K, T);
+    return c.bytes();
+}
 
 int tgp_debug_gemm_crt(long M, long N, long K, const double* A, long lda, const double* B, long ldb, double* C, long ldc, int T,
                        int tri_mode, int tri_rows, int lower_rows, int accumulate, int mn_major, void* scratch, void* stream) {
@@ -810,7 +726,8 @@ int tgp_debug_gemm_crt(long M, long N, long K, const double* A, long lda, const 
 
 int tgp_debug_export_step(const TgpModel* md, const void* step_ws, double* L, double* Linv, double* C, void* stream) {
     TGP_TRY(validate(md));
-    StepView s = carve_step(const_cast<void*>(step_ws), md->M, md->D);
+    Carve c(const_cast<void*>(step_ws));
+    const StepView s = step_layout(c, md).f64;
     cudaStream_t st = (cudaStream_t)stream;
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     if (L) k_copy_strided<<<md->M, 256, 0, st>>>(s.L, s.Mp, L, md->M, md->M);
