@@ -44,6 +44,11 @@ enum { TGP_FLOW_RESTRICT = 1,        /* set_restrictions: softplus on a (affine)
        TGP_FLOW_SWITCH = 8 };        /* step member with a trainable switch_off (models/flow.py:1130-1149): two more
                                       * GLOBAL parameters [s, t] after the layer's own; output softplus(s) g + t.
                                       * Not combinable with TGP_FLOW_PER_ROW                                  */
+enum { TGP_KERNEL_RBF = 0,           /* s exp(-r^2 / 2)                       gpytorch ScaleKernel(RBFKernel)        */
+       TGP_KERNEL_MATERN12 = 1,      /* s exp(-r)                             gpytorch ScaleKernel(MaternKernel(0.5)) */
+       TGP_KERNEL_MATERN32 = 2,      /* s (1 + sqrt3 r) exp(-sqrt3 r)         nu = 1.5                               */
+       TGP_KERNEL_MATERN52 = 3 };    /* s (1 + sqrt5 r + 5r^2/3) exp(-sqrt5 r)   nu = 2.5
+                                      * r^2 = sum_d ((x_d - z_d) / lengthscale_d)^2, computed by direct differences    */
 #define TGP_MAX_LAYERS 64
 
 typedef struct TgpFlowLayer {
@@ -68,6 +73,8 @@ typedef struct TgpModel {            /* host struct; describes one output GP */
     int n_rowparams;                 /* per-row flow parameters (ID_TGP), 0 otherwise                      */
     int n_layers;
     TgpFlowLayer layers[TGP_MAX_LAYERS];
+    int kernel;                      /* TGP_KERNEL_* (0 = RBF, so a zero-initialised description is unchanged).  Workspace
+                                      * sizes do not depend on it                                                   */
 } TgpModel;
 
 typedef struct TgpParams {           /* device pointers to the model parameters (same shapes as the reference's) */
@@ -261,6 +268,8 @@ int tgp_kmeans_iteration(const void* X, long N, int D, void* C, int M, int* assi
 
 /* Library options.  TGP_OPT_FUSED_FORWARD (tensor-core mode): 1 = tgp_qf_forward is ONE kernel that generates the K_xz
  * tiles inside the tcgen05 contraction and emits mu, v from the TMEM accumulators; 0 = staged planes + separate kernels.
+ * The fused kernel generates RBF tiles only: a model with a Matern kernel (or D above the fused kernel's limit) takes the
+ * staged path whatever the option says, and its backward reuses the K planes that path kept.
  * TGP_OPT_ROW_CHUNK (FP64 mode): rows per launch of the batch contractions (default 32768; a tuning knob — it changes the
  * workspace size, so set it before asking for tgp_batch_workspace_bytes). */
 enum { TGP_OPT_FUSED_FORWARD = 1, TGP_OPT_ROW_CHUNK = 2,

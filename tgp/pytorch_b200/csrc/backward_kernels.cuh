@@ -33,16 +33,18 @@ __global__ void __launch_bounds__(ABB_COLS) k_make_abbar(double* __restrict__ AB
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(dos, accv);
 }
 
-// Accumulates, for t[n,j] = Kbar[n,j] * k(x_n, z_j):
+// Accumulates, for t[n,j] = Kbar[n,j] * os * psi(x_n, z_j) (psi: Cov<KIND>, common.cuh; psi = phi for the RBF):
 //   dZ[j,d]  += zscale * sum_n t * (xs[n,d] - zs[j,d]) / ls[d]
 //   dls[d]   += sum_{n,j} t * (xs[n,d] - zs[j,d])^2 / ls[d]
-//   dos      += sum_{n,j} t / os
+//   dos      += sum_{n,j} Kbar[n,j] * k(x_n, z_j) / os
 // sym = 1 reads Kbar symmetrised, 0.5*(Kbar[n,j] + Kbar[j,n]) (the K_zz case, where X = Zs and R = M).
 // 256 rows per CTA: every CTA ends with one FP64 atomic per (column, dimension), so taller CTAs mean fewer
 // same-address atomics on dZ (128 row-blocks per 8192-row chunk serialised on each address with 64-row CTAs)
 constexpr int KG_TC = 64, KG_TR = 4, KG_THREADS = KG_TC * KG_TR;
 __host__ __device__ constexpr int kg_rows(int maxd) { return maxd <= 16 ? 256 : 64; }      // static shared memory stays below 48 KiB
-template <int MAXD, typename KBT>
+// Kval / Kfhi + Kflo: the forward's K tile, still resident, replaces the distance and the exponential.  RBF only, where
+// psi = phi; the launcher drops them for the other kinds, which recompute the tile from X and Z.
+template <int MAXD, typename KBT, int KIND>
 __global__ void __launch_bounds__(KG_THREADS) k_kernel_grads(const KBT* __restrict__ Kbar, long ldk,
                                                              const double* __restrict__ X, int x_scaled,
                                                              const double* __restrict__ Zs, const double* __restrict__ ls,
@@ -86,9 +88,9 @@ __global__ void __launch_bounds__(KG_THREADS) k_kernel_grads(const KBT* __restri
                 kbr[u] = ok ? (double)Kbar[n * ldk + j] : 0.0;
                 if (sym && ok) kbr[u] = 0.5 * (kbr[u] + (double)Kbar[(long)j * ldk + n]);
                 if constexpr (std::is_same<KBT, float>::value)       // FP32 planes: value = hi + lo exactly
-                    kvr[u] = (Kfhi && ok) ? (double)(Kfhi[n * ldkf + j] + Kflo[n * ldkf + j]) : 0.0;
+                    kvr[u] = (KIND == TGP_KERNEL_RBF && Kfhi && ok) ? (double)(Kfhi[n * ldkf + j] + Kflo[n * ldkf + j]) : 0.0;
                 else
-                    kvr[u] = (Kval && ok) ? Kval[n * ldkv + j] : 0.0;
+                    kvr[u] = (KIND == TGP_KERNEL_RBF && Kval && ok) ? Kval[n * ldkv + j] : 0.0;
             }
 #pragma unroll
             for (int u = 0; u < UR; ++u) {
@@ -100,29 +102,37 @@ __global__ void __launch_bounds__(KG_THREADS) k_kernel_grads(const KBT* __restri
                     float df[MAXD];
 #pragma unroll
                     for (int d = 0; d < MAXD; ++d) if (d < D) df[d] = (float)(xs[r][d] - zj[d]);
-                    float t;
-                    if (Kfhi) {                  // the forward's K planes are still resident
+                    float t, tk;
+                    if (KIND == TGP_KERNEL_RBF && Kfhi) {     // the forward's K planes are still resident
                         t = (float)kb * (float)kvr[u];
+                        tk = t;
                     } else {
                         float q = 0.f;
 #pragma unroll
                         for (int d = 0; d < MAXD; ++d) if (d < D) q = fmaf(df[d], df[d], q);
-                        t = (float)kb * (float)s * expf(-0.5f * q);
+                        float ph, ps;
+                        Cov<KIND>::phi_psi_f(q, ph, ps);
+                        t = (float)kb * (float)s * ps;
+                        tk = KIND == TGP_KERNEL_RBF ? t : (float)kb * (float)s * ph;
                     }
-                    asum += t;
+                    asum += tk;
 #pragma unroll
                     for (int d = 0; d < MAXD; ++d) if (d < D) { az[d] = fmaf(t, df[d], az[d]); al[d] = fmaf(t * df[d], df[d], al[d]); }
                 } else {
-                    double t;
-                    if (Kval) {                  // the forward's K tile is still resident: no distance / exponential needed
+                    double t, tk;
+                    if (KIND == TGP_KERNEL_RBF && Kval) {     // the forward's K tile is still resident: no distance / exponential
                         t = kb * kvr[u];
+                        tk = t;
                     } else {
                         double q = 0.0;
 #pragma unroll
                         for (int d = 0; d < MAXD; ++d) if (d < D) { const double df = xs[r][d] - zj[d]; q = fma(df, df, q); }
-                        t = kb * s * exp(-0.5 * q);
+                        double ph, ps;
+                        Cov<KIND>::phi_psi(q, ph, ps);
+                        t = kb * s * ps;
+                        tk = KIND == TGP_KERNEL_RBF ? t : kb * s * ph;
                     }
-                    asum += t;
+                    asum += tk;
 #pragma unroll
                     for (int d = 0; d < MAXD; ++d) if (d < D) {
                         const double df = xs[r][d] - zj[d];
@@ -167,12 +177,13 @@ __global__ void __launch_bounds__(KG_THREADS) k_kernel_grads(const KBT* __restri
     }
 }
 
-template <typename KBT>
+template <int KIND, typename KBT>
 inline int launch_kernel_grads(const KBT* Kbar, long ldk, const double* X, int x_scaled, const double* Zs,
                                const double* ls, const double* os, long R, int M, int D, int sym, double zscale,
                                double* dZ, double* dls, double* dos, cudaStream_t st, const double* Kval = nullptr,
                                long ldkv = 0, const float* Kfhi = nullptr, const float* Kflo = nullptr, long ldkf = 0) {
-#define TGP_KG(MD) k_kernel_grads<MD, KBT><<<dim3((unsigned)cdiv(M, KG_TC), (unsigned)cdiv(R, kg_rows(MD))), KG_THREADS, 0, st>>>(Kbar, ldk, X, x_scaled, Zs, ls, os, R, M, D, sym, \
+    if (KIND != TGP_KERNEL_RBF) { Kval = nullptr; Kfhi = Kflo = nullptr; }     // psi != phi: recompute the tile
+#define TGP_KG(MD) k_kernel_grads<MD, KBT, KIND><<<dim3((unsigned)cdiv(M, KG_TC), (unsigned)cdiv(R, kg_rows(MD))), KG_THREADS, 0, st>>>(Kbar, ldk, X, x_scaled, Zs, ls, os, R, M, D, sym, \
                                                                   zscale, dZ, dls, dos, Kval, ldkv, Kfhi, Kflo, ldkf)
     if (D <= 4) TGP_KG(4);
     else if (D <= 8) TGP_KG(8);

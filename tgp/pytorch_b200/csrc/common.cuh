@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <math.h>
+#include <type_traits>
+#include "../../../include/tgp_b200.h"
 
 #define TGP_WARP 32
 
@@ -126,5 +128,109 @@ struct PerDeviceOnce {
 // softplus and its derivative as torch.nn.functional.softplus (beta=1, threshold=20) evaluates them
 __device__ __forceinline__ double softplus_d(double x) { return x > 20.0 ? x : log1p(exp(x)); }
 __device__ __forceinline__ double sigmoid_d(double x) { return x > 20.0 ? 1.0 : 1.0 / (1.0 + exp(-x)); }
+
+// ---- covariance functions ------------------------------------------------------------------------------------------
+// k(x, z) = s phi(r), r^2 = d2 = sum_d (x_d / l_d - z_d / l_d)^2 (direct differences), TgpModel.kernel = KIND:
+//   RBF         phi = exp(-d2 / 2)                          psi = phi
+//   MATERN12    phi = exp(-r)                               psi = exp(-r) / r          (0 for d2 <= 1e-30)
+//   MATERN32    phi = (1 + sqrt3 r) exp(-sqrt3 r)           psi = 3 exp(-sqrt3 r)
+//   MATERN52    phi = (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r)   psi = 5/3 (1 + sqrt5 r) exp(-sqrt5 r)
+// with psi = -2 dphi / d(d2): the kernel gradients are dk/dz = s psi (x - z) / l^2 and dk/dl = s psi (x - z)^2 / l^3.
+// phi(0) = 1 and 0 <= phi <= 1 for every kind.  psi of MATERN12 is singular at r = 0 (a minibatch row on an inducing
+// point, the K_zz diagonal): such a pair contributes nothing to the Z / lengthscale gradients, which is what
+// sqrt(clamp_min(d2, 1e-30)) yields under autograd.  The other kinds take r = 0 there as well (their psi is smooth).
+// Three flavours, one per consumer:
+//   phi / phi_psi        FP64 (K tiles, FP64 kernel gradients);
+//   kf                   FP64 distance and argument, FP32 exponential exp(a) = expf(a_hi) (1 + a_lo), times s (TF32 planes);
+//   phi_psi_f            FP32 throughout (the FP32 kernel-gradient pass of the tensor-core mode).
+template <int KIND> struct Cov;
+
+template <> struct Cov<TGP_KERNEL_RBF> {
+    static __device__ __forceinline__ double phi(double d2) { return exp(-0.5 * d2); }
+    static __device__ __forceinline__ void phi_psi(double d2, double& ph, double& ps) { ph = exp(-0.5 * d2); ps = ph; }
+    static __device__ __forceinline__ float kf(double d2, float s) {
+        const double arg = -0.5 * d2;
+        const float ahi = (float)arg;
+        return s * expf(ahi) * (1.0f + (float)(arg - (double)ahi));
+    }
+    static __device__ __forceinline__ void phi_psi_f(float d2, float& ph, float& ps) { ph = expf(-0.5f * d2); ps = ph; }
+};
+
+constexpr double COV_R2_MIN = 1e-30;      // d2 at or below this counts as r = 0
+__device__ __forceinline__ double cov_r(double d2) { return d2 > COV_R2_MIN ? sqrt(d2) : 0.0; }
+__device__ __forceinline__ float cov_rf(float d2) { return d2 > (float)COV_R2_MIN ? sqrtf(d2) : 0.f; }
+__device__ __forceinline__ float exp_split(double a) {      // exp(a) with the argument kept in FP64, to FP32 accuracy
+    const float ahi = (float)a;
+    return expf(ahi) * (1.0f + (float)(a - (double)ahi));
+}
+
+template <> struct Cov<TGP_KERNEL_MATERN12> {
+    static __device__ __forceinline__ double phi(double d2) { return exp(-cov_r(d2)); }
+    static __device__ __forceinline__ void phi_psi(double d2, double& ph, double& ps) {
+        const double r = cov_r(d2);
+        ph = exp(-r);
+        ps = r > 0.0 ? ph / r : 0.0;
+    }
+    static __device__ __forceinline__ float kf(double d2, float s) { return s * exp_split(-cov_r(d2)); }
+    static __device__ __forceinline__ void phi_psi_f(float d2, float& ph, float& ps) {
+        const float r = cov_rf(d2);
+        ph = expf(-r);
+        ps = r > 0.f ? ph / r : 0.f;
+    }
+};
+
+template <> struct Cov<TGP_KERNEL_MATERN32> {
+    static constexpr double C = 1.7320508075688772;          // sqrt(3)
+    static __device__ __forceinline__ double phi(double d2) { const double a = C * cov_r(d2); return (1.0 + a) * exp(-a); }
+    static __device__ __forceinline__ void phi_psi(double d2, double& ph, double& ps) {
+        const double a = C * cov_r(d2), e = exp(-a);
+        ph = (1.0 + a) * e;
+        ps = 3.0 * e;
+    }
+    static __device__ __forceinline__ float kf(double d2, float s) {
+        const double a = C * cov_r(d2);
+        return s * exp_split(-a) * (float)(1.0 + a);
+    }
+    static __device__ __forceinline__ void phi_psi_f(float d2, float& ph, float& ps) {
+        const float a = (float)C * cov_rf(d2), e = expf(-a);
+        ph = (1.f + a) * e;
+        ps = 3.f * e;
+    }
+};
+
+template <> struct Cov<TGP_KERNEL_MATERN52> {
+    static constexpr double C = 2.23606797749979;            // sqrt(5)
+    static __device__ __forceinline__ double phi(double d2) {
+        const double a = C * cov_r(d2);
+        return (1.0 + a + a * a / 3.0) * exp(-a);
+    }
+    static __device__ __forceinline__ void phi_psi(double d2, double& ph, double& ps) {
+        const double a = C * cov_r(d2), e = exp(-a);
+        ph = (1.0 + a + a * a / 3.0) * e;
+        ps = (5.0 / 3.0) * (1.0 + a) * e;
+    }
+    static __device__ __forceinline__ float kf(double d2, float s) {
+        const double a = C * cov_r(d2);
+        return s * exp_split(-a) * (float)(1.0 + a + a * a / 3.0);
+    }
+    static __device__ __forceinline__ void phi_psi_f(float d2, float& ph, float& ps) {
+        const float a = (float)C * cov_rf(d2), e = expf(-a);
+        ph = (1.f + a + a * a / 3.f) * e;
+        ps = (5.f / 3.f) * (1.f + a) * e;
+    }
+};
+
+inline bool kernel_kind_valid(int kind) { return kind >= TGP_KERNEL_RBF && kind <= TGP_KERNEL_MATERN52; }
+
+// Runs f(std::integral_constant<int, KIND>{}) for the runtime kind: the one place a driver turns TgpModel.kernel into the
+// template parameter of its kernels (validate() has rejected unknown kinds before any driver runs)
+template <class F> inline int with_kernel(int kind, F&& f) {
+    switch (kind) {
+        case TGP_KERNEL_MATERN12: return f(std::integral_constant<int, TGP_KERNEL_MATERN12>{});
+        case TGP_KERNEL_MATERN32: return f(std::integral_constant<int, TGP_KERNEL_MATERN32>{});
+        case TGP_KERNEL_MATERN52: return f(std::integral_constant<int, TGP_KERNEL_MATERN52>{});
+        default: return f(std::integral_constant<int, TGP_KERNEL_RBF>{});
+    }
+}
 
 }  // namespace tgp

@@ -142,13 +142,14 @@ inline int combine(const uint8_t* R, long ldr, long plane_stride, long rows, int
 }
 
 // K_xz of a row chunk in one pass: FP64 values and residue planes (i8::k_rbf_residues)
+template <int KIND>
 inline int rbf_residues(const double* X, const double* Zs, const double* ls, const double* os, long R, int M, int D, double* Kout,
                         int T, uint8_t* planes, long ldp, long plane_stride, cudaStream_t st, int ctas_per_sm = 3) {
     const long n_tiles = cdiv(M, i8::RS_TC) * cdiv(R, i8::RS_TR);
     // ctas_per_sm = 0: one CTA per tile (short CTAs: a concurrent high-priority stream gets slots every few microseconds)
     const unsigned grid = (unsigned)((ctas_per_sm <= 0 || n_tiles < 148L * ctas_per_sm) ? n_tiles : 148L * ctas_per_sm);
     const i8::CrtTable& tab = i8::crt_table(T);
-#define TGP_RR(MD) i8::k_rbf_residues<MD><<<grid, 256, 0, st>>>(X, Zs, ls, os, R, M, D, Kout, M, 53, tab, planes, ldp, plane_stride)
+#define TGP_RR(MD) i8::k_rbf_residues<MD, KIND><<<grid, 256, 0, st>>>(X, Zs, ls, os, R, M, D, Kout, M, 53, tab, planes, ldp, plane_stride)
     if (D <= 4) TGP_RR(4);
     else if (D <= 8) TGP_RR(8);
     else if (D <= 16) TGP_RR(16);
@@ -279,8 +280,9 @@ __global__ void __launch_bounds__(256) k_wt_residues(const double* __restrict__ 
     i8::emit_residues_rt(tab.T, xi, tab, r, rows, c, M, planes, ldp, plane_stride);
 }
 
-inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, double* mu, double* v,
-                      cudaStream_t st) {
+template <int KIND>
+inline int qf_forward_k(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, double* mu, double* v,
+                        cudaStream_t st) {
     const int M = s.M, D = s.D;
     const int Tf = fwd_T(M), bits = fwd_bits_w(M);
     // K_xz (FP64 values + residue planes) of all rows in one launch.  It depends on Zs / ls / os only, not on the factorisation:
@@ -288,11 +290,11 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& 
     // (TGP_OPT_OVERLAP_KGEN, common.cuh), and runs under it.  K residues: one scale for the whole matrix (0 <= k <= outputscale),
     // shared by the forward and the weight contraction.
     {
-        const int rr = rbf_residues(X, s.Zs, s.ls, s.os, R, M, D, nullptr, T_ALL, b.Kp, b.ldk, R * b.ldk, st, 0);
+        const int rr = rbf_residues<KIND>(X, s.Zs, s.ls, s.os, R, M, D, nullptr, T_ALL, b.Kp, b.ldk, R * b.ldk, st, 0);
         if (rr != 0 && rr != -7) return rr;
         if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
         if (rr == -7) {
-            TGP_TRY(launch_rbf(X, s.Zs, s.ls, s.os, (int)R, M, D, 0, b.Kbuf, M, (int)R, M, 0.0, st));
+            TGP_TRY(launch_rbf<KIND>(X, s.Zs, s.ls, s.os, (int)R, M, D, 0, b.Kbuf, M, (int)R, M, 0.0, st));
             TGP_TRY(to_residues(b.Kbuf, M, R, M, 2, sp.k_exp, 53, T_ALL, b.Kp, b.ldk, R * b.ldk, st));
         }
     }
@@ -310,12 +312,19 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& 
     return 0;
 }
 
-inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
-                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
-                       cudaStream_t st) {
+inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, double* mu, double* v,
+                      cudaStream_t st) {
+    return with_kernel(s.kind, [&](auto k) { return qf_forward_k<decltype(k)::value>(s, sp, b, X, R, mu, v, st); });
+}
+
+template <int KIND>
+inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
+                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                         cudaStream_t st) {
     const int M = s.M, D = s.D;
     TGP_TRY(fill_int(b.zero_exp, 1, 0, st));
-    const double* const kval = b.Kbuf;            // NULL for D <= 32: k_kernel_grads recomputes the K_xz tile (same arithmetic)
+    // NULL for D <= 32: k_kernel_grads recomputes the K_xz tile (same arithmetic); only the RBF reads it for D > 32
+    const double* const kval = b.Kbuf;
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
         const double* ABc = b.AB + r0 * 2 * M;
@@ -353,7 +362,7 @@ inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView&
         }
         // reconstruction of Kbar, then Kbar o K -> dZ, dlengthscale, doutputscale
         TGP_TRY(combine(b.Kbp, b.ldk, (long)b.Rc * b.ldk, rc, M, Tb, bits_x + bits_w, b.zero_exp, 2, b.wc_exp, 1, b.Kbar, M, 0, 0, st));
-        TGP_TRY(launch_kernel_grads(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, kval ? kval + r0 * M : nullptr, M));
+        TGP_TRY(launch_kernel_grads<KIND>(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, kval ? kval + r0 * M : nullptr, M));
         {   // [Gbar; Cbar] (2M x M) += ABbar^T K: reduction over the chunk rows; both operands are row-major planes read MN-major
             i8::Params p{};
             p.Mrows = 2 * M; p.Ncols = M; p.K = rc; p.T = Tw; p.tri_mode = 0; p.tri_rows = 0; p.lower_rows = M; p.mn_major = 3;
@@ -368,6 +377,14 @@ inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView&
         }
     }
     return 0;
+}
+
+inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
+                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                       cudaStream_t st) {
+    return with_kernel(s.kind, [&](auto k) {
+        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+    });
 }
 
 // ---- test hook: C = A B^T through the residue pipeline ------------------------------------------------------------------

@@ -46,10 +46,13 @@ inline int qf_forward(const StepView& s, const BatchView& b, const double* X, lo
     const int M = s.M, D = s.D;
     // K_xz of every chunk depends on the transformed parameters only: it is enqueued BEFORE the join with the factorisation
     // (which may still be running on the library's high-priority stream, TGP_OPT_OVERLAP_KGEN) and runs under it
-    for (long r0 = 0; r0 < R; r0 += b.Rc) {
-        const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        TGP_TRY(launch_rbf(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, 0, b.Kbuf + r0 * M, M, rc, M, 0.0, st));
-    }
+    TGP_TRY(with_kernel(s.kind, [&](auto k) {
+        for (long r0 = 0; r0 < R; r0 += b.Rc) {
+            const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
+            TGP_TRY(launch_rbf<decltype(k)::value>(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, 0, b.Kbuf + r0 * M, M, rc, M, 0.0, st));
+        }
+        return 0;
+    }));
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
@@ -72,8 +75,9 @@ inline int qf_forward(const StepView& s, const BatchView& b, const double* X, lo
 // backward:
 //   Bbar = 2 g_v B;  Abar = g_mu m - 2 g_v A + Bbar L_S^T;  Kbar = Abar L^-1;
 //   Gbar += tril(Abar^T K);  dL_S += tril(A^T Bbar)   (accumulated in the `Cbar` slot of the reduce buffer)
-inline int qf_backward(const StepView& s, const BatchView& b, const double* X, long R, const double* g_mu, const double* g_v,
-                       double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, cudaStream_t st) {
+template <int KIND>
+inline int qf_backward_k(const StepView& s, const BatchView& b, const double* X, long R, const double* g_mu, const double* g_v,
+                         double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, cudaStream_t st) {
     const int M = s.M, D = s.D;
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
@@ -92,7 +96,8 @@ inline int qf_backward(const StepView& s, const BatchView& b, const double* X, l
         GemmArgs g1 = make_gemm(rc, M, M, b.Abar, M, 0, s.Linv, s.Mp, 1, b.Kbar, M);
         g1.b_tri = 2; g1.tag = 1;
         TGP_TRY(gemm_f64(g1, st));
-        TGP_TRY(launch_kernel_grads(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, Kc, M));
+        // the RBF reads K from Kc; the other kinds recompute it (launch_kernel_grads)
+        TGP_TRY(launch_kernel_grads<KIND>(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, Kc, M));
         // Gbar += tril(Abar^T K)      (reduction over the rows of the chunk)
         GemmArgs g3 = make_gemm(M, M, rc, b.Abar, M, 1, Kc, M, 1, Gbar, s.Mp, 1.0, 1.0);
         g3.c_lower = 1; g3.splitk = weight_splitk(M, rc, true); g3.tag = 1;
@@ -103,6 +108,13 @@ inline int qf_backward(const StepView& s, const BatchView& b, const double* X, l
         TGP_TRY(gemm_f64(g4, st));
     }
     return 0;
+}
+
+inline int qf_backward(const StepView& s, const BatchView& b, const double* X, long R, const double* g_mu, const double* g_v,
+                       double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, cudaStream_t st) {
+    return with_kernel(s.kind, [&](auto k) {
+        return qf_backward_k<decltype(k)::value>(s, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+    });
 }
 
 }  // namespace f64

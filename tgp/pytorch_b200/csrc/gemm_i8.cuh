@@ -246,12 +246,12 @@ __global__ void __launch_bounds__(256) k_to_residues(const double* __restrict__ 
     }
 }
 
-// ARD-RBF K tile generated in registers (same arithmetic as k_rbf_tile_reg: x / ls differences, FMA chain, FP64 exp) and
+// ARD K tile generated in registers (same arithmetic as k_rbf_tile_reg: x / ls differences, FMA chain, Cov<KIND>::phi) and
 // converted on the spot: FP64 K (kept for the kernel gradients) and its residue planes in ONE pass.  The same planes serve
 // the forward (reduction over the inducing index: K-major) and the weight contraction (reduction over the rows: MN-major).
-// One scale for the whole matrix: 0 <= k <= outputscale < 2^kexp, kexp derived from the outputscale in-kernel (the kernel
+// One scale for the whole matrix, for every kind: 0 <= k <= outputscale < 2^kexp, kexp derived from the outputscale in-kernel (the kernel
 // depends on nothing the factorisation produces, so it can run on a side stream under it).
-template <int MAXD>
+template <int MAXD, int KIND>
 __global__ void __launch_bounds__(256) k_rbf_residues(const double* __restrict__ X, const double* __restrict__ Zs,
                                                       const double* __restrict__ ls, const double* __restrict__ os, long R, int M, int D,
                                                       double* __restrict__ Kout, long ldk_out, int bits,
@@ -294,7 +294,7 @@ __global__ void __launch_bounds__(256) k_rbf_residues(const double* __restrict__
                 double acc = 0.0;
 #pragma unroll
                 for (int d = 0; d < MAXD; ++d) { const double df = xr[d] - zs[d][tcb + i + (tid & 7)]; acc = fma(df, df, acc); }
-                val = s * exp(-0.5 * acc);
+                val = s * Cov<KIND>::phi(acc);
                 if (Kout) Kout[r * ldk_out + c] = val;
             }
             xi[i] = __double2ll_rn(mul_pow2(val, sh));

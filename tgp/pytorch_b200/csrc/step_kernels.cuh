@@ -20,10 +20,11 @@ __global__ void k_transform_params(const double* __restrict__ Z, const double* _
     if (i < M * D) Zs[i] = Z[i] / softplus_d(raw_ls[i % D]);
 }
 
-// out[n*ldo + j] = os * exp(-0.5 * sum_d (X[n,d]/ls[d] - Zs[j,d])^2)   for n < R, j < M
+// out[n*ldo + j] = os * phi(sum_d (X[n,d]/ls[d] - Zs[j,d])^2)   for n < R, j < M   (phi: Cov<KIND>, common.cuh)
 // pad_identity: rows/cols in [M, Mp) get the identity (used for the padded K_zz); jitter is added on the diagonal.
 // x_scaled: X is already divided by ls (K_zz case, X = Zs).
 constexpr int RBF_TR = 32, RBF_TC = 64, RBF_THREADS = 256;
+template <int KIND>
 __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile(const double* __restrict__ X, const double* __restrict__ Zs,
                                                           const double* __restrict__ ls, const double* __restrict__ os,
                                                           int R, int M, int D, int x_scaled, double* __restrict__ out,
@@ -53,7 +54,7 @@ __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile(const double* __restri
         if (n < R && j < M) {
             double acc = 0.0;
             for (int d = 0; d < D; ++d) { const double df = xs[r * DP + d] - zs[c * DP + d]; acc = fma(df, df, acc); }
-            val = s * exp(-0.5 * acc);
+            val = s * Cov<KIND>::phi(acc);
             if (n == j) val += jitter;
         } else {
             val = (n == j) ? 1.0 : 0.0;
@@ -65,7 +66,7 @@ __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile(const double* __restri
 // Register-blocked variant for D <= 64 (every shipped configuration): a thread owns one column j — its inducing point
 // lives in registers, zero-padded to MAXD — and walks the tile's rows; the X rows are read from shared memory as
 // warp-uniform 16-byte broadcasts (MAXD/2 LDS per element instead of 2*D 8-byte ones in the generic kernel above).
-template <int MAXD>
+template <int MAXD, int KIND>
 __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile_reg(const double* __restrict__ X, const double* __restrict__ Zs,
                                                               const double* __restrict__ ls, const double* __restrict__ os,
                                                               int R, int M, int D, int x_scaled, double* __restrict__ out,
@@ -98,7 +99,7 @@ __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile_reg(const double* __re
                 acc = fma(d0, d0, acc);
                 acc = fma(d1, d1, acc);
             }
-            val = s * exp(-0.5 * acc);
+            val = s * Cov<KIND>::phi(acc);
             if (n == j) val += jitter;
         } else {
             val = (n == j) ? 1.0 : 0.0;
@@ -107,10 +108,11 @@ __global__ void __launch_bounds__(RBF_THREADS) k_rbf_tile_reg(const double* __re
     }
 }
 
+template <int KIND>
 inline int launch_rbf(const double* X, const double* Zs, const double* ls, const double* os, int R, int M, int D,
                       int x_scaled, double* out, long ldo, int Rp, int Mp, double jitter, cudaStream_t st) {
     dim3 grid((unsigned)cdiv(Mp, RBF_TC), (unsigned)cdiv(Rp, RBF_TR));
-#define TGP_RBF(MD) k_rbf_tile_reg<MD><<<grid, RBF_THREADS, 0, st>>>(X, Zs, ls, os, R, M, D, x_scaled, out, ldo, Rp, Mp, jitter)
+#define TGP_RBF(MD) k_rbf_tile_reg<MD, KIND><<<grid, RBF_THREADS, 0, st>>>(X, Zs, ls, os, R, M, D, x_scaled, out, ldo, Rp, Mp, jitter)
     if (D <= 4) { TGP_RBF(4); return check_launch("k_rbf_tile_reg"); }
     if (D <= 8) { TGP_RBF(8); return check_launch("k_rbf_tile_reg"); }
     if (D <= 16) { TGP_RBF(16); return check_launch("k_rbf_tile_reg"); }
@@ -120,8 +122,8 @@ inline int launch_rbf(const double* X, const double* Zs, const double* ls, const
     const size_t smem = (size_t)(RBF_TR + RBF_TC) * (D + 1) * sizeof(double);
     if (smem > 200 * 1024) return set_error(-2, "input dimension too large for the RBF tile kernel");
     if (smem > 48 * 1024)       // generic kernel for D > 64 only: set per call (per-device attribute, rare path)
-        cudaFuncSetAttribute(k_rbf_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_rbf_tile<<<grid, RBF_THREADS, smem, st>>>(X, Zs, ls, os, R, M, D, x_scaled, out, ldo, Rp, Mp, jitter);
+        cudaFuncSetAttribute(k_rbf_tile<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    k_rbf_tile<KIND><<<grid, RBF_THREADS, smem, st>>>(X, Zs, ls, os, R, M, D, x_scaled, out, ldo, Rp, Mp, jitter);
     return check_launch("k_rbf_tile");
 }
 
@@ -279,6 +281,7 @@ __global__ void k_halve_diag(double* __restrict__ P, long ld, int M) {
 
 struct StepView {       // carved views into the per-step workspace (all doubles)
     int M, Mp, D;
+    int kind;           // TGP_KERNEL_* of the model (not part of the layout)
     double *ls, *os, *Zs, *kl3, *Dinv, *mvec;
     double *Kzz, *L, *Linv, *LS, *Cm, *S0, *S1, *S2, *S3;
 };
@@ -293,7 +296,7 @@ inline int pad_M(int M) {
 // run_prepare zeroes L and Linv with one memset, and the region ends on a 256-byte boundary.
 inline StepView step_view(Carve& c, int M, int D) {
     StepView v;
-    v.M = M; v.D = D; v.Mp = pad_M(M);
+    v.M = M; v.D = D; v.Mp = pad_M(M); v.kind = TGP_KERNEL_RBF;
     const size_t mm = (size_t)v.Mp * v.Mp;
     v.ls = c.take<double>(D);
     v.os = c.take<double>(1);
@@ -331,7 +334,9 @@ inline int run_prepare(const StepView& v, const double* Z, const double* raw_ls,
     // everything above stays on the caller's stream (kl_out is an output in stream order); the factorisation proper forks
     // onto the high-priority stream `fst` when the caller passed one (tgp_prepare), see common.cuh
     st = fst ? fst : st;
-    TGP_TRY(launch_rbf(v.Zs, v.Zs, v.ls, v.os, M, M, D, 1, v.Kzz, Mp, Mp, Mp, jitter, st));
+    TGP_TRY(with_kernel(v.kind, [&](auto k) {
+        return launch_rbf<decltype(k)::value>(v.Zs, v.Zs, v.ls, v.os, M, M, D, 1, v.Kzz, Mp, Mp, Mp, jitter, st);
+    }));
 
     // right-looking blocked Cholesky; the panel solve is a GEMM with the inverted diagonal block
     for (int kb = 0; kb < nb; ++kb) {

@@ -11,6 +11,10 @@ namespace tc {
 constexpr long TC_ROW_CHUNK = 16384;
 extern int g_fused_forward;      // 1: forward = ONE kernel (K tiles generated inside the tcgen05 contraction); 0: staged planes
 
+// The fused forward generates RBF tiles only (D <= FUSED_MAX_D): other models take the staged path under either option.  The
+// backward asks the same question to know whether the forward left K planes behind.
+inline bool fused_forward(const StepView& s) { return g_fused_forward && s.D <= FUSED_MAX_D && s.kind == TGP_KERNEL_RBF; }
+
 struct StepPlanes { float *Whi, *Wlo, *Wthi, *Wtlo; double* u; long ldk, ld2m; };      // u = L^-T m (FP64, M)
 struct BatchPlanes {
     float *AB;                       // (R x ld2m) saved forward -> backward
@@ -68,7 +72,7 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes
                       cudaStream_t st) {
     const int M = s.M, D = s.D;
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
-    if (g_fused_forward && D <= FUSED_MAX_D) {
+    if (fused_forward(s)) {
         FusedFwdParams fp;
         fp.X = X; fp.Zs = s.Zs; fp.ls = s.ls; fp.os = s.os; fp.mvec = s.mvec;
         fp.R = (int)R; fp.M = M; fp.D = D; fp.AB = b.AB; fp.ldab = b.ld2m; fp.mu = mu; fp.v = v; fp.u = sp.u;
@@ -77,28 +81,32 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes
     }
     // mu = K_xz (L^-T m) is accumulated in FP64 by the K generation
     cudaMemsetAsync(mu, 0, (size_t)R * sizeof(double), st);
-    for (long r0 = 0; r0 < R; r0 += b.Rc) {
-        const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        const long kt_off = (r0 / b.Rc) * (long)M * b.ldt;
-        float *Khi = b.Khi + r0 * b.ldk, *Klo = b.Klo + r0 * b.ldk;
-        TGP_TRY(launch_rbf_planes(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, Khi, Klo, b.ldk, b.KThi + kt_off, b.KTlo + kt_off,
-                                  b.ldt, st, sp.u, mu + r0));
-        Params p{};
-        p.Mrows = rc; p.Ncols = 2 * M; p.K = M;
-        p.tri_mode = 1; p.tri_rows = M;
-        p.out_mode = 0; p.lower_rows = 0; p.Cf = b.AB + r0 * b.ld2m; p.Cd = nullptr; p.ldc = b.ld2m; p.splitk = 1;
-        Operand A{Khi, Klo, rc, M, b.ldk};
-        Operand B{sp.Whi, sp.Wlo, 2L * M, M, sp.ldk};
-        TGP_TRY(gemm_tf32x3(A, B, p, st));
-    }
+    TGP_TRY(with_kernel(s.kind, [&](auto k) {
+        for (long r0 = 0; r0 < R; r0 += b.Rc) {
+            const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
+            const long kt_off = (r0 / b.Rc) * (long)M * b.ldt;
+            float *Khi = b.Khi + r0 * b.ldk, *Klo = b.Klo + r0 * b.ldk;
+            TGP_TRY(launch_rbf_planes<decltype(k)::value>(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, Khi, Klo, b.ldk, b.KThi + kt_off,
+                                                          b.KTlo + kt_off, b.ldt, st, sp.u, mu + r0));
+            Params p{};
+            p.Mrows = rc; p.Ncols = 2 * M; p.K = M;
+            p.tri_mode = 1; p.tri_rows = M;
+            p.out_mode = 0; p.lower_rows = 0; p.Cf = b.AB + r0 * b.ld2m; p.Cd = nullptr; p.ldc = b.ld2m; p.splitk = 1;
+            Operand A{Khi, Klo, rc, M, b.ldk};
+            Operand B{sp.Whi, sp.Wlo, 2L * M, M, sp.ldk};
+            TGP_TRY(gemm_tf32x3(A, B, p, st));
+        }
+        return 0;
+    }));
     k_row_stats_f32<<<row_grid128(R), 128, 0, st>>>(b.AB, b.ld2m, s.mvec, s.os, (int)R, M, nullptr, v);
     return check_launch("k_row_stats_f32");
 }
 
 // backward: ABbar planes (+transposes), K^T planes; Kbar = ABbar Wt^T; kernel gradients; Gbar / Cbar += ABbar^T K
-inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
-                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
-                       cudaStream_t st) {
+template <int KIND>
+inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
+                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                         cudaStream_t st) {
     const int M = s.M, D = s.D;
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
@@ -110,8 +118,8 @@ inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlane
         }
         const long kt_off = (r0 / b.Rc) * (long)M * b.ldt;          // K^T planes of this chunk, kept by the forward
         float *KThi = b.KThi + kt_off, *KTlo = b.KTlo + kt_off;
-        if (g_fused_forward && D <= FUSED_MAX_D)                     // the fused forward never wrote K: generate it here
-            TGP_TRY(launch_rbf_planes(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk, KThi,
+        if (fused_forward(s))                                        // the fused forward never wrote K: generate it here
+            TGP_TRY(launch_rbf_planes<KIND>(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk, KThi,
                                       KTlo, b.ldt, st));
         {   // Kbar (rc x M) = ABbar (rc x 2M) * Wt (M x 2M)^T ; for k < M only k >= n contributes
             Params p{};
@@ -122,8 +130,9 @@ inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlane
             Operand B{sp.Wthi, sp.Wtlo, M, 2L * M, sp.ld2m};
             TGP_TRY(gemm_tf32x3(A, B, p, st));
         }
-        TGP_TRY(launch_kernel_grads<float>(b.Kbar, b.ldk, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st,
-                                           nullptr, 0, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk));
+        // the RBF reads K from the planes; the other kinds recompute it (launch_kernel_grads)
+        TGP_TRY((launch_kernel_grads<KIND, float>(b.Kbar, b.ldk, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st,
+                                                  nullptr, 0, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk)));
         const int kblocks = (rc + BK - 1) / BK;
         int split = (int)cdiv(2 * 148, cdiv(M, BM) * cdiv(M, BN));
         if (split > kblocks / 8) split = kblocks / 8 > 0 ? kblocks / 8 : 1;
@@ -145,6 +154,14 @@ inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlane
         }
     }
     return 0;
+}
+
+inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
+                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                       cudaStream_t st) {
+    return with_kernel(s.kind, [&](auto k) {
+        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+    });
 }
 
 }  // namespace tc

@@ -183,9 +183,7 @@ fwd_fused_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_constant
                         for (int e = 0; e < 8; ++e) {
                             float val = 0.f;
                             if (row < p.R && k + c0 + e < M) {
-                                const double arg = -0.5 * fmax(acc[e], 0.0);
-                                const float ahi = (float)arg;
-                                val = sf * expf(ahi) * (1.0f + (float)(arg - (double)ahi));
+                                val = Cov<TGP_KERNEL_RBF>::kf(fmax(acc[e], 0.0), sf);
                                 if (take_mu) mu_acc = fma((double)val, __ldg(p.u + k + c0 + e), mu_acc);
                             }
                             hi[e] = tf32_hi(val);

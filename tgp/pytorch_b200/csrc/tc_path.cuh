@@ -30,9 +30,10 @@ __device__ __forceinline__ void put_planes(float* __restrict__ hi, float* __rest
 
 inline long pad4(long x) { return (x + 3) / 4 * 4; }
 
-// K tile in FP64 arithmetic (same formula as k_rbf_tile), written as FP32 planes: row-major (rows x ldk) and/or
+// K tile (distance in FP64, as k_rbf_tile; exponential in FP32: Cov<KIND>::kf, common.cuh), written as FP32 planes: row-major (rows x ldk) and/or
 // transposed (M x ldt).  32 x 64 tile per CTA staged through shared memory so that both writes are coalesced.
 constexpr int RP_TR = 32, RP_TC = 64, RP_THREADS = 256;
+template <int KIND>
 // If u != NULL (u = L^-T m, FP64, one per step) the marginal mean is accumulated here as well: mu[n] += sum_j K[n,j] u[j] in FP64 —
 // the reference's own evaluation order mu = K_xz (L^-T m) (sparse_MF_SP.py:354-355).  Taking mu from the FP32 rows a = L^-1 k
 // instead lets the conditioning of L^-1 amplify the FP32 rounding of a (measured at cfg4: max |dmu| 3.3e-4 against 2.3e-5, ELBO
@@ -67,9 +68,7 @@ __global__ void __launch_bounds__(RP_THREADS) k_rbf_planes(const double* __restr
             double acc = 0.0;
             for (int d = 0; d < D; ++d) { const double df = xs[r * DP + d] - zs[c * DP + d]; acc = fma(df, df, acc); }
             // argument in FP64 (exact to ~1e-16), exponential in FP32: exp(a) = expf(a_hi) * (1 + a_lo)
-            const double arg = -0.5 * acc;
-            const float ahi = (float)arg;
-            val = (float)s * expf(ahi) * (1.0f + (float)(arg - (double)ahi));
+            val = Cov<KIND>::kf(acc, (float)s);
         }
         tile[r * (RP_TC + 1) + c] = val;
         if (Khi && n < R && j < M) { put_planes(Khi, Klo, (long)n * ldk + j, val); }
@@ -91,13 +90,14 @@ __global__ void __launch_bounds__(RP_THREADS) k_rbf_planes(const double* __restr
     }
 }
 
+template <int KIND>
 inline int launch_rbf_planes(const double* X, const double* Zs, const double* ls, const double* os, int R, int M, int D,
                              float* Khi, float* Klo, long ldk, float* KThi, float* KTlo, long ldt, cudaStream_t st,
                              const double* u = nullptr, double* mu = nullptr) {
     const size_t smem = (size_t)(RP_TR + RP_TC) * (D + 1) * sizeof(double) + (size_t)RP_TR * (RP_TC + 1) * sizeof(float);
     if (smem > 48 * 1024) return set_error(-2, "input dimension too large for the plane-generating RBF kernel");
     dim3 grid((unsigned)cdiv(M, RP_TC), (unsigned)cdiv(R, RP_TR));
-    k_rbf_planes<<<grid, RP_THREADS, smem, st>>>(X, Zs, ls, os, R, M, D, Khi, Klo, ldk, KThi, KTlo, ldt, u, mu);
+    k_rbf_planes<KIND><<<grid, RP_THREADS, smem, st>>>(X, Zs, ls, os, R, M, D, Khi, Klo, ldk, KThi, KTlo, ldt, u, mu);
     return check_launch("k_rbf_planes");
 }
 

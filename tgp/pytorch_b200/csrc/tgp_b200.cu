@@ -68,6 +68,8 @@ inline int validate(const TgpModel* md) {
     if (md->dtype != TGP_F64 && md->dtype != TGP_F32 && md->dtype != TGP_F64_I8)
         return set_error(-1, "dtype must be TGP_F64, TGP_F32 or TGP_F64_I8");
     if (md->M < 1 || md->D < 1) return set_error(-1, "M and D must be positive");
+    if (!kernel_kind_valid(md->kernel))
+        return set_error(-1, "kernel must be TGP_KERNEL_RBF, TGP_KERNEL_MATERN12, TGP_KERNEL_MATERN32 or TGP_KERNEL_MATERN52");
     if (md->n_layers < 0 || md->n_layers > TGP_MAX_LAYERS) return set_error(-1, "too many flow layers");
     if (md->n_theta < 0 || md->n_theta > MAX_THETA) return set_error(-1, "too many global flow parameters");
     if (md->n_rowparams < 0 || md->n_rowparams > MAX_ROWP) return set_error(-1, "too many per-row flow parameters");
@@ -122,6 +124,7 @@ struct StepWorkspace { StepView f64; tc::StepPlanes tc; crt::StepPlanes crt; };
 inline StepWorkspace step_layout(Carve& c, const TgpModel* md) {
     StepWorkspace w{};
     w.f64 = step_view(c, md->M, md->D);
+    w.f64.kind = md->kernel;
     if (md->dtype == TGP_F32) w.tc = tc::step_planes(c, md->M);
     if (md->dtype == TGP_F64_I8) w.crt = crt::step_planes(c, md->M);
     return w;
@@ -337,7 +340,9 @@ int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, co
     double* dos_acc = dls_acc + even(D);
     cudaMemcpyAsync(dls_acc, reduce_buf + l.dls, (size_t)D * sizeof(double), cudaMemcpyDeviceToDevice, st);
     cudaMemcpyAsync(dos_acc, reduce_buf + l.dos, sizeof(double), cudaMemcpyDeviceToDevice, st);
-    TGP_TRY(launch_kernel_grads(s.S2, Mp, s.Zs, 1, s.Zs, s.ls, s.os, M, M, D, 1, 2.0, dZacc, dls_acc, dos_acc, st));
+    TGP_TRY(with_kernel(s.kind, [&](auto k) {
+        return launch_kernel_grads<decltype(k)::value>(s.S2, Mp, s.Zs, 1, s.Zs, s.ls, s.os, M, M, D, 1, 2.0, dZacc, dls_acc, dos_acc, st);
+    }));
     {
         const int n = M * D > M ? M * D : M;
         const int nn = n > md->n_theta ? n : md->n_theta;

@@ -1,5 +1,5 @@
-"""ARD-RBF and scale kernels carrying the parameter names the reference's gpytorch objects expose
-(`raw_lengthscale` (Dy,1,D), `raw_outputscale` (Dy,), `base_kernel`, `batch_shape`).
+"""ARD-RBF, ARD-Matern and scale kernels carrying the parameter names the reference's gpytorch objects expose
+(`raw_lengthscale` (Dy,1,D), `raw_outputscale` (Dy,), `base_kernel`, `batch_shape`, and `nu` for the Matern kernel).
 
 On the hot path only the *parameters* of these modules are read (the fused kernels regenerate K tiles from X, Z and
 the raw parameters).  `__call__` exists for API parity (`kernel(x1, x2, diag=...)` with `.evaluate()` on non-diag
@@ -51,6 +51,41 @@ class RBFKernel(Kernel):
             return torch.exp(-0.5 * (a - b).pow(2).sum(-1))
         d2 = (a.unsqueeze(-2) - b.unsqueeze(-3)).pow(2).sum(-1)
         return torch.exp(-0.5 * d2)
+
+
+class MaternKernel(Kernel):
+    """gpytorch's MaternKernel for nu in {0.5, 1.5, 2.5}.  r = ||(x1 - x2) / lengthscale|| by direct differences (gpytorch
+    uses an expanded quadratic form, whose rounding leaves r ~ 1e-8 ||x|| where x1 == x2)."""
+    NUS = (0.5, 1.5, 2.5)
+
+    def __init__(self, nu=2.5, ard_num_dims=None, batch_shape=torch.Size([])):
+        super().__init__(batch_shape)
+        if nu not in self.NUS:
+            raise ValueError('nu must be one of 0.5, 1.5, 2.5, got {}'.format(nu))
+        self.nu = float(nu)
+        self.ard_num_dims = ard_num_dims
+        self.raw_lengthscale = nn.Parameter(torch.zeros(*batch_shape, 1, 1 if ard_num_dims is None else ard_num_dims))
+
+    @property
+    def lengthscale(self):
+        return F.softplus(self.raw_lengthscale)
+
+    def forward(self, x1, x2, diag=False):
+        a, b = x1 / self.lengthscale, x2 / self.lengthscale
+        d2 = (a - b).pow(2).sum(-1) if diag else (a.unsqueeze(-2) - b.unsqueeze(-3)).pow(2).sum(-1)
+        return matern_phi(d2, self.nu)
+
+
+def matern_phi(d2, nu):
+    """phi_nu(r) with r = sqrt(d2); pairs with d2 <= 1e-30 take r = 0 (and no gradient)."""
+    r = torch.where(d2 > 1e-30, d2.clamp_min(1e-30).sqrt(), torch.zeros_like(d2))
+    if nu == 0.5:
+        return torch.exp(-r)
+    if nu == 1.5:
+        a = r * 3.0 ** 0.5
+        return (1.0 + a) * torch.exp(-a)
+    a = r * 5.0 ** 0.5
+    return (1.0 + a + a * a / 3.0) * torch.exp(-a)
 
 
 class ScaleKernel(Kernel):

@@ -2,7 +2,7 @@
 
 Re-exports the names the reference's `code/main.py:26-37` imports from `dsp.models`:
 
-* `instance_kernel`  — factory of the (Scale)RBF-ARD kernel parameter holders,
+* `instance_kernel`  — factory of the (Scale)RBF-ARD and (Scale)Matern-ARD kernel parameter holders,
 * `sparse_MF_SP`     — sparse variational transformed GP (TGP / ID_TGP) whose ELBO, marginals and test log-likelihood run
                        in the sm_100a kernels of libtgp_b200.so,
 * `sparse_MF_GP`     — SVGP, the same model with identity flows,

@@ -5,8 +5,8 @@ Same constructor, attributes and method signatures as the reference class (:47-1
 `test_log_likelihood` is enqueued on the B200 through libtgp_b200.so (tgp/pytorch_b200/functional.py); this file only
 gathers parameters from the unchanged nn.Module tree and shapes the results like the reference does.
 
-Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened q(u), zero mean, (Scale)RBF-ARD
-kernel, diagonal marginals, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
+Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened q(u), zero mean, (Scale)RBF-ARD or
+(Scale)Matern-ARD (nu = 1/2, 3/2, 5/2) kernel, diagonal marginals, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
 layers (optionally input-dependent with MC-dropout MLPs).  Multi-output models loop over outputs.
 """
 import numpy
@@ -17,7 +17,7 @@ import torch.distributions as td
 from .. import config as cg
 from ... import functional as Fn
 from ...engine import Engine, FlowLayout
-from ..kernels import CholeskyVariationalDistribution, ScaleKernel, RBFKernel
+from ..kernels import CholeskyVariationalDistribution, ScaleKernel, RBFKernel, MaternKernel
 from ..likelihoods.GaussianLinearMean import GaussianLinearMean
 from ..likelihoods.GaussianNonLinearMean import GaussianNonLinearMean
 from ..likelihoods.Bernoulli import Bernoulli
@@ -29,7 +29,8 @@ from .flow import instance_flow
 from .utils_models import return_mean, enable_eval_dropout
 
 _LIK_KIND = {GaussianLinearMean: 'gauss_linear', GaussianNonLinearMean: 'gauss_nonlinear', Bernoulli: 'bernoulli'}
-_INV_SOFTPLUS_ONE = 0.5413248546129181       # softplus^-1(1): outputscale of a bare RBF kernel
+_INV_SOFTPLUS_ONE = 0.5413248546129181       # softplus^-1(1): outputscale of a bare (unscaled) kernel
+_MATERN_KIND = {0.5: 'matern12', 1.5: 'matern32', 2.5: 'matern52'}
 
 
 class sparse_MF_SP(nn.Module):
@@ -116,9 +117,16 @@ class sparse_MF_SP(nn.Module):
         if cg.strict_flag:
             want = torch.Size([1]) if self.kernel_is_shared else torch.Size([self.out_dim])
             assert kernel.batch_shape == want, 'Got a kernel with batch_shape {}, expected {}'.format(kernel.batch_shape, want)
-        if not isinstance(kernel, (ScaleKernel, RBFKernel)):
-            raise NotImplementedError('the fused path covers (Scale)RBF-ARD kernels')
+        base = kernel.base_kernel if isinstance(kernel, ScaleKernel) else kernel
+        if not isinstance(base, (RBFKernel, MaternKernel)):
+            raise NotImplementedError('the fused path covers (Scale)RBF-ARD and (Scale)Matern-ARD kernels')
         self.covariance_function = kernel
+
+    def _kernel_kind(self):
+        """Engine kernel name of the covariance function ('rbf', 'matern12', 'matern32', 'matern52')."""
+        kern = self.covariance_function
+        base = kern.base_kernel if isinstance(kern, ScaleKernel) else kern
+        return _MATERN_KIND[base.nu] if isinstance(base, MaternKernel) else 'rbf'
 
     def initialize_flows(self, flow_connection, flow_specs):
         if flow_connection == 'shared':
@@ -170,10 +178,11 @@ class sparse_MF_SP(nn.Module):
 
     def _engine(self, dy, layout, device):
         kind = _LIK_KIND[type(self.likelihood)]
-        key = (dy, kind, self.quad_points, tuple(tuple(sorted(l.items())) for l in layout.layers), str(device), self._compute())
+        key = (dy, kind, self.quad_points, tuple(tuple(sorted(l.items())) for l in layout.layers), str(device), self._compute(),
+               self._kernel_kind())
         if key not in self._engines:
             self._engines[key] = Engine(self.M, self.inp_dim, kind, self.quad_points if kind != 'gauss_linear' else 0,
-                                        layout, device, compute=self._compute())
+                                        layout, device, compute=self._compute(), kernel=self._kernel_kind())
         return self._engines[key]
 
     def _compute(self):
@@ -210,10 +219,10 @@ class sparse_MF_SP(nn.Module):
         mus, vs = [], []
         for dy in range(self.out_dim):
             Z, raw_ls, raw_os, m, L_raw = self._gp_params(dy)
-            key = ('qf', dy, str(X.device), self._compute())
+            key = ('qf', dy, str(X.device), self._compute(), self._kernel_kind())
             if key not in self._engines:     # marginals do not involve the flow / likelihood
                 self._engines[key] = Engine(self.M, self.inp_dim, 'gauss_linear', 0, FlowLayout([]), X.device,
-                                            compute=self._compute())
+                                            compute=self._compute(), kernel=self._kernel_kind())
             eng = self._engines[key]
             if not cg.cache_factorisation_in_eval:
                 eng.prepared_key = None

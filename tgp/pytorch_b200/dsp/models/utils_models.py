@@ -1,9 +1,10 @@
 """Kernel / mean factories and the MC-dropout switch (reference code/dsp/models/utils_models.py:145-193, 285-294,
-358-364).  Only the kernels reachable from the reference's main.py are built: 'scale_rbf' and 'rbf'."""
+358-364).  Kernels: 'scale_rbf' and 'rbf' (what the reference's main.py builds), and 'scale_matern' / 'matern' with
+init_params['nu'] in {0.5, 1.5, 2.5} (default 2.5, gpytorch's default)."""
 import torch
 
 from .. import config as cg
-from ..kernels import RBFKernel, ScaleKernel, ZeroMean
+from ..kernels import MaternKernel, RBFKernel, ScaleKernel, ZeroMean
 from ..utils import inv_softplus
 
 
@@ -15,16 +16,19 @@ def instance_kernel(name, ard_num_dim, num_multioutput, kernel_is_shared, init_p
     if kernel_is_shared:
         num_multioutput = 1
     batch = torch.Size([num_multioutput])
-    if name in ('rbf', 'scale_rbf'):
-        rbf = RBFKernel(ard_num_dims=ard_num_dim, batch_shape=batch)
-        rbf.raw_lengthscale.data = inv_softplus(torch.ones(num_multioutput, 1, rbf.raw_lengthscale.size(-1), dtype=cg.dtype) * ls)
-        if name == 'rbf':
-            return rbf
-        K = ScaleKernel(rbf, batch_shape=batch)
+    if name in ('rbf', 'scale_rbf', 'matern', 'scale_matern'):
+        if name in ('rbf', 'scale_rbf'):
+            base = RBFKernel(ard_num_dims=ard_num_dim, batch_shape=batch)
+        else:
+            base = MaternKernel(nu=init_params.get('nu', 2.5), ard_num_dims=ard_num_dim, batch_shape=batch)
+        base.raw_lengthscale.data = inv_softplus(torch.ones(num_multioutput, 1, base.raw_lengthscale.size(-1), dtype=cg.dtype) * ls)
+        if not name.startswith('scale_'):
+            return base
+        K = ScaleKernel(base, batch_shape=batch)
         K.raw_outputscale.data = inv_softplus(torch.ones(num_multioutput, dtype=cg.dtype) * ks)
         return K
-    raise NotImplementedError("kernel %r is outside the fused hot-path scope (the reference's main.py builds 'scale_rbf' "
-                              "only, main.py:229)" % (name,))
+    raise NotImplementedError("kernel %r is outside the fused hot-path scope ('rbf', 'scale_rbf', 'matern', "
+                              "'scale_matern')" % (name,))
 
 
 def return_mean(name, input_dim, output_dim, W):

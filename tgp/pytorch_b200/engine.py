@@ -115,8 +115,13 @@ def _chk(t, name, shape=None):
         raise ValueError('%s has shape %s, expected %s' % (name, tuple(t.shape), tuple(shape)))
 
 
+# covariance function of the engine -> TgpModel.kernel
+KERNELS = {'rbf': _lib.KERNEL_RBF, 'matern12': _lib.KERNEL_MATERN12, 'matern32': _lib.KERNEL_MATERN32,
+           'matern52': _lib.KERNEL_MATERN52}
+
+
 class Engine:
-    def __init__(self, M, D, likelihood, n_quad, flow_layout, device, compute='f64'):
+    def __init__(self, M, D, likelihood, n_quad, flow_layout, device, compute='f64', kernel='rbf'):
         self.lib = _lib.load()
         self.device = torch.device(device)
         if self.device.type != 'cuda':
@@ -132,6 +137,10 @@ class Engine:
         self.compute = compute
         self.model.dtype = {'f64': _lib.TGP_F64, 'tf32x3': _lib.TGP_F32, 'i8crt': _lib.TGP_F64_I8}[compute]
         self.model.M, self.model.D = self.M, self.D
+        if kernel not in KERNELS:
+            raise ValueError('kernel must be one of %s' % (', '.join(repr(k) for k in KERNELS),))
+        self.kernel = kernel
+        self.model.kernel = KERNELS[kernel]
         self.model.likelihood = _LIK[likelihood]
         self.model.n_quad = int(n_quad)
         flow_layout.fill(self.model)
