@@ -116,6 +116,26 @@ int tgp_factor_status(int* status_out);
 int tgp_qf_forward(const TgpModel* model, const void* step_ws, void* batch_ws, const void* X, long R, void* mu,
                    void* v, void* stream);
 
+/* ---- full covariance of q(f) over a test batch and joint samples (evaluation only, no backward) ---------------------
+ * tgp_qf_cov_forward: mu (R) and Sigma = s Phi(X, X) - A A^T + B B^T (R x R, row-major, ld ldc >= R, exactly symmetric) of
+ * R rows, A = K_xz L^-T, B = A L_S: the non-diagonal form of sparse_MF_SP.py:376-382.  Reads a step workspace prepared by
+ * tgp_prepare in any compute mode and does not touch the batch workspace, so it may run between an ELBO forward and its
+ * backward.  FP64 DMMA in every mode.  cov_ws: tgp_qf_cov_workspace_bytes(model, R) bytes, about (3M + 1) R doubles. */
+size_t tgp_qf_cov_workspace_bytes(const TgpModel* model, long R);
+int tgp_qf_cov_forward(const TgpModel* model, const void* step_ws, void* cov_ws, const void* X, long R, void* mu, void* cov,
+                       long ldc, void* stream);
+
+/* L (R x R, ld ldl, lower triangular, upper triangle exactly 0) = chol(cov + jitter I) with the blocked factorisation of
+ * tgp_prepare; only the lower triangle of cov is read.  status (device): 0, or the 1-based index of the first pivot that is
+ * not above 8 eps * scale_dev[0] (a device scalar, e.g. the outputscale).  chol_ws: tgp_cov_cholesky_workspace_bytes(R)
+ * bytes (two Rp x Rp matrices, Rp = R rounded up to 64). */
+size_t tgp_cov_cholesky_workspace_bytes(long R);
+int tgp_cov_cholesky(long R, const void* cov, long ldc, double jitter, const double* scale_dev, void* chol_ws, void* L, long ldl,
+                     int* status, void* stream);
+
+/* out (S x R, row-major) = mu + eps L^T for eps (S x R) drawn by the caller: S joint samples from N(mu, L L^T). */
+int tgp_cov_sample(long R, int S, const void* mu, const void* L, long ldl, const void* eps, void* out, void* stream);
+
 /* Expected log-likelihood of R rows given (mu, v): flow o Gauss-Hermite o likelihood, with analytic gradients.
  * Replaces likelihood.expected_log_prob (GaussianNonLinearMean.py:113-150, GaussianLinearMean.py:60-87,
  * Bernoulli.py:50-95) and sparse_MF_SP.ELL's N/MB scaling (sparse_MF_SP.py:601-626; `scale` = N/MB_global).

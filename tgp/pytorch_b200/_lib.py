@@ -75,6 +75,11 @@ SIGNATURES = {
     'tgp_prepare': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _D, _P, _P, _P, _P]),
     'tgp_factor_status': (_I, [C.POINTER(C.c_int)]),
     'tgp_qf_forward': (_I, [C.POINTER(TgpModel), _P, _P, _P, _L, _P, _P, _P]),
+    'tgp_qf_cov_workspace_bytes': (C.c_size_t, [C.POINTER(TgpModel), _L]),
+    'tgp_qf_cov_forward': (_I, [C.POINTER(TgpModel), _P, _P, _P, _L, _P, _P, _L, _P]),
+    'tgp_cov_cholesky_workspace_bytes': (C.c_size_t, [_L]),
+    'tgp_cov_cholesky': (_I, [_L, _P, _L, _D, _P, _P, _P, _L, _P, _P]),
+    'tgp_cov_sample': (_I, [_L, _I, _P, _P, _L, _P, _P, _P]),
     'tgp_ell_forward': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _D, _P, _P, _I, _P, _P, _P,
                              _P, _P, _P]),
     'tgp_qf_backward': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _L, _P, _P, _P, _P]),

@@ -41,6 +41,22 @@ inline int weight_splitk(int M, int rc, bool lower) {
     return best;
 }
 
+// [A | B] of rc rows (ld 2M) from their K_xz (ld M): the two triangular contractions of the forward.  Also the first stage
+// of the full covariance over a test batch (cov_kernels.cuh), in every compute mode.
+inline int ab_rows(const StepView& s, const double* K, int rc, double* AB, cudaStream_t st) {
+    const int M = s.M;
+    // A = K L^-T   (Bop[n,k] = Linv[n,k], nonzero k <= n)
+    GemmArgs ga = make_gemm(rc, M, M, K, M, 0, s.Linv, s.Mp, 0, AB, 2 * M);
+    ga.b_tri = 1;
+    ga.tag = 1;
+    TGP_TRY(gemm_f64(ga, st));
+    // B = A L_S   (Bop[n,k] = L_S[k,n], nonzero k >= n) — the reference's two-contraction form, both triangular
+    GemmArgs gb = make_gemm(rc, M, M, AB, 2 * M, 0, s.LS, s.Mp, 1, AB + M, 2 * M);
+    gb.b_tri = 2;
+    gb.tag = 1;
+    return gemm_f64(gb, st);
+}
+
 // forward: K_xz per chunk -> A = K L^-T, B = A L_S -> row statistics
 inline int qf_forward(const StepView& s, const BatchView& b, const double* X, long R, double* mu, double* v, cudaStream_t st) {
     const int M = s.M, D = s.D;
@@ -56,17 +72,7 @@ inline int qf_forward(const StepView& s, const BatchView& b, const double* X, lo
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
-        double* Kc = b.Kbuf + r0 * M;
-        // A = K L^-T   (Bop[n,k] = Linv[n,k], nonzero k <= n)
-        GemmArgs ga = make_gemm(rc, M, M, Kc, M, 0, s.Linv, s.Mp, 0, b.AB + r0 * 2 * M, 2 * M);
-        ga.b_tri = 1;
-        ga.tag = 1;
-        TGP_TRY(gemm_f64(ga, st));
-        // B = A L_S   (Bop[n,k] = L_S[k,n], nonzero k >= n) — the reference's two-contraction form, both triangular
-        GemmArgs gb = make_gemm(rc, M, M, b.AB + r0 * 2 * M, 2 * M, 0, s.LS, s.Mp, 1, b.AB + r0 * 2 * M + M, 2 * M);
-        gb.b_tri = 2;
-        gb.tag = 1;
-        TGP_TRY(gemm_f64(gb, st));
+        TGP_TRY(ab_rows(s, b.Kbuf + r0 * M, rc, b.AB + r0 * 2 * M, st));
     }
     k_row_stats<<<row_grid(R), ROW_THREADS, 0, st>>>(b.AB, s.mvec, s.os, (int)R, M, mu, v);
     return check_launch("k_row_stats");

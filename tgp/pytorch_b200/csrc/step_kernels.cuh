@@ -310,14 +310,38 @@ inline StepView step_view(Carve& c, int M, int D) {
     return v;
 }
 
+// Right-looking blocked Cholesky of the Np x Np lower triangle of Aw (Np a multiple of POTRF_NB, ld = Np); the panel solve
+// is a GEMM with the inverted diagonal block.  L -> L (its upper triangle must hold zeros already), the diagonal blocks of
+// L^-1 -> Linv (same ld; only block (kb, kb) of Linv + kb (NB ld + NB) is written), Dinv: POTRF_NB^2 scratch.  Aw's
+// trailing blocks are overwritten.  status: first pivot not above 8 eps * scale[0] (tgp_prepare's meaning).
+inline int blocked_cholesky(double* Aw, double* L, double* Linv, double* Dinv, int Np, const double* scale, int* status,
+                            cudaStream_t st) {
+    const int NB = POTRF_NB, nb = Np / NB;
+    static PerDeviceOnce potrf_once;
+    if (potrf_once.first()) cudaFuncSetAttribute(k_potrf_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF_SMEM);
+    for (int kb = 0; kb < nb; ++kb) {
+        k_potrf_diag<<<1, POTRF_THREADS, POTRF_SMEM, st>>>(Aw, L, Linv, Dinv, kb, Np, scale, status);
+        TGP_TRY(check_launch("k_potrf_diag"));
+        const int rem = Np - (kb + 1) * NB;
+        if (rem <= 0) break;
+        const long off_panel = (long)(kb + 1) * NB * Np + (long)kb * NB;
+        GemmArgs p = make_gemm(rem, NB, NB, Aw + off_panel, Np, 0, Dinv, NB, 0, L + off_panel, Np);
+        p.b_tri = 1;
+        TGP_TRY(gemm_f64(p, st));
+        const long off_trail = (long)(kb + 1) * NB * Np + (long)(kb + 1) * NB;
+        GemmArgs t = make_gemm(rem, rem, NB, L + off_panel, Np, 0, L + off_panel, Np, 0, Aw + off_trail, Np, -1.0, 1.0);
+        t.c_lower = 1;
+        TGP_TRY(gemm_f64(t, st));
+    }
+    return 0;
+}
+
 // K_zz (+jitter) -> L, L^-1 (explicit), C = L_S^T L^-1, KL.  Everything stays on `st`; no host sync.
 inline int run_prepare(const StepView& v, const double* Z, const double* raw_ls, const double* raw_os,
                        const double* m, const double* Lraw, double jitter, double* kl_out, int* status,
                        bool need_C, cudaStream_t st, cudaStream_t (*fork)(cudaStream_t) = nullptr) {
-    const int M = v.M, Mp = v.Mp, D = v.D, NB = POTRF_NB, nb = Mp / NB;
+    const int M = v.M, Mp = v.Mp, D = v.D, NB = POTRF_NB;
     const size_t mm = (size_t)Mp * Mp;
-    static PerDeviceOnce potrf_once;
-    if (potrf_once.first()) cudaFuncSetAttribute(k_potrf_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF_SMEM);
     cudaMemsetAsync(status, 0, sizeof(int), st);
     cudaMemsetAsync(v.kl3, 0, 8 * sizeof(double), st);
     cudaMemsetAsync(v.L, 0, 2 * mm * sizeof(double), st);          // L and Linv are contiguous
@@ -338,22 +362,7 @@ inline int run_prepare(const StepView& v, const double* Z, const double* raw_ls,
         return launch_rbf<decltype(k)::value>(v.Zs, v.Zs, v.ls, v.os, M, M, D, 1, v.Kzz, Mp, Mp, Mp, jitter, st);
     }));
 
-    // right-looking blocked Cholesky; the panel solve is a GEMM with the inverted diagonal block
-    for (int kb = 0; kb < nb; ++kb) {
-        k_potrf_diag<<<1, POTRF_THREADS, POTRF_SMEM, st>>>(v.Kzz, v.L, v.Linv, v.Dinv, kb, Mp, v.os, status);
-        TGP_TRY(check_launch("k_potrf_diag"));
-        const int rem = Mp - (kb + 1) * NB;
-        if (rem <= 0) break;
-        const long off_panel = (long)(kb + 1) * NB * Mp + (long)kb * NB;
-        GemmArgs p = make_gemm(rem, NB, NB, v.Kzz + off_panel, Mp, 0, v.Dinv, NB, 0, v.L + off_panel, Mp);
-        p.b_tri = 1;
-        TGP_TRY(gemm_f64(p, st));
-        const long off_trail = (long)(kb + 1) * NB * Mp + (long)(kb + 1) * NB;
-        GemmArgs t = make_gemm(rem, rem, NB, v.L + off_panel, Mp, 0, v.L + off_panel, Mp, 0, v.Kzz + off_trail, Mp,
-                               -1.0, 1.0);
-        t.c_lower = 1;
-        TGP_TRY(gemm_f64(t, st));
-    }
+    TGP_TRY(blocked_cholesky(v.Kzz, v.L, v.Linv, v.Dinv, Mp, v.os, status, st));
     // explicit inverse by recursive doubling: inv([[A,0],[B,C]]) = [[A^-1,0],[-C^-1 B A^-1, C^-1]]
     for (int b = NB; b < Mp; b *= 2) {
         const int batch = Mp / (2 * b);

@@ -7,6 +7,7 @@
 #include "row_kernels.cuh"
 #include "backward_kernels.cuh"
 #include "f64_driver.cuh"
+#include "cov_kernels.cuh"
 #include "tc_driver.cuh"
 #include "flow_mlp.cuh"
 #include "crt_driver.cuh"
@@ -226,6 +227,52 @@ int tgp_qf_forward(const TgpModel* md, const void* step_ws, void* batch_ws, cons
     if (md->dtype == TGP_F64_I8)
         return crt::qf_forward(w.f64, w.crt, crt::batch_view(cb, M, D, R), Xd, R, (double*)mu, (double*)v, st);
     return f64::qf_forward(w.f64, f64::batch_view(cb, M, R), Xd, R, (double*)mu, (double*)v, st);
+}
+
+size_t tgp_qf_cov_workspace_bytes(const TgpModel* md, long R) {
+    if (validate(md) || R < 1) return 0;
+    Carve c(nullptr);
+    cov::cov_view(c, md->M, R);
+    return c.bytes();
+}
+
+// Reads the step workspace only (any compute mode; the batch workspace is not touched), joins the factorisation after
+// enqueuing the K_xz generation
+int tgp_qf_cov_forward(const TgpModel* md, const void* step_ws, void* cov_ws, const void* X, long R, void* mu, void* cov,
+                       long ldc, void* stream) {
+    TGP_TRY(validate(md));
+    if (R < 1) return set_error(-1, "R must be >= 1");
+    if (ldc < R) return set_error(-1, "ldc must be >= R");
+    if (!step_ws || !cov_ws || !X || !mu || !cov) return set_error(-1, "NULL argument to tgp_qf_cov_forward");
+    Carve cs(const_cast<void*>(step_ws)), cw(cov_ws);
+    const StepWorkspace w = step_layout(cs, md);
+    return cov::qf_cov_forward(w.f64, cov::cov_view(cw, md->M, R), (const double*)X, R, (double*)mu, (double*)cov, ldc,
+                               (cudaStream_t)stream);
+}
+
+size_t tgp_cov_cholesky_workspace_bytes(long R) {
+    if (R < 1) return 0;
+    Carve c(nullptr);
+    cov::chol_view(c, R);
+    return c.bytes();
+}
+
+int tgp_cov_cholesky(long R, const void* cov, long ldc, double jitter, const double* scale_dev, void* chol_ws, void* L, long ldl,
+                     int* status, void* stream) {
+    if (R < 1) return set_error(-1, "R must be >= 1");
+    if (ldc < R || ldl < R) return set_error(-1, "ldc and ldl must be >= R");
+    if (!(jitter >= 0.0)) return set_error(-1, "jitter must be >= 0");
+    if (!cov || !scale_dev || !chol_ws || !L || !status) return set_error(-1, "NULL argument to tgp_cov_cholesky");
+    Carve c(chol_ws);
+    return cov::cholesky(cov::chol_view(c, R), R, (const double*)cov, ldc, jitter, scale_dev, (double*)L, ldl, status,
+                         (cudaStream_t)stream);
+}
+
+int tgp_cov_sample(long R, int S, const void* mu, const void* L, long ldl, const void* eps, void* out, void* stream) {
+    if (R < 1 || S < 1) return set_error(-1, "R and S must be >= 1");
+    if (ldl < R) return set_error(-1, "ldl must be >= R");
+    if (!mu || !L || !eps || !out) return set_error(-1, "NULL argument to tgp_cov_sample");
+    return cov::sample(R, S, (const double*)mu, (const double*)L, ldl, (const double*)eps, (double*)out, (cudaStream_t)stream);
 }
 
 int tgp_ell_forward(const TgpModel* md, const TgpParams* p, const void* mu, const void* v, const void* Y,

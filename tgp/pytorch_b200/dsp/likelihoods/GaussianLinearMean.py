@@ -40,7 +40,9 @@ class GaussianLinearMean(nn.Module):
         return self.expected_log_prob_rows(Y, gauss_mean, gauss_cov)[0]
 
     def marginal_moments(self, gauss_mean, gauss_cov, diagonal, **kwargs):
+        """(mean, covariance) of p(y*): gauss_cov (Dy,MB) + noise, or with diagonal=False the full (Dy,MB,MB) + noise I."""
         if not diagonal:
-            raise NotImplementedError('full-covariance moments belong to the exact-GP path (out of scope)')
+            eye = torch.eye(gauss_cov.size(-1), dtype=gauss_cov.dtype, device=gauss_cov.device)
+            return gauss_mean.clone(), gauss_cov + positive_transform(self._noise()).view(-1, 1, 1) * eye
         C_Y = positive_transform(self._noise()).expand(-1, gauss_mean.size(1)) + gauss_cov
         return gauss_mean.clone(), C_Y

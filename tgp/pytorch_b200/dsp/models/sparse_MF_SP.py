@@ -6,8 +6,9 @@ Same constructor, attributes and method signatures as the reference class (:47-1
 gathers parameters from the unchanged nn.Module tree and shapes the results like the reference does.
 
 Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened q(u), zero mean, (Scale)RBF-ARD or
-(Scale)Matern-ARD (nu = 1/2, 3/2, 5/2) kernel, diagonal marginals, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
-layers (optionally input-dependent with MC-dropout MLPs).  Multi-output models loop over outputs.
+(Scale)Matern-ARD (nu = 1/2, 3/2, 5/2) kernel, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
+layers (optionally input-dependent with MC-dropout MLPs).  Multi-output models loop over outputs.  Marginals are differentiable;
+the full covariance over a batch (`diagonal=False`) and the joint samples drawn from it are evaluation-only (no backward).
 """
 import numpy
 import torch
@@ -210,22 +211,59 @@ class sparse_MF_SP(nn.Module):
         return global_scale(self.N, rows)
 
     # ---- model computation ---------------------------------------------------------------------------------------
+    def _qf_engine(self, dy, device):
+        """The engine of the q(f) evaluations of output `dy` (marginals and full covariance share it, and with it the cached
+        factorisation); they do not involve the flow / likelihood."""
+        key = ('qf', dy, str(device), self._compute(), self._kernel_kind())
+        if key not in self._engines:
+            self._engines[key] = Engine(self.M, self.inp_dim, 'gauss_linear', 0, FlowLayout([]), device,
+                                        compute=self._compute(), kernel=self._kernel_kind())
+        eng = self._engines[key]
+        if not cg.cache_factorisation_in_eval:
+            eng.prepared_key = None
+        return eng
+
+    def _joint_qf(self, X, is_duvenaud):
+        """[(engine, mu (MB,), Sigma (MB, MB))] per output, FP64, for rows X (Dy, MB, D): the full covariance of q(f)."""
+        if is_duvenaud:
+            raise NotImplementedError('is_duvenaud (the deep-GP form) is outside the fused single-layer path')
+        self._check_fused_scope(X)
+        out = []
+        for dy in range(self.out_dim):
+            eng = self._qf_engine(dy, X.device)
+            mu, cov = Fn.qf_covariance(eng, X[dy].to(torch.float64).contiguous(), *self._gp_params(dy),
+                                       cg.check_cholesky_status, self._jitter())
+            out.append((eng, mu, cov))
+        return out
+
+    def _joint_samples(self, joint, S):
+        """f0 (Dy, S, MB) FP64: S joint samples mu + e L^T per output, L = psd_safe_cholesky(Sigma), e ~ N(0, I) (Dy, S, MB)
+        drawn here from torch's generator in FP64."""
+        MB = joint[0][1].shape[0]
+        e = torch.randn(self.out_dim, S, MB, dtype=torch.float64, device=joint[0][1].device)
+        constant, base = self._jitter()
+        f0 = []
+        for dy, (eng, mu, cov) in enumerate(joint):
+            L, _ = Fn.cov_cholesky_ladder(eng, cov, base, constant)
+            f0.append(eng.cov_sample(mu, L, e[dy].contiguous()))
+        return torch.stack(f0)
+
     def marginal_variational_qf_parameters(self, X, diagonal, is_duvenaud, init_Z=None):
-        """q(f) = int p(f|u) q(u) du at the rows of X: mean (Dy,MB,1), diagonal covariance (Dy,MB,1)."""
-        if not diagonal or is_duvenaud:
-            raise NotImplementedError('the fused path returns diagonal marginals of a single-layer model')
+        """q(f) = int p(f|u) q(u) du at the rows of X: mean (Dy,MB,1) and diagonal covariance (Dy,MB,1), or with
+        diagonal=False the full covariance over the rows (Dy,MB,MB).  The full covariance has no backward: call it under
+        torch.no_grad().  Under row sharding it is the covariance of this rank's rows."""
         X = self._rows3(X)
+        if not diagonal:
+            joint = self._joint_qf(X, is_duvenaud)
+            mean = torch.stack([mu for _, mu, _ in joint]).unsqueeze(2)
+            return mean.to(self.Z.dtype), torch.stack([cov for _, _, cov in joint]).to(self.Z.dtype)
+        if is_duvenaud:
+            raise NotImplementedError('is_duvenaud (the deep-GP form) is outside the fused single-layer path')
         self._check_fused_scope(X)
         mus, vs = [], []
         for dy in range(self.out_dim):
             Z, raw_ls, raw_os, m, L_raw = self._gp_params(dy)
-            key = ('qf', dy, str(X.device), self._compute(), self._kernel_kind())
-            if key not in self._engines:     # marginals do not involve the flow / likelihood
-                self._engines[key] = Engine(self.M, self.inp_dim, 'gauss_linear', 0, FlowLayout([]), X.device,
-                                            compute=self._compute(), kernel=self._kernel_kind())
-            eng = self._engines[key]
-            if not cg.cache_factorisation_in_eval:
-                eng.prepared_key = None
+            eng = self._qf_engine(dy, X.device)
             mu, v = Fn.qf_marginals(eng, X[dy].to(torch.float64).contiguous(), Z, raw_ls, raw_os, m, L_raw,
                                     cg.check_cholesky_status, self._jitter())
             mus.append(mu)
@@ -321,19 +359,23 @@ class sparse_MF_SP(nn.Module):
             assert enable_eval_dropout(self.modules()), 'fully bayesian mode needs dropout layers in the flow networks'
 
     def predictive_distribution(self, X, diagonal=True, S_MC_NNet=None):
-        """Predictive mean / variance (Dy,MB) plus the q(f) marginals (Dy,MB,1)."""
+        """Predictive mean / variance (Dy,MB) plus the q(f) marginals (Dy,MB,1).  diagonal=False (GaussianLinearMean only):
+        the predictive covariance Sigma + noise I (Dy,MB,MB) plus q(f)'s mean (Dy,MB,1) and full covariance (Dy,MB,MB)."""
         X = self._rows3(X)
         assert not self.is_training, 'This method only works in eval mode'
-        if not diagonal:
-            raise NotImplementedError('predictive distribution with correlations is not supported')
+        lik = self.likelihood
+        if not diagonal and not isinstance(lik, GaussianLinearMean):
+            raise NotImplementedError('correlated predictive moments are implemented for the Gaussian likelihood with identity '
+                                      'link (GaussianLinearMean); under the other likelihoods the joint predictive is not Gaussian')
         self._eval_mode()
         if self.fully_bayesian:
             assert S_MC_NNet is not None, 'S_MC_NNet is required when the model is fully bayesian'
         n_mc = S_MC_NNet if self.fully_bayesian else 1
         with torch.no_grad():
-            mean_q_f, cov_q_f = self.marginal_variational_qf_parameters(X, diagonal=True, is_duvenaud=False)
-            lik = self.likelihood
-            if isinstance(lik, GaussianLinearMean):
+            mean_q_f, cov_q_f = self.marginal_variational_qf_parameters(X, diagonal=diagonal, is_duvenaud=False)
+            if not diagonal:
+                m1, m2 = lik.marginal_moments(mean_q_f.squeeze(2), cov_q_f, diagonal=False)
+            elif isinstance(lik, GaussianLinearMean):
                 m1, m2 = lik.marginal_moments(mean_q_f.squeeze(2), cov_q_f.squeeze(2), diagonal=True)
             elif isinstance(lik, GaussianNonLinearMean):
                 m1, m2 = [], []
@@ -444,9 +486,14 @@ class sparse_MF_SP(nn.Module):
 
     # ---- sampling (caller-side utilities; element-wise torch ops on the kernel outputs) --------------------------
     def sample_from_variational_marginal_base(self, X, diagonal, is_duvenaud, init_Z=None):
-        if not diagonal:
-            raise NotImplementedError('This function only works with diagonal=True')
+        """One sample of q(f) per row (Dy,MB), with the mean (Dy,MB,1) and covariance it was drawn from; diagonal=False draws
+        one JOINT sample over the rows of each output from the full covariance (Dy,MB,MB) (no backward: torch.no_grad())."""
         X = self._rows3(X)
+        if not diagonal:
+            joint = self._joint_qf(X, is_duvenaud)
+            f = self._joint_samples(joint, 1)[:, 0, :].to(self.Z.dtype)
+            mean = torch.stack([mu for _, mu, _ in joint]).unsqueeze(2).to(self.Z.dtype)
+            return f, mean, torch.stack([cov for _, _, cov in joint]).to(self.Z.dtype)
         mean_q_f, cov_q_f = self.marginal_variational_qf_parameters(X, diagonal=True, is_duvenaud=is_duvenaud, init_Z=init_Z)
         e = torch.randn(mean_q_f.shape, dtype=mean_q_f.dtype, device=mean_q_f.device)
         f = (e * cov_q_f.sqrt() + mean_q_f).squeeze(dim=2)
@@ -455,14 +502,26 @@ class sparse_MF_SP(nn.Module):
     def sample_from_variational_marginal(self, X, S, diagonal, is_duvenaud, init_Z=None):
         """S warped samples per row.  The reference repeats X S times through the whole q(f) computation
         (sparse_MF_SP.py:911-922), i.e. S x the cost of the marginals; mu and v do not depend on the sample, so they are
-        computed ONCE here and repeated (same distribution of samples, 1/S of the work; SURVEY.md §8f rank 1)."""
-        if not diagonal:
-            raise NotImplementedError('This function only works with diagonal=True')
+        computed ONCE here and repeated (same distribution of samples, 1/S of the work; SURVEY.md §8f rank 1).
+
+        diagonal=False: S joint samples over the rows of each output, f0 = mu + e L^T with L = psd_safe_cholesky(Sigma) and
+        e ~ N(0, I) (Dy, S, MB) in FP64.  f0 (Dy, S*MB) keeps the sample-major layout of the diagonal case, and f = G(f0, X)
+        goes through the flow modules the same way.  The mean is repeated as (Dy, S*MB, 1); the covariance is returned once,
+        (Dy, MB, MB), not repeated.  No backward: call it under torch.no_grad()."""
         X = self._rows3(X)
         if self.is_training:
             self.train()
         else:
             self._eval_mode()
+        if not diagonal:
+            joint = self._joint_qf(X, is_duvenaud)
+            f0 = self._joint_samples(joint, S).reshape(self.out_dim, -1).to(self.Z.dtype)
+            mean_q_f0 = torch.stack([mu for _, mu, _ in joint]).unsqueeze(2).repeat(1, S, 1).to(self.Z.dtype)
+            cov_q_f = torch.stack([cov for _, _, cov in joint]).to(self.Z.dtype)
+            Xr = X.repeat(1, S, 1)
+            f = torch.stack([g(f0[idx, :], Xr[idx]) for idx, g in enumerate(self.G_matrix)])
+            self.train()
+            return f, mean_q_f0, cov_q_f, f0
         mean1, cov1 = self.marginal_variational_qf_parameters(X, diagonal=True, is_duvenaud=is_duvenaud, init_Z=init_Z)
         mean_q_f0, cov_q_f0 = mean1.repeat(1, S, 1), cov1.repeat(1, S, 1)
         e = torch.randn(mean_q_f0.shape, dtype=mean_q_f0.dtype, device=mean_q_f0.device)

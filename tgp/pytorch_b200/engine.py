@@ -154,6 +154,8 @@ class Engine:
         self.kl = torch.zeros(1, dtype=torch.float64, device=self.device)
         self.status = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._batch_ws = None
+        self._cov_ws = None
+        self._chol_ws = None
         self._rb = None
         self._packed = None
         self.last_ell_sum = None
@@ -236,6 +238,51 @@ class Engine:
         _lib.check(self.lib.tgp_qf_forward(self.model, _ptr(self.step_ws), _ptr(self.batch_ws(R)), _ptr(X), R, _ptr(mu),
                                            _ptr(v), _stream(self.device)), 'tgp_qf_forward')
         return mu, v
+
+    # -- full covariance over a test batch (evaluation only: no backward) ----------------------------------------------
+    @_on_device
+    def qf_cov(self, X):
+        """(mu (R,), Sigma (R, R)) of q(f) at the rows of X from the factorisation in the step workspace (prepare() first).
+        Leaves the batch workspace alone, so it may run between an ELBO forward and its backward."""
+        R = X.shape[0]
+        _chk(X, 'X', (R, self.D))
+        nbytes = self.lib.tgp_qf_cov_workspace_bytes(self.model, R)
+        if self._cov_ws is None or self._cov_ws.numel() < nbytes:
+            self._cov_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        mu = torch.empty(R, dtype=torch.float64, device=self.device)
+        cov = torch.empty(R, R, dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.tgp_qf_cov_forward(self.model, _ptr(self.step_ws), _ptr(self._cov_ws), _ptr(X), R, _ptr(mu),
+                                               _ptr(cov), R, _stream(self.device)), 'tgp_qf_cov_forward')
+        return mu, cov
+
+    @_on_device
+    def cov_cholesky(self, cov, jitter=0.0, scale=None):
+        """(L, status): L = chol(cov + jitter I), lower with an exactly zero upper triangle; status (device int32) is 0 or the
+        1-based index of the first pivot not above 8 eps * scale.  scale: device scalar, default the outputscale of the
+        parameters last set (the prior variance, which bounds every diagonal entry of a posterior covariance)."""
+        R = cov.shape[0]
+        _chk(cov, 'cov', (R, R))
+        if scale is None:
+            scale = torch.nn.functional.softplus(self._keep[2]).reshape(1)
+        _chk(scale, 'scale', (1,))
+        nbytes = self.lib.tgp_cov_cholesky_workspace_bytes(R)
+        if self._chol_ws is None or self._chol_ws.numel() < nbytes:
+            self._chol_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        L = torch.empty(R, R, dtype=torch.float64, device=self.device)
+        status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        _lib.check(self.lib.tgp_cov_cholesky(R, _ptr(cov), R, float(jitter), _ptr(scale), _ptr(self._chol_ws), _ptr(L), R,
+                                             _ptr(status), _stream(self.device)), 'tgp_cov_cholesky')
+        return L, status
+
+    @_on_device
+    def cov_sample(self, mu, L, eps):
+        """mu + eps L^T (S, R) for eps (S, R) drawn by the caller."""
+        S, R = eps.shape
+        _chk(mu, 'mu', (R,)); _chk(L, 'L', (R, R)); _chk(eps, 'eps', (S, R))
+        out = torch.empty(S, R, dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.tgp_cov_sample(R, S, _ptr(mu), _ptr(L), R, _ptr(eps), _ptr(out), _stream(self.device)),
+                   'tgp_cov_sample')
+        return out
 
     @_on_device
     def ell_forward(self, mu, v, Y, rowparams, scale, reduce_buf, want_grad=True):

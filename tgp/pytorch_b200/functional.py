@@ -206,22 +206,28 @@ def elbo_terms(engine, X, Y, scale, Z, raw_ls, raw_os, m, L_raw, log_var_noise, 
                             raw_os, m, L_raw, log_var_noise, theta, rowparams)
 
 
+def _on_factorisation(engine, params, frozen, work, check_status, jitter):
+    """`work()` on the factorisation of `params` = (Z, raw_ls, raw_os, m, L_raw).  With frozen parameters (no gradient
+    wanted) whose identity and version match the factorisation already in the step workspace, that factorisation is
+    reused (evaluation over many batches; the reference refactorises K_zz for every batch, sparse_MF_SP.py:330);
+    otherwise prepare_then factorises first."""
+    key = _param_key(params) + (tuple(jitter),)
+    if frozen and engine.prepared_key == key:
+        engine.generation += 1
+        return work()
+    _, out = prepare_then(engine, work, check=check_status, base_jitter=jitter[1], constant_jitter=jitter[0])
+    engine.prepared_key = key if check_status else None
+    return out
+
+
 class _QfMarginals(torch.autograd.Function):
     """mu, v of q(f) with a hand-written backward (used by marginal_variational_qf_parameters when called alone)."""
 
     @staticmethod
     def forward(ctx, engine, X, check_status, jitter, Z, raw_ls, raw_os, m, L_raw):
         engine.set_params(Z.detach(), raw_ls.detach(), raw_os.detach(), m.detach(), L_raw.detach(), None, None)
-        key = _param_key((Z, raw_ls, raw_os, m, L_raw)) + (tuple(jitter),)
-        if not any(ctx.needs_input_grad) and engine.prepared_key == key:
-            # evaluation over many batches with frozen parameters: the factorisation in the step workspace is still
-            # valid (the reference refactorises K_zz for every batch, sparse_MF_SP.py:330)
-            engine.generation += 1
-            mu, v = engine.qf_forward(X)
-        else:
-            _, (mu, v) = prepare_then(engine, lambda: engine.qf_forward(X), check=check_status, base_jitter=jitter[1],
-                                      constant_jitter=jitter[0])
-            engine.prepared_key = key if check_status else None
+        mu, v = _on_factorisation(engine, (Z, raw_ls, raw_os, m, L_raw), not any(ctx.needs_input_grad),
+                                  lambda: engine.qf_forward(X), check_status, jitter)
         ctx.engine, ctx.X = engine, X
         ctx.generation = engine.generation
         return mu, v
@@ -240,6 +246,38 @@ class _QfMarginals(torch.autograd.Function):
 
 def qf_marginals(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None)):
     return _QfMarginals.apply(engine, X, bool(check_status), tuple(jitter), Z, raw_ls, raw_os, m, L_raw)
+
+
+def qf_covariance(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None)):
+    """(mu (R,), Sigma (R, R)) of q(f) at the rows of X: the full covariance over the batch (tgp_qf_cov_forward), FP64 in
+    every compute mode.  Evaluation only: there is no backward, so a call that would need one raises instead of returning
+    a silently detached result.  Under row sharding each rank gets the covariance of its own rows."""
+    params = (Z, raw_ls, raw_os, m, L_raw)
+    if torch.is_grad_enabled() and any(t.requires_grad for t in params + (X,)):
+        raise NotImplementedError('the full covariance of q(f) has no backward: call it under torch.no_grad()')
+    engine.set_params(Z.detach(), raw_ls.detach(), raw_os.detach(), m.detach(), L_raw.detach(), None, None)
+    return _on_factorisation(engine, params, True, lambda: engine.qf_cov(X), check_status, jitter)
+
+
+def cov_cholesky_ladder(engine, cov, base_jitter=None, constant_jitter=0.0):
+    """L with L L^T = cov + jitter I, with the semantics of psd_safe_cholesky (code/dsp/utils.py:222-270) as in
+    _jitter_ladder: factorise with the constant jitter only; on failure check for NaN (NanError), then add base * 10^i,
+    i = 0..2, warning each time; raise after the third failure.  base: as sparse_MF_SP._jitter() (default 1e-8).
+    Returns (L, jitter added on top of the constant one)."""
+    L, status = engine.cov_cholesky(cov, constant_jitter)
+    fail = int(status.item())
+    if fail == 0:
+        return L, 0.0
+    if torch.isnan(cov).any():
+        raise NanError('cholesky: the covariance matrix has NaN entries')
+    jitter = 1e-8 if base_jitter is None else base_jitter
+    for i in range(3):
+        j = jitter * (10 ** i)
+        L, status = engine.cov_cholesky(cov, constant_jitter + j)
+        if int(status.item()) == 0:
+            warnings.warn('A not p.d., added jitter of %g to the diagonal' % j, NumericalWarning)
+            return L, j
+    raise RuntimeError('cholesky: matrix not positive definite after 3 jitter escalations (first bad pivot %d)' % fail)
 
 
 # ---- input-dependent flow MLPs on the device (tgp_flow_mlp_forward / _backward) ---------------------------------------
