@@ -11,7 +11,7 @@
  *  - the caller owns every buffer; the library never allocates device memory.  Workspaces are sized by the
  *    *_bytes() queries and carved deterministically, so the same workspace can be reused every step;
  *  - return 0 = ok; < 0 = usage / launch error (text from tgp_last_error());
- *  - one output GP per call (the reference's Dy > 1 case is a loop over outputs), whitened q(u);
+ *  - one output GP per call (the reference's Dy > 1 case is a loop over outputs); q(u) whitened or not (TgpModel.q_u_form);
  *  - dtype: TGP_F64 is what the reference's main.py runs (set_maximum_precission, config.py:37-46).
  */
 #ifndef TGP_B200_H
@@ -49,6 +49,10 @@ enum { TGP_KERNEL_RBF = 0,           /* s exp(-r^2 / 2)                       gp
        TGP_KERNEL_MATERN32 = 2,      /* s (1 + sqrt3 r) exp(-sqrt3 r)         nu = 1.5                               */
        TGP_KERNEL_MATERN52 = 3 };    /* s (1 + sqrt5 r + 5r^2/3) exp(-sqrt5 r)   nu = 2.5
                                       * r^2 = sum_d ((x_d - z_d) / lengthscale_d)^2, computed by direct differences    */
+enum { TGP_QU_WHITENED = 0,          /* u = L v, q(v) = N(m, P P^T), p(v) = N(0, I)    sparse_MF_SP.py:354-382, 406-431  */
+       TGP_QU_UNWHITENED = 1 };      /* q(u) = N(m, P P^T), p(u) = N(0, K_zz)         sparse_MF_SP.py:357-360, 386-391, 433-453
+                                      * P = tril(L_raw), L = chol(K_zz + jitter I).  Every entry point runs the whitened algebra on
+                                      * (L^-1 m, L^-1 P), which gives the same q(f) and KL; tgp_chain_backward maps the gradients back */
 #define TGP_MAX_LAYERS 64
 
 typedef struct TgpFlowLayer {
@@ -75,6 +79,8 @@ typedef struct TgpModel {            /* host struct; describes one output GP */
     TgpFlowLayer layers[TGP_MAX_LAYERS];
     int kernel;                      /* TGP_KERNEL_* (0 = RBF, so a zero-initialised description is unchanged).  Workspace
                                       * sizes do not depend on it                                                   */
+    int q_u_form;                    /* TGP_QU_* (0 = whitened, so a zero-initialised description is unchanged).  A non-whitened
+                                      * model's step workspace holds one more Mp x Mp matrix (tril(L_raw))                     */
 } TgpModel;
 
 typedef struct TgpParams {           /* device pointers to the model parameters (same shapes as the reference's) */
@@ -100,9 +106,13 @@ size_t tgp_step_workspace_bytes(const TgpModel* model);
 size_t tgp_batch_workspace_bytes(const TgpModel* model, long R);
 int tgp_reduce_layout(const TgpModel* model, TgpReduceLayout* out);
 
-/* K_zz -> psd-safe Cholesky -> explicit L^-1, C = L_S^T L^-1, whitened KL.
+/* K_zz -> psd-safe Cholesky -> explicit L^-1, C = L_S^T L^-1, KL.
  * Replaces sparse_MF_SP.py:316,330,344-346 and KLD :406-431, utils.py:222-270 (the wrapper drives the jitter
- * ladder: status[0] > 0 is the 1-based index of the first non-positive pivot).  kl_out, status: device. */
+ * ladder: status[0] > 0 is the 1-based index of the first non-positive pivot).  kl_out, status: device.
+ * TGP_QU_UNWHITENED: L_S = L^-1 tril(L_raw) and L^-1 m replace tril(L_raw) and m (the whitened pair of the same q(u)), and
+ * KL(N(m, P P^T) || N(0, L L^T)) uses the jittered L of the factorisation.  That KL needs L, so it is finished behind the
+ * factorisation: kl_out is then ready in the caller's stream order once a consuming entry point (tgp_qf_forward,
+ * tgp_qf_backward, tgp_chain_backward, tgp_qf_cov_forward) has been enqueued on it, or once tgp_factor_status() has returned. */
 int tgp_prepare(const TgpModel* model, const TgpParams* params, double jitter, void* step_ws, double* kl_out,
                 int* status, void* stream);
 
@@ -160,7 +170,9 @@ int tgp_qf_backward(const TgpModel* model, const TgpParams* params, const void* 
  * dZ (M,D), draw_lengthscale (D), draw_outputscale (1), dm (M), dL_raw (M,M; upper triangle exactly 0),
  * dlog_var_noise (1), dtheta (n_theta).  Replaces autograd's cholesky_backward / triangular_solve_backward.
  * g_dev: optional DEVICE pointer to {gE, gK}; when non-NULL it overrides the host scalars (no host sync needed to
- * read autograd's upstream gradients). */
+ * read autograd's upstream gradients).  TGP_QU_UNWHITENED: dm and dL_raw are the gradients w.r.t. the user's m and L_raw;
+ * the chain first forms the adjoints of the whitened pair (L^-1 m, L^-1 P) and maps them back, and the KL term reaches
+ * K_zz (and so Z, lengthscale, outputscale) through L.  gE = 0 is valid (the KL alone). */
 int tgp_chain_backward(const TgpModel* model, const TgpParams* params, void* step_ws, const double* reduce_buf,
                        double gE, double gK, const double* g_dev, void* dZ, void* draw_lengthscale, void* draw_outputscale, void* dm,
                        void* dL_raw, void* dlog_var_noise, void* dtheta, void* stream);
@@ -297,8 +309,9 @@ enum { TGP_OPT_FUSED_FORWARD = 1, TGP_OPT_ROW_CHUNK = 2,
                                       * tgp_qf_forward enqueues K_xz generation on the caller's stream and joins afterwards, every
                                       * other consumer of the step workspace joins first; 0: everything on the caller's stream.
                                       * Either way the outputs of each entry point are ready in the order of the caller's stream
-                                      * once a consuming entry point has been enqueued on it; kl_out is always in stream order,
-                                      * status is read with tgp_factor_status() */
+                                      * once a consuming entry point has been enqueued on it; kl_out is in stream order for
+                                      * whitened models (see tgp_prepare for non-whitened ones), status is read with
+                                      * tgp_factor_status() */
 int tgp_set_option(int key, int value);
 
 /* Number of kernels this library has launched so far in the process (bench.py's gpu_launches). */

@@ -14,6 +14,7 @@ LIK_GAUSS_LINEAR, LIK_GAUSS_NONLINEAR, LIK_BERNOULLI = 0, 1, 2
 FLOW_IDENTITY, FLOW_AFFINE, FLOW_TANH_STEP, FLOW_SAL, FLOW_ARCSINH, FLOW_BOXCOX, FLOW_INV_BOXCOX = 0, 1, 2, 3, 4, 5, 6
 FLOW_STEP_GROUP = 7
 KERNEL_RBF, KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2, 3
+QU_WHITENED, QU_UNWHITENED = 0, 1
 FLOW_RESTRICT, FLOW_ADD_F0, FLOW_PER_ROW, FLOW_SWITCH = 1, 2, 4, 8
 MAX_LAYERS = 64
 OPT_FUSED_FORWARD = 1
@@ -28,7 +29,7 @@ class TgpFlowLayer(C.Structure):
 class TgpModel(C.Structure):
     _fields_ = [('dtype', C.c_int), ('M', C.c_int), ('D', C.c_int), ('likelihood', C.c_int), ('n_quad', C.c_int),
                 ('n_theta', C.c_int), ('n_rowparams', C.c_int), ('n_layers', C.c_int),
-                ('layers', TgpFlowLayer * MAX_LAYERS), ('kernel', C.c_int)]
+                ('layers', TgpFlowLayer * MAX_LAYERS), ('kernel', C.c_int), ('q_u_form', C.c_int)]
 
 
 class TgpParams(C.Structure):

@@ -228,6 +228,49 @@ __global__ void k_finalize_LS(const double* __restrict__ dLS, const double* __re
     }
 }
 
+// Non-whitened q(u): the batch pass and the KL see the whitened pair (m~, P~) = (L^-1 m, L^-1 P).  For rows r < M, c <= r:
+//   m~bar[r]  = gE dm_ell[r] + gK m~[r]                                     -> mbar
+//   P~bar     = gE dLS + gK (P~ - diag(1 / P~_ii))                          (dLS in place)
+//   Gtot      = gE Gtot + m~bar m^T                                         (in place; P~bar P^T is added by a GEMM)
+// Gtot then is the complete dF/dL^-1 of F = gE ELL + gK KL, which the Murray chain carries to K_zz.
+__global__ void __launch_bounds__(256) k_unwhiten_adjoints(double* __restrict__ dLS, const double* __restrict__ LSt,
+                                                           double* __restrict__ Gtot, long ld, int M,
+                                                           const double* __restrict__ dm_ell, const double* __restrict__ mt,
+                                                           const double* __restrict__ m, double gE, double gK,
+                                                           const double* __restrict__ g_dev, double* __restrict__ mbar) {
+    const int r = blockIdx.x;
+    if (g_dev) { gE = g_dev[0]; gK = g_dev[1]; }
+    const double mb = gE * dm_ell[r] + gK * mt[r];
+    if (threadIdx.x == 0) mbar[r] = mb;
+    const double inv_d = 1.0 / LSt[(long)r * ld + r];
+    for (int c = threadIdx.x; c <= r; c += blockDim.x) {
+        const long i = (long)r * ld + c;
+        dLS[i] = gE * dLS[i] + gK * (LSt[i] - (c == r ? inv_d : 0.0));
+        Gtot[i] = gE * Gtot[i] + mb * m[c];
+    }
+}
+
+// Final raw-parameter gradients of a non-whitened model.  The K_zz-side accumulators (acc_*) already carry gE and gK
+// (through Gtot); the K_xz-side sums of the reduce buffer (rb_*) are scaled by gE here.  dm and dL_raw are written by the chain.
+__global__ void k_finalize_small_unwhitened(const double* __restrict__ raw_ls, const double* __restrict__ raw_os, int M, int D,
+                                            int n_theta, double gE, const double* __restrict__ g_dev,
+                                            const double* __restrict__ acc_dZ, const double* __restrict__ acc_dls,
+                                            const double* __restrict__ acc_dos, const double* __restrict__ rb_dZ,
+                                            const double* __restrict__ rb_dls, const double* __restrict__ rb_dos,
+                                            const double* __restrict__ rb_dlogvar, const double* __restrict__ rb_dtheta,
+                                            double* __restrict__ out_dZ, double* __restrict__ out_dls, double* __restrict__ out_dos,
+                                            double* __restrict__ out_dlogvar, double* __restrict__ out_dtheta) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g_dev) gE = g_dev[0];
+    if (i < M * D) out_dZ[i] = acc_dZ[i] + gE * rb_dZ[i];
+    if (i < D) out_dls[i] = (acc_dls[i] + gE * rb_dls[i]) * sigmoid_d(raw_ls[i]);
+    if (i == 0) {
+        out_dos[0] = (acc_dos[0] + gE * rb_dos[0]) * sigmoid_d(raw_os[0]);
+        if (out_dlogvar) out_dlogvar[0] = gE * rb_dlogvar[0];
+    }
+    if (i < n_theta) out_dtheta[i] = gE * rb_dtheta[i];
+}
+
 __global__ void k_copy_strided(const double* __restrict__ src, long lds, double* __restrict__ dst, long ldd, int M) {
     const int r = blockIdx.x;
     for (int c = threadIdx.x; c < M; c += blockDim.x) dst[(long)r * ldd + c] = src[(long)r * lds + c];

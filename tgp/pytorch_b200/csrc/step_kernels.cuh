@@ -274,6 +274,45 @@ __global__ void k_kl_finish(const double* __restrict__ kl, int M, double* __rest
     out[0] = 0.5 * (-kl[0] + kl[1] + kl[2] - (double)M);
 }
 
+// sum of v over the 256 threads of the CTA, valid in thread 0
+__device__ __forceinline__ double block_sum_256(double v) {
+    __shared__ double part[8];
+    v = warp_sum(v);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double t = 0.0;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < 8; ++w) t += part[w];
+    return t;
+}
+
+// y = L x (trans = 0) or y = L^T x (trans = 1) for a lower-triangular L (M x M, ld ld); one CTA of 256 threads per element
+__global__ void __launch_bounds__(256) k_trmv_lower(const double* __restrict__ L, long ld, int M, const double* __restrict__ x,
+                                                    double* __restrict__ y, int trans) {
+    const int i = blockIdx.x;
+    double acc = 0.0;
+    if (trans) for (int k = i + threadIdx.x; k < M; k += 256) acc = fma(L[(long)k * ld + i], x[k], acc);
+    else for (int k = threadIdx.x; k <= i; k += 256) acc = fma(L[(long)i * ld + k], x[k], acc);
+    acc = block_sum_256(acc);
+    if (threadIdx.x == 0) y[i] = acc;
+}
+
+// The KL sums of k_tril_kl for a lower-triangular P (ld ld) that is already in place:
+// kl[0] += sum_i log(P_ii^2)   kl[1] += sum_i m_i^2   kl[2] += ||P||_F^2
+__global__ void __launch_bounds__(256) k_kl_rows(const double* __restrict__ P, long ld, const double* __restrict__ m, int M,
+                                                 double* __restrict__ kl) {
+    const int r = blockIdx.x;
+    double fro = 0.0;
+    for (int c = threadIdx.x; c <= r; c += 256) { const double v = P[(long)r * ld + c]; fro = fma(v, v, fro); }
+    fro = block_sum_256(fro);
+    if (threadIdx.x == 0) {
+        const double d = P[(long)r * ld + r];
+        atomicAdd(kl + 0, log(d * d));
+        atomicAdd(kl + 1, m[r] * m[r]);
+        atomicAdd(kl + 2, fro);
+    }
+}
+
 __global__ void k_halve_diag(double* __restrict__ P, long ld, int M) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < M) P[(long)i * ld + i] *= 0.5;
@@ -284,6 +323,8 @@ struct StepView {       // carved views into the per-step workspace (all doubles
     int kind;           // TGP_KERNEL_* of the model (not part of the layout)
     double *ls, *os, *Zs, *kl3, *Dinv, *mvec;
     double *Kzz, *L, *Linv, *LS, *Cm, *S0, *S1, *S2, *S3;
+    // TGP_QU_UNWHITENED only (nullptr otherwise): P = tril(L_raw), while LS and mvec hold the whitened pair L^-1 P, L^-1 m
+    double* P;
 };
 
 inline int pad_M(int M) {
@@ -307,6 +348,7 @@ inline StepView step_view(Carve& c, int M, int D) {
     v.Kzz = c.take<double>(mm); v.L = c.take<double>(mm); v.Linv = c.take<double>(mm); v.LS = c.take<double>(mm);
     v.Cm = c.take<double>(mm);
     v.S0 = c.take<double>(mm); v.S1 = c.take<double>(mm); v.S2 = c.take<double>(mm); v.S3 = c.take<double>(mm);
+    v.P = nullptr;      // carved last by step_layout for non-whitened models, so that no other offset depends on the form
     return v;
 }
 
@@ -337,26 +379,30 @@ inline int blocked_cholesky(double* Aw, double* L, double* Linv, double* Dinv, i
 }
 
 // K_zz (+jitter) -> L, L^-1 (explicit), C = L_S^T L^-1, KL.  Everything stays on `st`; no host sync.
+// Non-whitened q(u) (v.P set): L_S = L^-1 P and mvec = L^-1 m, the whitened pair of the same q(u), and the KL of that pair.
 inline int run_prepare(const StepView& v, const double* Z, const double* raw_ls, const double* raw_os,
                        const double* m, const double* Lraw, double jitter, double* kl_out, int* status,
                        bool need_C, cudaStream_t st, cudaStream_t (*fork)(cudaStream_t) = nullptr) {
     const int M = v.M, Mp = v.Mp, D = v.D, NB = POTRF_NB;
     const size_t mm = (size_t)Mp * Mp;
+    const bool unwhitened = v.P != nullptr;
     cudaMemsetAsync(status, 0, sizeof(int), st);
     cudaMemsetAsync(v.kl3, 0, 8 * sizeof(double), st);
-    cudaMemsetAsync(v.L, 0, 2 * mm * sizeof(double), st);          // L and Linv are contiguous
-    cudaMemcpyAsync(v.mvec, m, (size_t)M * sizeof(double), cudaMemcpyDeviceToDevice, st);
+    // L and Linv are contiguous, and so is LS after them: the non-whitened transform writes its lower triangle only
+    cudaMemsetAsync(v.L, 0, (unwhitened ? 3 : 2) * mm * sizeof(double), st);
+    if (!unwhitened) cudaMemcpyAsync(v.mvec, m, (size_t)M * sizeof(double), cudaMemcpyDeviceToDevice, st);
     {
         const int n = max(M * D, D);
         k_transform_params<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(Z, raw_ls, raw_os, M, D, v.ls, v.os, v.Zs);
         TGP_TRY(check_launch("k_transform_params"));
     }
-    k_tril_kl<<<Mp, 256, 0, st>>>(Lraw, m, M, v.LS, Mp, Mp, v.kl3);
+    // non-whitened: tril(L_raw) goes to P, and the sums of this kernel (of the untransformed pair) to unused slots of kl3
+    k_tril_kl<<<Mp, 256, 0, st>>>(Lraw, m, M, unwhitened ? v.P : v.LS, Mp, Mp, unwhitened ? v.kl3 + 4 : v.kl3);
     TGP_TRY(check_launch("k_tril_kl"));
-    k_kl_finish<<<1, 1, 0, st>>>(v.kl3, M, kl_out);
+    if (!unwhitened) k_kl_finish<<<1, 1, 0, st>>>(v.kl3, M, kl_out);
     cudaStream_t fst = fork ? fork(st) : nullptr;
-    // everything above stays on the caller's stream (kl_out is an output in stream order); the factorisation proper forks
-    // onto the high-priority stream `fst` when the caller passed one (tgp_prepare), see common.cuh
+    // everything above stays on the caller's stream (a whitened model's kl_out is an output in stream order); the factorisation
+    // proper forks onto the high-priority stream `fst` when the caller passed one (tgp_prepare), see common.cuh
     st = fst ? fst : st;
     TGP_TRY(with_kernel(v.kind, [&](auto k) {
         return launch_rbf<decltype(k)::value>(v.Zs, v.Zs, v.ls, v.os, M, M, D, 1, v.Kzz, Mp, Mp, Mp, jitter, st);
@@ -375,6 +421,18 @@ inline int run_prepare(const StepView& v, const double* Z, const double* raw_ls,
         GemmArgs x = make_gemm(b, b, b, v.Linv + off_C, Mp, 0, v.S0 + off_B, Mp, 1, v.Linv + off_B, Mp, -1.0, 0.0);
         x.a_tri = 1; x.batch = batch; x.strideA = x.strideB = x.strideC = stride;
         TGP_TRY(gemm_f64(x, st));
+    }
+    if (unwhitened) {
+        // L_S = L^-1 P   (Aop[m,k] = Linv[m,k], nonzero k <= m;  Bop[n,k] = P[k,n], nonzero k >= n)
+        GemmArgs t = make_gemm(M, M, M, v.Linv, Mp, 0, v.P, Mp, 1, v.LS, Mp);
+        t.a_tri = 1; t.b_tri = 2; t.c_lower = 1;
+        TGP_TRY(gemm_f64(t, st));
+        k_trmv_lower<<<M, 256, 0, st>>>(v.Linv, Mp, M, m, v.mvec, 0);
+        TGP_TRY(check_launch("k_trmv_lower"));
+        // KL(N(m, P P^T) || N(0, L L^T)) = the whitened KL of (L^-1 m, L^-1 P): it needs L, so it is finished here
+        k_kl_rows<<<M, 256, 0, st>>>(v.LS, Mp, v.mvec, M, v.kl3);
+        TGP_TRY(check_launch("k_kl_rows"));
+        k_kl_finish<<<1, 1, 0, st>>>(v.kl3, M, kl_out);
     }
     // C = L_S^T L^-1   (Aop[m,k] = LS[k,m], nonzero k >= m;  Bop[n,k] = Linv[k,n], nonzero k >= n)
     if (need_C) {      // only the tensor-core mode contracts with C; the FP64 mode applies L_S to A directly

@@ -71,6 +71,8 @@ inline int validate(const TgpModel* md) {
     if (md->M < 1 || md->D < 1) return set_error(-1, "M and D must be positive");
     if (!kernel_kind_valid(md->kernel))
         return set_error(-1, "kernel must be TGP_KERNEL_RBF, TGP_KERNEL_MATERN12, TGP_KERNEL_MATERN32 or TGP_KERNEL_MATERN52");
+    if (md->q_u_form != TGP_QU_WHITENED && md->q_u_form != TGP_QU_UNWHITENED)
+        return set_error(-1, "q_u_form must be TGP_QU_WHITENED or TGP_QU_UNWHITENED");
     if (md->n_layers < 0 || md->n_layers > TGP_MAX_LAYERS) return set_error(-1, "too many flow layers");
     if (md->n_theta < 0 || md->n_theta > MAX_THETA) return set_error(-1, "too many global flow parameters");
     if (md->n_rowparams < 0 || md->n_rowparams > MAX_ROWP) return set_error(-1, "too many per-row flow parameters");
@@ -120,7 +122,8 @@ inline int gemm_small(GemmArgs g, cudaStream_t st) {
     return gemm_f64(g, st);
 }
 
-// The step workspace: the FP64 region, then the planes of the active tensor-core mode (TGP_F64 has none)
+// The step workspace: the FP64 region, then the planes of the active tensor-core mode (TGP_F64 has none), then tril(L_raw)
+// of a non-whitened model
 struct StepWorkspace { StepView f64; tc::StepPlanes tc; crt::StepPlanes crt; };
 inline StepWorkspace step_layout(Carve& c, const TgpModel* md) {
     StepWorkspace w{};
@@ -128,6 +131,7 @@ inline StepWorkspace step_layout(Carve& c, const TgpModel* md) {
     w.f64.kind = md->kernel;
     if (md->dtype == TGP_F32) w.tc = tc::step_planes(c, md->M);
     if (md->dtype == TGP_F64_I8) w.crt = crt::step_planes(c, md->M);
+    if (md->q_u_form == TGP_QU_UNWHITENED) w.f64.P = c.take<double>((size_t)w.f64.Mp * w.f64.Mp);
     return w;
 }
 }  // namespace tgp
@@ -357,6 +361,27 @@ int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, co
         cudaMemcpyAsync(s.S0, Cbar, mm * sizeof(double), cudaMemcpyDeviceToDevice, st);
         cudaMemcpyAsync(Gtot, reduce_buf + l.Gbar, mm * sizeof(double), cudaMemcpyDeviceToDevice, st);
     }
+    const bool unwhitened = s.P != nullptr;
+    if (unwhitened) {
+        // S0 and Gtot hold dELL/dL_S and dELL/dL^-1 of the whitened pair (m~, P~) = (L^-1 m, L^-1 P).  With its adjoints
+        // m~bar, P~bar (k_unwhiten_adjoints):  dm = L^-T m~bar,  dP = tril(L^-T P~bar),  dL^-1 = gE Gtot + tril(m~bar m^T + P~bar P^T).
+        // gE and gK both enter Gtot here, before the Murray chain; the final kernel does not scale the K_zz side again.
+        double* mbar = s.S3;                       // S3 is free until Phi
+        k_unwhiten_adjoints<<<M, 256, 0, st>>>(s.S0, s.LS, Gtot, Mp, M, reduce_buf + l.dm, s.mvec, (const double*)p->m, gE, gK,
+                                               g_dev, mbar);
+        TGP_TRY(check_launch("k_unwhiten_adjoints"));
+        // Gtot += tril(P~bar P^T)   (Aop[m,k] = P~bar[m,k], nonzero k <= m;  Bop[n,k] = P[n,k], nonzero k <= n)
+        GemmArgs u1 = make_gemm(M, M, M, s.S0, Mp, 0, s.P, Mp, 0, Gtot, Mp, 1.0, 1.0);
+        u1.a_tri = 1; u1.b_tri = 1; u1.c_lower = 1;
+        TGP_TRY(gemm_small(u1, st));
+        k_trmv_lower<<<M, 256, 0, st>>>(s.Linv, Mp, M, mbar, (double*)dm, 1);
+        TGP_TRY(check_launch("k_trmv_lower"));
+        // dL_raw = tril(L^-T P~bar)   (Aop[m,k] = Linv[k,m], nonzero k >= m;  Bop[n,k] = P~bar[k,n], nonzero k >= n)
+        cudaMemsetAsync(dL_raw, 0, (size_t)M * M * sizeof(double), st);
+        GemmArgs u2 = make_gemm(M, M, M, s.Linv, Mp, 1, s.S0, Mp, 1, (double*)dL_raw, M, 1.0, 1.0);
+        u2.a_tri = 2; u2.b_tri = 2; u2.c_lower = 1;
+        TGP_TRY(gemm_small(u2, st));
+    }
     // T1 = Gtot * Linv^T
     GemmArgs a3 = make_gemm(M, M, M, Gtot, Mp, 0, s.Linv, Mp, 0, s.S1, Mp);
     a3.a_tri = 1; a3.b_tri = 1;
@@ -380,16 +405,28 @@ int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, co
     a7.a_tri = 2;
     TGP_TRY(gemm_small(a7, st));
     // K_zz -> Z (both index roles: factor 2 on the symmetrised matrix), lengthscale, outputscale.
-    // accumulators: start from the K_xz-side sums of the reduce buffer
+    // accumulators: start from the K_xz-side sums of the reduce buffer (whitened)
     dZacc = s.S3;   // Phi is dead now
-    cudaMemcpyAsync(dZacc, reduce_buf + l.dZ, (size_t)M * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
     double* dls_acc = dZacc + even((long)M * D);
     double* dos_acc = dls_acc + even(D);
-    cudaMemcpyAsync(dls_acc, reduce_buf + l.dls, (size_t)D * sizeof(double), cudaMemcpyDeviceToDevice, st);
-    cudaMemcpyAsync(dos_acc, reduce_buf + l.dos, sizeof(double), cudaMemcpyDeviceToDevice, st);
+    if (unwhitened) {   // the K_zz side alone (it carries gE and gK); the final kernel adds gE times the K_xz-side sums
+        cudaMemsetAsync(dZacc, 0, (size_t)(even((long)M * D) + even(D) + 1) * sizeof(double), st);
+    } else {
+        cudaMemcpyAsync(dZacc, reduce_buf + l.dZ, (size_t)M * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(dls_acc, reduce_buf + l.dls, (size_t)D * sizeof(double), cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(dos_acc, reduce_buf + l.dos, sizeof(double), cudaMemcpyDeviceToDevice, st);
+    }
     TGP_TRY(with_kernel(s.kind, [&](auto k) {
         return launch_kernel_grads<decltype(k)::value>(s.S2, Mp, s.Zs, 1, s.Zs, s.ls, s.os, M, M, D, 1, 2.0, dZacc, dls_acc, dos_acc, st);
     }));
+    if (unwhitened) {
+        const int n = M * D > md->n_theta ? M * D : md->n_theta;
+        k_finalize_small_unwhitened<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(
+            (const double*)p->raw_lengthscale, (const double*)p->raw_outputscale, M, D, md->n_theta, gE, g_dev, dZacc, dls_acc,
+            dos_acc, reduce_buf + l.dZ, reduce_buf + l.dls, reduce_buf + l.dos, reduce_buf + l.dlogvar, reduce_buf + l.dtheta,
+            (double*)dZ, (double*)draw_ls, (double*)draw_os, (double*)dlogvar, (double*)dtheta);
+        return check_launch("k_finalize_small_unwhitened");
+    }
     {
         const int n = M * D > M ? M * D : M;
         const int nn = n > md->n_theta ? n : md->n_theta;

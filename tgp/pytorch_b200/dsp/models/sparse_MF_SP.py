@@ -5,7 +5,7 @@ Same constructor, attributes and method signatures as the reference class (:47-1
 `test_log_likelihood` is enqueued on the B200 through libtgp_b200.so (tgp/pytorch_b200/functional.py); this file only
 gathers parameters from the unchanged nn.Module tree and shapes the results like the reference does.
 
-Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened q(u), zero mean, (Scale)RBF-ARD or
+Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened or non-whitened q(u), zero mean, (Scale)RBF-ARD or
 (Scale)Matern-ARD (nu = 1/2, 3/2, 5/2) kernel, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
 layers (optionally input-dependent with MC-dropout MLPs).  Multi-output models loop over outputs.  Marginals are differentiable;
 the full covariance over a batch (`diagonal=False`) and the joint samples drawn from it are evaluation-only (no backward).
@@ -144,8 +144,6 @@ class sparse_MF_SP(nn.Module):
 
     # ---- parameter gathering for the kernels ---------------------------------------------------------------------
     def _check_fused_scope(self, X):
-        if not self.is_whiten:
-            raise NotImplementedError('the fused path implements the whitened representation (every shipped configuration)')
         if X.dtype not in (torch.float64, torch.float32):
             raise NotImplementedError('inputs must be float64 (cg.set_maximum_precission(), as main.py does) or float32')
         if not X.is_cuda:
@@ -180,10 +178,10 @@ class sparse_MF_SP(nn.Module):
     def _engine(self, dy, layout, device):
         kind = _LIK_KIND[type(self.likelihood)]
         key = (dy, kind, self.quad_points, tuple(tuple(sorted(l.items())) for l in layout.layers), str(device), self._compute(),
-               self._kernel_kind())
+               self._kernel_kind(), bool(self.is_whiten))
         if key not in self._engines:
             self._engines[key] = Engine(self.M, self.inp_dim, kind, self.quad_points if kind != 'gauss_linear' else 0,
-                                        layout, device, compute=self._compute(), kernel=self._kernel_kind())
+                                        layout, device, compute=self._compute(), kernel=self._kernel_kind(), whiten=self.is_whiten)
         return self._engines[key]
 
     def _compute(self):
@@ -214,10 +212,10 @@ class sparse_MF_SP(nn.Module):
     def _qf_engine(self, dy, device):
         """The engine of the q(f) evaluations of output `dy` (marginals and full covariance share it, and with it the cached
         factorisation); they do not involve the flow / likelihood."""
-        key = ('qf', dy, str(device), self._compute(), self._kernel_kind())
+        key = ('qf', dy, str(device), self._compute(), self._kernel_kind(), bool(self.is_whiten))
         if key not in self._engines:
             self._engines[key] = Engine(self.M, self.inp_dim, 'gauss_linear', 0, FlowLayout([]), device,
-                                        compute=self._compute(), kernel=self._kernel_kind())
+                                        compute=self._compute(), kernel=self._kernel_kind(), whiten=self.is_whiten)
         eng = self._engines[key]
         if not cg.cache_factorisation_in_eval:
             eng.prepared_key = None
@@ -259,22 +257,45 @@ class sparse_MF_SP(nn.Module):
             return mean.to(self.Z.dtype), torch.stack([cov for _, _, cov in joint]).to(self.Z.dtype)
         if is_duvenaud:
             raise NotImplementedError('is_duvenaud (the deep-GP form) is outside the fused single-layer path')
+        mean, cov, _ = self._marginals(X)
+        return mean, cov
+
+    def _marginals(self, X, with_kl=False):
+        """q(f) marginals (Dy,MB,1) x 2 at the rows of X (Dy,MB,D), and with_kl=True the KL term of each output (Dy,) from
+        the same factorisation (else None)."""
         self._check_fused_scope(X)
-        mus, vs = [], []
+        mus, vs, kls = [], [], []
         for dy in range(self.out_dim):
             Z, raw_ls, raw_os, m, L_raw = self._gp_params(dy)
             eng = self._qf_engine(dy, X.device)
-            mu, v = Fn.qf_marginals(eng, X[dy].to(torch.float64).contiguous(), Z, raw_ls, raw_os, m, L_raw,
-                                    cg.check_cholesky_status, self._jitter())
-            mus.append(mu)
-            vs.append(v)
-        return torch.stack(mus).unsqueeze(2).to(self.Z.dtype), torch.stack(vs).unsqueeze(2).to(self.Z.dtype)
+            out = Fn.qf_marginals(eng, X[dy].to(torch.float64).contiguous(), Z, raw_ls, raw_os, m, L_raw,
+                                  cg.check_cholesky_status, self._jitter(), with_kl=with_kl)
+            mus.append(out[0])
+            vs.append(out[1])
+            if with_kl:
+                kls.append(out[2])
+        d = self.Z.dtype
+        return torch.stack(mus).unsqueeze(2).to(d), torch.stack(vs).unsqueeze(2).to(d), torch.stack(kls) if with_kl else None
+
+    def _kl_engine(self, dy, device):
+        """The engine of a stand-alone non-whitened KLD() of output `dy`: a factorisation of its own, so that KLD() leaves the
+        workspaces of a pending ELBO or marginals backward alone.  The KL is FP64 in every compute mode: 'f64' suffices."""
+        key = ('kl', dy, str(device), self._kernel_kind())
+        if key not in self._engines:
+            self._engines[key] = Engine(self.M, self.inp_dim, 'gauss_linear', 0, FlowLayout([]), device, compute='f64',
+                                        kernel=self._kernel_kind(), whiten=False)
+        return self._engines[key]
 
     def KLD(self):
-        """KL[q(u) || p(u)] per output, whitened: 0.5 (-log|S| + m'm + tr S - M).  Stand-alone helper (a few
-        element-wise ops on the parameters); `ELBO` takes the same quantity from the fused prepare kernel."""
+        """KL[q(u) || p(u)] per output (Dy,).  Whitened: 0.5 (-log|S| + m'm + tr S - M), a few element-wise ops on the
+        parameters; `ELBO` takes the same quantity from the fused prepare kernel.  Non-whitened: KL(N(m, S) || N(0, K_zz)),
+        which needs the factorisation of K_zz (with the jitter ladder of the marginals): one prepare per output on an engine of
+        its own, differentiable through the hand-written chain."""
         if not self.is_whiten:
-            raise NotImplementedError('only the whitened representation is implemented')
+            self._check_fused_scope(self.Z)
+            kls = [Fn.kl_term(self._kl_engine(dy, self.Z.device), *self._gp_params(dy), jitter=self._jitter())
+                   for dy in range(self.out_dim)]
+            return torch.stack(kls).to(self.Z.dtype)
         m = self.q_U.variational_mean
         L = self.q_U.chol_variational_covar.tril()
         if self.q_U_is_shared:
@@ -321,7 +342,10 @@ class sparse_MF_SP(nn.Module):
         through `Fn.qf_marginals`), then ONE Monte-Carlo kernel over all classes (tgp_mc_softmax_rows).  Under row sharding the
         marginals' backward all-reduces its packed buffer (one collective per class) and the flow scalars are summed across
         ranks; the returned ELL is the global one when cg.sync_elbo_in_forward is set, else this rank's share."""
-        mean, cov = self.marginal_variational_qf_parameters(X, diagonal=True, is_duvenaud=False)
+        if self.is_whiten:
+            mean, cov = self.marginal_variational_qf_parameters(X, diagonal=True, is_duvenaud=False)
+        else:   # each class's KL from the factorisation of its marginals (KLD() would factorise again and void their backward)
+            mean, cov, kl_classes = self._marginals(X, with_kl=True)
         ell = self.likelihood.expected_log_prob(Y.t(), mean.squeeze(dim=2), cov.squeeze(dim=2), flow=self.G_matrix, X=X)
         dist = Fn._world()
         if dist is not None and cg.sync_elbo_in_forward:
@@ -329,7 +353,7 @@ class sparse_MF_SP(nn.Module):
             dist.all_reduce(tot)
             ell = ell + (tot - ell.detach())
         ELL = scale * ell
-        KLD = self.KLD().sum()
+        KLD = self.KLD().sum() if self.is_whiten else kl_classes.sum()
         KLD_flow = 0.0
         for flow in self.G_matrix:
             KLD_flow = KLD_flow + flow.KLD()

@@ -121,7 +121,7 @@ KERNELS = {'rbf': _lib.KERNEL_RBF, 'matern12': _lib.KERNEL_MATERN12, 'matern32':
 
 
 class Engine:
-    def __init__(self, M, D, likelihood, n_quad, flow_layout, device, compute='f64', kernel='rbf'):
+    def __init__(self, M, D, likelihood, n_quad, flow_layout, device, compute='f64', kernel='rbf', whiten=True):
         self.lib = _lib.load()
         self.device = torch.device(device)
         if self.device.type != 'cuda':
@@ -141,6 +141,9 @@ class Engine:
             raise ValueError('kernel must be one of %s' % (', '.join(repr(k) for k in KERNELS),))
         self.kernel = kernel
         self.model.kernel = KERNELS[kernel]
+        # q(u) = N(m, P P^T) of the whitened variable (True) or of u itself (False, the reference's is_whiten=False)
+        self.whiten = bool(whiten)
+        self.model.q_u_form = _lib.QU_WHITENED if self.whiten else _lib.QU_UNWHITENED
         self.model.likelihood = _LIK[likelihood]
         self.model.n_quad = int(n_quad)
         flow_layout.fill(self.model)

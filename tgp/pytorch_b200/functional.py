@@ -221,7 +221,9 @@ def _on_factorisation(engine, params, frozen, work, check_status, jitter):
 
 
 class _QfMarginals(torch.autograd.Function):
-    """mu, v of q(f) with a hand-written backward (used by marginal_variational_qf_parameters when called alone)."""
+    """mu, v of q(f) with a hand-written backward (used by marginal_variational_qf_parameters when called alone), and the
+    KL term of the same factorisation: a model that needs both (the multiclass ELBO) cannot factorise twice, because the
+    second factorisation would overwrite what the marginals' backward reads."""
 
     @staticmethod
     def forward(ctx, engine, X, check_status, jitter, Z, raw_ls, raw_os, m, L_raw):
@@ -230,22 +232,55 @@ class _QfMarginals(torch.autograd.Function):
                                   lambda: engine.qf_forward(X), check_status, jitter)
         ctx.engine, ctx.X = engine, X
         ctx.generation = engine.generation
-        return mu, v
+        return mu, v, engine.kl.clone().reshape(())        # the KL is in stream order once qf_forward has been enqueued
 
     @staticmethod
-    def backward(ctx, g_mu, g_v):
+    def backward(ctx, g_mu, g_v, g_kl):
         engine, X = ctx.engine, ctx.X
         _check_generation(ctx)
         rb = engine.new_reduce_buffer()
         zeros = torch.zeros(X.shape[0], dtype=torch.float64, device=X.device)
         engine.qf_backward(X, zeros if g_mu is None else g_mu.contiguous(), zeros if g_v is None else g_v.contiguous(), rb)
         allreduce_packed(engine, rb)               # row-sharded callers (multiclass ELBO): sum over ranks before the chain
-        out = engine.chain_backward(rb, 1.0, 0.0)
+        if g_kl is None:
+            out = engine.chain_backward(rb, 1.0, 0.0)
+        else:
+            g_dev = torch.stack([torch.ones((), dtype=torch.float64, device=X.device), g_kl.reshape(()).to(torch.float64)])
+            out = engine.chain_backward(rb, g_dev=g_dev.contiguous())
         return None, None, None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw']
 
 
-def qf_marginals(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None)):
-    return _QfMarginals.apply(engine, X, bool(check_status), tuple(jitter), Z, raw_ls, raw_os, m, L_raw)
+def qf_marginals(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None), with_kl=False):
+    """(mu, v) of q(f) at the rows of X; with_kl=True: (mu, v, KL) with the KL term of the same factorisation."""
+    mu, v, kl = _QfMarginals.apply(engine, X, bool(check_status), tuple(jitter), Z, raw_ls, raw_os, m, L_raw)
+    return (mu, v, kl) if with_kl else (mu, v)
+
+
+class _KlTerm(torch.autograd.Function):
+    """KL[q(u) || p(u)] of one output GP from its own factorisation (sparse_MF_SP.KLD of a non-whitened model, whose KL
+    depends on K_zz).  The backward is the chain with a zero reduce buffer and gE = 0."""
+
+    @staticmethod
+    def forward(ctx, engine, jitter, Z, raw_ls, raw_os, m, L_raw):
+        engine.set_params(Z.detach(), raw_ls.detach(), raw_os.detach(), m.detach(), L_raw.detach(), None, None)
+        # the status read blocks the host until the factorisation, and the KL behind it, is done (no entry point consumes
+        # the factorisation in this forward): it is also the psd_safe_cholesky check of the reference's KLD
+        kl, _ = prepare_then(engine, lambda: None, check=True, base_jitter=jitter[1], constant_jitter=jitter[0])
+        ctx.engine = engine
+        ctx.generation = engine.generation
+        return kl.clone().reshape(())
+
+    @staticmethod
+    def backward(ctx, g_kl):
+        engine = ctx.engine
+        _check_generation(ctx)
+        g_dev = torch.stack([torch.zeros((), dtype=torch.float64, device=g_kl.device), g_kl.reshape(()).to(torch.float64)])
+        out = engine.chain_backward(engine.new_reduce_buffer(), g_dev=g_dev.contiguous())
+        return None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw']
+
+
+def kl_term(engine, Z, raw_ls, raw_os, m, L_raw, jitter=(0.0, None)):
+    return _KlTerm.apply(engine, tuple(jitter), Z, raw_ls, raw_os, m, L_raw)
 
 
 def qf_covariance(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None)):
