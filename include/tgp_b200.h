@@ -100,6 +100,7 @@ typedef struct TgpReduceLayout {
 } TgpReduceLayout;
 
 const char* tgp_last_error(void);
+/* 101: adds tgp_qf_backward_dx, tgp_flow_mlp_backward_dx and TgpGrads.dX (input gradients); 100: the initial interface */
 int tgp_version(void);
 
 size_t tgp_step_workspace_bytes(const TgpModel* model);
@@ -164,6 +165,11 @@ int tgp_ell_forward(const TgpModel* model, const TgpParams* params, const void* 
  * kernel-parameter gradients are RECOMPUTED from X and Z (K_xz is never written in FP64 for D <= 32). */
 int tgp_qf_backward(const TgpModel* model, const TgpParams* params, const void* step_ws, void* batch_ws,
                     const void* X, long R, const void* g_mu, const void* g_v, double* reduce_buf, void* stream);
+/* tgp_qf_backward, and also the gradient w.r.t. the inputs X of sum_n g_mu[n] mu_n + g_v[n] v_n, ACCUMULATED into the
+ * caller-zeroed dX (R, D) (D <= 64).  dX = NULL computes nothing more: tgp_qf_backward is this call with dX = NULL.  dX is
+ * row-local: under row sharding each rank gets its own rows, and it takes no part in the reduce buffer's all-reduce. */
+int tgp_qf_backward_dx(const TgpModel* model, const TgpParams* params, const void* step_ws, void* batch_ws,
+                       const void* X, long R, const void* g_mu, const void* g_v, double* reduce_buf, void* dX, void* stream);
 
 /* The replicated O(M^3) chain after the all-reduce: (Gbar, Cbar) -> L_S, L^-1 -> L -> K_zz -> Z, lengthscale,
  * outputscale, plus the KL gradient.  Outputs are d(gE*ELL + gK*KL)/dparam in the raw parameterisation:
@@ -234,6 +240,9 @@ int tgp_flow_mlp_forward(const TgpMlp* mlp, const void* weights, const void* X, 
                          void* stream);
 int tgp_flow_mlp_backward(const TgpMlp* mlp, const void* weights, const void* X, long R, const unsigned char* mask,
                           const void* dout, void* dweights, void* stream);
+/* tgp_flow_mlp_backward, and also the gradient w.r.t. X (R, n_in), ACCUMULATED into dX; NULL computes nothing more */
+int tgp_flow_mlp_backward_dx(const TgpMlp* mlp, const void* weights, const void* X, long R, const unsigned char* mask,
+                             const void* dout, void* dweights, void* dX, void* stream);
 
 /* ---- single-call interface (the entry points SURVEY.md 8b proposes), thin over the stages above -------------------
  * A TgpHandle is a HOST object created once per (model description, device, maximum minibatch rows): it remembers the
@@ -258,6 +267,8 @@ typedef struct TgpFwdOut {          /* device pointers; any of ell_rows / mu / v
 typedef struct TgpGrads {           /* device pointers, raw parameterisation; same meaning as tgp_chain_backward's outputs */
     void* dZ; void* draw_lengthscale; void* draw_outputscale; void* dm; void* dL_raw; void* dlog_var_noise; void* dtheta;
     void* drowparams;               /* (R, n_rowparams), NULL when the flow is not input-dependent */
+    void* dX;                       /* (R, D) d(g[0] * ELL)/dX, written; NULL = not computed (tgp_version() >= 101: callers
+                                     * built against an older header must rebuild and zero-initialise the struct) */
 } TgpGrads;
 /* Sum `count` doubles at `buf` over the ranks of the job, enqueued on `stream` (e.g. ncclAllReduce).  NULL = one rank. */
 typedef int (*TgpAllReduceFn)(double* buf, long count, void* user, void* stream);

@@ -53,7 +53,7 @@ class TgpFwdOut(C.Structure):
 
 class TgpGrads(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('dZ', 'draw_lengthscale', 'draw_outputscale', 'dm', 'dL_raw', 'dlog_var_noise',
-                                          'dtheta', 'drowparams')]
+                                          'dtheta', 'drowparams', 'dX')]
 
 
 class TgpMlp(C.Structure):
@@ -84,6 +84,7 @@ SIGNATURES = {
     'tgp_ell_forward': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _D, _P, _P, _I, _P, _P, _P,
                              _P, _P, _P]),
     'tgp_qf_backward': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _L, _P, _P, _P, _P]),
+    'tgp_qf_backward_dx': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _L, _P, _P, _P, _P, _P]),
     'tgp_chain_backward': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _D, _D, _P, _P, _P, _P, _P, _P, _P,
                                 _P, _P]),
     'tgp_test_rows': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _I, _D, _P, _P, _P, _P, _P,
@@ -103,6 +104,7 @@ SIGNATURES = {
     'tgp_flow_mlp_net_doubles': (_L, [C.POINTER(TgpMlp)]),
     'tgp_flow_mlp_forward': (_I, [C.POINTER(TgpMlp), _P, _P, _L, _P, _P, C.c_ulonglong, _P, _P, _P]),
     'tgp_flow_mlp_backward': (_I, [C.POINTER(TgpMlp), _P, _P, _L, _P, _P, _P, _P]),
+    'tgp_flow_mlp_backward_dx': (_I, [C.POINTER(TgpMlp), _P, _P, _L, _P, _P, _P, _P, _P]),
     'tgp_adam_step': (_I, [_I, _L, _P, _P, _P, _P, _P, _P, _D, _D, _D, _P, _P]),
     'tgp_kmeans_iteration': (_I, [_P, _L, _I, _P, _I, _P, _P, _P, _P, _I, _P]),
     'tgp_set_option': (_I, [_I, _I]),

@@ -195,6 +195,108 @@ inline int launch_kernel_grads(const KBT* Kbar, long ldk, const double* X, int x
     return check_launch("k_kernel_grads");
 }
 
+// Input gradients, the row-side twin of the dZ sum of k_kernel_grads:
+//   dX[n,d] += -(1 / ls[d]) * sum_j t[n,j] * (xs[n,d] - zs[j,d]),     t = Kbar[n,j] * os * psi(x_n, z_j)
+// Each warp owns ig_rows(MAXD) rows and loops over all M columns in tiles of 32, lane c taking column j0 + c: Kbar is read
+// coalesced along j, and the tile's Zs rows are staged in shared memory once per CTA (read from L2 once per 8 warps).  No
+// row is split across warps, so dX needs no atomics and the result does not depend on scheduling.  For D <= 16 the warp's
+// scaled rows and each lane's Zs row are held in registers; wider inputs read both from shared memory per use to stay
+// within the register file.  FP64 throughout (a float Kbar is widened); the distance is taken by direct differences, as the FP64 path of
+// k_kernel_grads does.
+constexpr int IG_WARPS = 8, IG_THREADS = 32 * IG_WARPS;
+__host__ __device__ constexpr int ig_rows(int maxd) { return maxd <= 8 ? 2 : 1; }      // rows per warp
+template <int MAXD, typename KBT, int KIND>
+__global__ void __launch_bounds__(IG_THREADS) k_input_grads(const KBT* __restrict__ Kbar, long ldk, const double* __restrict__ X,
+                                                            const double* __restrict__ Zs, const double* __restrict__ ls,
+                                                            const double* __restrict__ os, long R, int M, int D,
+                                                            double* __restrict__ dX) {
+    constexpr int UR = ig_rows(MAXD), ROWS = IG_WARPS * UR;
+    constexpr bool REG = MAXD <= 16;
+    __shared__ double xsh[ROWS][MAXD];
+    __shared__ double zt[32][MAXD + 1];               // the CTA's current tile of Zs rows, shared by its 8 warps
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const long n0 = (long)blockIdx.x * ROWS;
+    for (int i = tid; i < ROWS * D; i += IG_THREADS) {
+        const int r = i / D, d = i % D;
+        const long n = n0 + r;
+        xsh[r][d] = n < R ? X[n * D + d] / ls[d] : 0.0;
+    }
+    __syncthreads();
+    const long nw = n0 + warp * UR;                   // first row of this warp
+    double xr[REG ? UR : 1][REG ? MAXD : 1];
+    if constexpr (REG) {
+#pragma unroll
+        for (int u = 0; u < UR; ++u)
+#pragma unroll
+            for (int d = 0; d < MAXD; ++d) xr[u][d] = d < D ? xsh[warp * UR + u][d] : 0.0;
+    }
+    const double s = os[0];
+    double acc[UR][MAXD];
+#pragma unroll
+    for (int u = 0; u < UR; ++u)
+#pragma unroll
+        for (int d = 0; d < MAXD; ++d) acc[u][d] = 0.0;
+    for (int j0 = 0; j0 < M; j0 += 32) {
+        __syncthreads();                              // the previous tile has been read
+        for (int i = tid; i < 32 * D; i += IG_THREADS) {
+            const int c = i / D, d = i % D;
+            zt[c][d] = j0 + c < M ? Zs[(long)(j0 + c) * D + d] : 0.0;
+        }
+        __syncthreads();
+        const int j = j0 + lane;
+        if (nw >= R || j >= M) continue;
+        double zj[REG ? MAXD : 1];
+        if constexpr (REG) {
+#pragma unroll
+            for (int d = 0; d < MAXD; ++d) zj[d] = d < D ? zt[lane][d] : 0.0;
+        }
+        double kb[UR];
+#pragma unroll
+        for (int u = 0; u < UR; ++u) kb[u] = nw + u < R ? (double)Kbar[(nw + u) * ldk + j] : 0.0;
+#pragma unroll
+        for (int u = 0; u < UR; ++u) {          // rows past R carry kb = 0 and add nothing
+            // wide inputs take the differences twice rather than hold them (the register file would not)
+            auto diff = [&](int d) {
+                if constexpr (REG) return xr[u][d] - zj[d];
+                else return d < D ? xsh[warp * UR + u][d] - zt[lane][d] : 0.0;
+            };
+            double q = 0.0;
+#pragma unroll
+            for (int d = 0; d < MAXD; ++d) { const double df = diff(d); q = fma(df, df, q); }
+            double ph, ps;
+            Cov<KIND>::phi_psi(q, ph, ps);
+            const double t = kb[u] * s * ps;
+#pragma unroll
+            for (int d = 0; d < MAXD; ++d) acc[u][d] = fma(t, diff(d), acc[u][d]);
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < UR; ++u) {
+        const long n = nw + u;
+#pragma unroll
+        for (int d = 0; d < MAXD; ++d) {
+            if (d >= D) break;
+            const double v = warp_sum(acc[u][d]);
+            if (lane == 0 && n < R) dX[n * D + d] -= v / ls[d];
+        }
+    }
+}
+
+template <int KIND, typename KBT>
+inline int launch_input_grads(const KBT* Kbar, long ldk, const double* X, const double* Zs, const double* ls, const double* os,
+                              long R, int M, int D, double* dX, cudaStream_t st) {
+#define TGP_IG(MD) k_input_grads<MD, KBT, KIND><<<(unsigned)cdiv(R, IG_WARPS * ig_rows(MD)), IG_THREADS, 0, st>>>(Kbar, ldk, X, Zs, ls, \
+                                                                                                             os, R, M, D, dX)
+    if (D <= 4) TGP_IG(4);
+    else if (D <= 8) TGP_IG(8);
+    else if (D <= 16) TGP_IG(16);
+    else if (D <= 32) TGP_IG(32);
+    else if (D <= 64) TGP_IG(64);
+    else return set_error(-2, "input dimension > 64 not supported by the input-gradient kernel");
+#undef TGP_IG
+    return check_launch("k_input_grads");
+}
+
 // Final raw-parameter gradients of gE*ELL + gK*KL  (softplus' = sigmoid; KL: dm = m, dL_S = L_S - diag(1/L_ii)).
 __global__ void k_finalize_small(const double* __restrict__ raw_ls, const double* __restrict__ raw_os,
                                  const double* __restrict__ m, int M, int D, int n_theta, double gE, double gK,

@@ -319,7 +319,7 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchView& 
 
 template <int KIND>
 inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
-                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
                          cudaStream_t st) {
     const int M = s.M, D = s.D;
     TGP_TRY(fill_int(b.zero_exp, 1, 0, st));
@@ -363,6 +363,7 @@ inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchVie
         // reconstruction of Kbar, then Kbar o K -> dZ, dlengthscale, doutputscale
         TGP_TRY(combine(b.Kbp, b.ldk, (long)b.Rc * b.ldk, rc, M, Tb, bits_x + bits_w, b.zero_exp, 2, b.wc_exp, 1, b.Kbar, M, 0, 0, st));
         TGP_TRY(launch_kernel_grads<KIND>(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, kval ? kval + r0 * M : nullptr, M));
+        if (dX) TGP_TRY(launch_input_grads<KIND>(b.Kbar, M, X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, dX + r0 * D, st));
         {   // [Gbar; Cbar] (2M x M) += ABbar^T K: reduction over the chunk rows; both operands are row-major planes read MN-major
             i8::Params p{};
             p.Mrows = 2 * M; p.Ncols = M; p.K = rc; p.T = Tw; p.tri_mode = 0; p.tri_rows = 0; p.lower_rows = M; p.mn_major = 3;
@@ -380,10 +381,10 @@ inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchVie
 }
 
 inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchView& b, const double* X, long R, const double* g_mu,
-                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
                        cudaStream_t st) {
     return with_kernel(s.kind, [&](auto k) {
-        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, dX, st);
     });
 }
 

@@ -83,7 +83,8 @@ inline int qf_forward(const StepView& s, const BatchView& b, const double* X, lo
 //   Gbar += tril(Abar^T K);  dL_S += tril(A^T Bbar)   (accumulated in the `Cbar` slot of the reduce buffer)
 template <int KIND>
 inline int qf_backward_k(const StepView& s, const BatchView& b, const double* X, long R, const double* g_mu, const double* g_v,
-                         double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, cudaStream_t st) {
+                         double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
+                         cudaStream_t st) {
     const int M = s.M, D = s.D;
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
         const int rc = (int)((R - r0) < b.Rc ? (R - r0) : b.Rc);
@@ -104,6 +105,7 @@ inline int qf_backward_k(const StepView& s, const BatchView& b, const double* X,
         TGP_TRY(gemm_f64(g1, st));
         // the RBF reads K from Kc; the other kinds recompute it (launch_kernel_grads)
         TGP_TRY(launch_kernel_grads<KIND>(b.Kbar, M, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st, Kc, M));
+        if (dX) TGP_TRY(launch_input_grads<KIND>(b.Kbar, M, X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, dX + r0 * D, st));
         // Gbar += tril(Abar^T K)      (reduction over the rows of the chunk)
         GemmArgs g3 = make_gemm(M, M, rc, b.Abar, M, 1, Kc, M, 1, Gbar, s.Mp, 1.0, 1.0);
         g3.c_lower = 1; g3.splitk = weight_splitk(M, rc, true); g3.tag = 1;
@@ -117,9 +119,10 @@ inline int qf_backward_k(const StepView& s, const BatchView& b, const double* X,
 }
 
 inline int qf_backward(const StepView& s, const BatchView& b, const double* X, long R, const double* g_mu, const double* g_v,
-                       double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, cudaStream_t st) {
+                       double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
+                       cudaStream_t st) {
     return with_kernel(s.kind, [&](auto k) {
-        return qf_backward_k<decltype(k)::value>(s, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+        return qf_backward_k<decltype(k)::value>(s, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, dX, st);
     });
 }
 

@@ -13,7 +13,8 @@
 //   2  explicit mask supplied by the caller (parity mode: the reference's masks come from torch's global RNG and cannot
 //      be regenerated, SURVEY.md §7.7).
 // The backward recomputes the forward of each row, then back-propagates analytically; weight gradients are accumulated
-// per CTA in shared memory (FP64 shared atomics) and flushed with one global atomic per weight per CTA.
+// per CTA in shared memory (FP64 shared atomics) and flushed with one global atomic per weight per CTA.  Input gradients
+// (dX, optional, k_flow_mlp<true, true>) are added per row by the warp that owns the row.
 #pragma once
 #include "common.cuh"
 #include "../../../include/tgp_b200.h"
@@ -35,6 +36,7 @@ struct MlpArgs {
     double* out;                // forward: R x n_nets
     const double* dout;         // backward: R x n_nets
     double* dW;                 // backward: n_nets x net_size, accumulated
+    double* dX;                 // backward: R x n_in, accumulated; NULL = not computed
 };
 
 __host__ __device__ inline int mlp_net_size(int n_in, int H, int L) { return H * n_in + H + (L - 1) * (H * H + H) + H + 1; }
@@ -69,7 +71,9 @@ __device__ __forceinline__ double mlp_act(int act, double z, double& dz) {
     dz = 1.0; return z;                                                              // linear
 }
 
-template <bool BWD>
+// DX (backward only): also the input gradients, in an instantiation of its own, so that the forward and the plain backward
+// compile exactly as without it
+template <bool BWD, bool DX = false>
 __global__ void __launch_bounds__(MLP_THREADS) k_flow_mlp(MlpArgs a) {
     extern __shared__ double sm_mlp[];
     const int nsz = mlp_net_size(a.n_in, a.H, a.L);
@@ -153,6 +157,15 @@ __global__ void __launch_bounds__(MLP_THREADS) k_flow_mlp(MlpArgs a) {
                 }
                 __syncwarp();
             }
+            if constexpr (DX) {     // dX[row] += W_0^T dz_0: a row belongs to one warp for every net, so no atomics
+                const double* dz0 = dzb + 64 * cur;
+                for (int k = lane; k < nin; k += 32) {
+                    double s = 0.0;
+#pragma unroll 1
+                    for (int h = 0; h < H; ++h) s = fma(w[h * nin + k], dz0[h], s);
+                    a.dX[row * nin + k] += s;
+                }
+            }
         }
         if (BWD) {
             __syncthreads();
@@ -181,13 +194,15 @@ inline int launch_flow_mlp(const TgpMlp* m, MlpArgs a, bool bwd, cudaStream_t st
     const int nsz = mlp_net_size(m->n_in, m->hidden, m->n_hidden_layers);
     const size_t smem = ((size_t)nsz * (bwd ? 2 : 1) + (size_t)MLP_WARPS * 64 * (1 + 2 * MLP_MAX_LAYERS + 2)) * sizeof(double);
     if (smem > 200 * 1024) return set_error(-2, "flow MLP too large for shared memory");
-    static PerDeviceOnce once_f, once_b;
-    if (bwd) { if (once_b.first()) cudaFuncSetAttribute(k_flow_mlp<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); }
+    static PerDeviceOnce once_f, once_b, once_dx;
+    if (bwd && a.dX) { if (once_dx.first()) cudaFuncSetAttribute(k_flow_mlp<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); }
+    else if (bwd) { if (once_b.first()) cudaFuncSetAttribute(k_flow_mlp<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); }
     else { if (once_f.first()) cudaFuncSetAttribute(k_flow_mlp<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); }
     long blocks = cdiv(a.R, MLP_WARPS);
     if (blocks > 148 * 2) blocks = 148 * 2;
     if (blocks < 1) blocks = 1;
-    if (bwd) k_flow_mlp<true><<<(unsigned)blocks, MLP_THREADS, smem, st>>>(a);
+    if (bwd && a.dX) k_flow_mlp<true, true><<<(unsigned)blocks, MLP_THREADS, smem, st>>>(a);
+    else if (bwd) k_flow_mlp<true><<<(unsigned)blocks, MLP_THREADS, smem, st>>>(a);
     else k_flow_mlp<false><<<(unsigned)blocks, MLP_THREADS, smem, st>>>(a);
     return check_launch("k_flow_mlp");
 }

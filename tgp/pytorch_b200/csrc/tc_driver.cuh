@@ -105,7 +105,7 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes
 // backward: ABbar planes (+transposes), K^T planes; Kbar = ABbar Wt^T; kernel gradients; Gbar / Cbar += ABbar^T K
 template <int KIND>
 inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
-                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                         const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
                          cudaStream_t st) {
     const int M = s.M, D = s.D;
     for (long r0 = 0; r0 < R; r0 += b.Rc) {
@@ -133,6 +133,7 @@ inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchPla
         // the RBF reads K from the planes; the other kinds recompute it (launch_kernel_grads)
         TGP_TRY((launch_kernel_grads<KIND, float>(b.Kbar, b.ldk, X + r0 * D, 0, s.Zs, s.ls, s.os, rc, M, D, 0, 1.0, dZ, dls, dos, st,
                                                   nullptr, 0, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk)));
+        if (dX) TGP_TRY(launch_input_grads<KIND>(b.Kbar, b.ldk, X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, dX + r0 * D, st));
         const int kblocks = (rc + BK - 1) / BK;
         int split = (int)cdiv(2 * 148, cdiv(M, BM) * cdiv(M, BN));
         if (split > kblocks / 8) split = kblocks / 8 > 0 ? kblocks / 8 : 1;
@@ -157,10 +158,10 @@ inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchPla
 }
 
 inline int qf_backward(const StepView& s, const StepPlanes& sp, const BatchPlanes& b, const double* X, long R, const double* g_mu,
-                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar,
+                       const double* g_v, double* dm, double* dos, double* dZ, double* dls, double* Gbar, double* Cbar, double* dX,
                        cudaStream_t st) {
     return with_kernel(s.kind, [&](auto k) {
-        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, st);
+        return qf_backward_k<decltype(k)::value>(s, sp, b, X, R, g_mu, g_v, dm, dos, dZ, dls, Gbar, Cbar, dX, st);
     });
 }
 

@@ -141,7 +141,7 @@ using namespace tgp;
 extern "C" {
 
 const char* tgp_last_error(void) { return g_last_error; }
-int tgp_version(void) { return 100; }
+int tgp_version(void) { return 101; }
 
 size_t tgp_step_workspace_bytes(const TgpModel* md) {
     if (validate(md)) return 0;
@@ -307,10 +307,16 @@ int tgp_ell_forward(const TgpModel* md, const TgpParams* p, const void* mu, cons
 
 int tgp_qf_backward(const TgpModel* md, const TgpParams* p, const void* step_ws, void* batch_ws, const void* X,
                     long R, const void* g_mu, const void* g_v, double* reduce_buf, void* stream) {
+    return tgp_qf_backward_dx(md, p, step_ws, batch_ws, X, R, g_mu, g_v, reduce_buf, nullptr, stream);
+}
+
+int tgp_qf_backward_dx(const TgpModel* md, const TgpParams* p, const void* step_ws, void* batch_ws, const void* X,
+                       long R, const void* g_mu, const void* g_v, double* reduce_buf, void* dX, void* stream) {
     TGP_TRY(validate(md));
     if (R <= 0) return 0;
     if (!p || !step_ws || !batch_ws || !X || !g_mu || !g_v || !reduce_buf)
         return set_error(-1, "NULL argument to tgp_qf_backward");
+    if (dX && md->D > 64) return set_error(-2, "input gradients need D <= 64");
     cudaStream_t st = (cudaStream_t)stream;
     const int M = md->M, D = md->D;
     Carve cs(const_cast<void*>(step_ws)), cb(batch_ws);
@@ -320,12 +326,13 @@ int tgp_qf_backward(const TgpModel* md, const TgpParams* p, const void* step_ws,
     const double *gm = (const double*)g_mu, *gv = (const double*)g_v;
     double *dm = reduce_buf + l.dm, *dos = reduce_buf + l.dos, *dZ = reduce_buf + l.dZ, *dls = reduce_buf + l.dls;
     double *Gbar = reduce_buf + l.Gbar, *Cbar = reduce_buf + l.Cbar;
+    double* dXd = (double*)dX;
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
     if (md->dtype == TGP_F32)
-        return tc::qf_backward(w.f64, w.tc, tc::batch_planes(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
+        return tc::qf_backward(w.f64, w.tc, tc::batch_planes(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, dXd, st);
     if (md->dtype == TGP_F64_I8)
-        return crt::qf_backward(w.f64, w.crt, crt::batch_view(cb, M, D, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
-    return f64::qf_backward(w.f64, f64::batch_view(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, st);
+        return crt::qf_backward(w.f64, w.crt, crt::batch_view(cb, M, D, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, dXd, st);
+    return f64::qf_backward(w.f64, f64::batch_view(cb, M, R), Xd, R, gm, gv, dm, dos, dZ, dls, Gbar, Cbar, dXd, st);
 }
 
 int tgp_chain_backward(const TgpModel* md, const TgpParams* p, void* step_ws, const double* reduce_buf, double gE,
@@ -556,6 +563,11 @@ int tgp_flow_mlp_forward(const TgpMlp* m, const void* weights, const void* X, lo
 
 int tgp_flow_mlp_backward(const TgpMlp* m, const void* weights, const void* X, long R, const unsigned char* mask,
                           const void* dout, void* dweights, void* stream) {
+    return tgp_flow_mlp_backward_dx(m, weights, X, R, mask, dout, dweights, nullptr, stream);
+}
+
+int tgp_flow_mlp_backward_dx(const TgpMlp* m, const void* weights, const void* X, long R, const unsigned char* mask,
+                             const void* dout, void* dweights, void* dX, void* stream) {
     TGP_TRY(mlp_validate(m));
     if (R <= 0) return 0;
     if (!weights || !X || !dout || !dweights) return set_error(-1, "NULL argument to tgp_flow_mlp_backward");
@@ -564,6 +576,7 @@ int tgp_flow_mlp_backward(const TgpMlp* m, const void* weights, const void* X, l
     a.n_nets = m->n_nets; a.n_in = m->n_in; a.H = m->hidden; a.L = m->n_hidden_layers; a.act = m->activation;
     a.mask_mode = m->mask_mode; a.p_drop = m->p_drop; a.R = R;
     a.W = (const double*)weights; a.X = (const double*)X; a.mask_in = mask; a.dout = (const double*)dout; a.dW = (double*)dweights;
+    a.dX = (double*)dX;
     return launch_flow_mlp(m, a, true, (cudaStream_t)stream);
 }
 
@@ -607,6 +620,10 @@ namespace tgp {
 __global__ void k_fwd_terms(const double* __restrict__ rb_ell, const double* __restrict__ kl, double scale, double* __restrict__ terms) {
     terms[0] = scale * rb_ell[0];
     terms[1] = kl[0];
+}
+__global__ void k_scale_by_dev(double* __restrict__ x, long n, const double* __restrict__ g) {
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) x[i] *= g[0];
 }
 inline int handle_ready(TgpHandle* h, const TgpBatch* b) {
     if (!h) return set_error(-1, "handle is NULL");
@@ -676,7 +693,14 @@ int tgp_elbo_bwd(TgpHandle* h, const TgpParams* p, const TgpBatch* b, const doub
         return set_error(-1, "input-dependent flows: use the staged entry points (drowparams flows back to the caller's MLP)");
     const TgpReduceLayout l = reduce_layout(md);
     const HandleView& w = h->ws;
-    TGP_TRY(tgp_qf_backward(md, p, w.step, w.batch, b->X, b->R, w.g_mu, w.g_v, w.reduce, stream));
+    if (g->dX && cudaMemsetAsync(g->dX, 0, (size_t)b->R * md->D * sizeof(double), (cudaStream_t)stream) != cudaSuccess)
+        return set_error(-100, "zeroing dX failed");
+    TGP_TRY(tgp_qf_backward_dx(md, p, w.step, w.batch, b->X, b->R, w.g_mu, w.g_v, w.reduce, g->dX, stream));
+    if (g->dX && b->R > 0) {         // dX is row-local (never all-reduced); the ELL weight g_dev[0] is applied here
+        const long n = b->R * md->D;
+        k_scale_by_dev<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((double*)g->dX, n, g_dev);
+        TGP_TRY(check_launch("k_scale_by_dev"));
+    }
     if (allreduce) {
         TGP_TRY(tgp_reduce_pack(md, w.reduce, w.packed, stream));
         if (allreduce(w.packed, l.packed_total, user, stream) != 0) return set_error(-103, "the all-reduce callback failed");

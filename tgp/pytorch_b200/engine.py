@@ -305,12 +305,20 @@ class Engine:
         return ell_rows, g_mu, g_v, drow
 
     @_on_device
-    def qf_backward(self, X, g_mu, g_v, reduce_buf):
+    def qf_backward(self, X, g_mu, g_v, reduce_buf, dX=None):
+        """Accumulates the pre-chain sums into reduce_buf; with dX (R, D), zeroed by the caller, also accumulates there the
+        gradient of sum_n g_mu[n] mu_n + g_v[n] v_n w.r.t. the rows of X."""
         R = X.shape[0]
         _chk(g_mu, 'g_mu', (R,)); _chk(g_v, 'g_v', (R,))
-        _lib.check(self.lib.tgp_qf_backward(self.model, self._params, _ptr(self.step_ws), _ptr(self.batch_ws(R)),
-                                            _ptr(X), R, _ptr(g_mu), _ptr(g_v), _ptr(reduce_buf), _stream(self.device)),
-                   'tgp_qf_backward')
+        if dX is None:
+            _lib.check(self.lib.tgp_qf_backward(self.model, self._params, _ptr(self.step_ws), _ptr(self.batch_ws(R)),
+                                                _ptr(X), R, _ptr(g_mu), _ptr(g_v), _ptr(reduce_buf), _stream(self.device)),
+                       'tgp_qf_backward')
+            return
+        _chk(dX, 'dX', (R, self.D))
+        _lib.check(self.lib.tgp_qf_backward_dx(self.model, self._params, _ptr(self.step_ws), _ptr(self.batch_ws(R)),
+                                               _ptr(X), R, _ptr(g_mu), _ptr(g_v), _ptr(reduce_buf), _ptr(dX),
+                                               _stream(self.device)), 'tgp_qf_backward_dx')
 
     @_on_device
     def chain_backward(self, reduce_buf, gE=1.0, gK=-1.0, g_dev=None):

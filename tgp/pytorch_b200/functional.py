@@ -152,7 +152,7 @@ class _ElboTerms(torch.autograd.Function):
     @staticmethod
     def forward(ctx, engine, X, Y, scale, check_status, jitter, sync_ell, Z, raw_ls, raw_os, m, L_raw, log_var_noise, theta,
                 rowparams):
-        need_grad = any(ctx.needs_input_grad[7:])
+        need_grad = ctx.needs_input_grad[1] or any(ctx.needs_input_grad[7:])
         engine.set_params(Z.detach(), raw_ls.detach(), raw_os.detach(), m.detach(), L_raw.detach(),
                           None if log_var_noise is None else log_var_noise.detach(),
                           None if theta is None else theta.detach())
@@ -182,15 +182,17 @@ class _ElboTerms(torch.autograd.Function):
         if g_mu is None:
             raise RuntimeError('backward called on an ELBO evaluated without gradients')
         _check_generation(ctx)
-        engine.qf_backward(X, g_mu, g_v, rb)
-        allreduce_packed(engine, rb)               # the one collective of the step (SURVEY.md §8e)
+        dX = torch.zeros_like(X) if ctx.needs_input_grad[1] else None
+        engine.qf_backward(X, g_mu, g_v, rb, dX)
+        allreduce_packed(engine, rb)               # the one collective of the step (SURVEY.md §8e); dX is row-local
         engine.last_ell_sum = rb[engine.layout.ell_sum]        # global sum_n ell_n (unscaled), valid after backward
         zero = torch.zeros((), dtype=torch.float64, device=rb.device)
         g_dev = torch.stack([g_ell if g_ell is not None else zero, g_kl if g_kl is not None else zero]).contiguous()
         out = engine.chain_backward(rb, 0.0, 0.0, g_dev=g_dev)
         has_noise, has_theta, has_rowp = ctx.has
         g_rowp = drow * g_dev[0] if (has_rowp and drow is not None) else None
-        return (None, None, None, None, None, None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw'],
+        g_X = dX * g_dev[0] if dX is not None else None            # the KL does not depend on X
+        return (None, g_X, None, None, None, None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw'],
                 out['log_var_noise'] if has_noise else None, out['theta'] if has_theta else None, g_rowp)
 
 
@@ -240,14 +242,15 @@ class _QfMarginals(torch.autograd.Function):
         _check_generation(ctx)
         rb = engine.new_reduce_buffer()
         zeros = torch.zeros(X.shape[0], dtype=torch.float64, device=X.device)
-        engine.qf_backward(X, zeros if g_mu is None else g_mu.contiguous(), zeros if g_v is None else g_v.contiguous(), rb)
+        dX = torch.zeros_like(X) if ctx.needs_input_grad[1] else None
+        engine.qf_backward(X, zeros if g_mu is None else g_mu.contiguous(), zeros if g_v is None else g_v.contiguous(), rb, dX)
         allreduce_packed(engine, rb)               # row-sharded callers (multiclass ELBO): sum over ranks before the chain
         if g_kl is None:
             out = engine.chain_backward(rb, 1.0, 0.0)
         else:
             g_dev = torch.stack([torch.ones((), dtype=torch.float64, device=X.device), g_kl.reshape(()).to(torch.float64)])
             out = engine.chain_backward(rb, g_dev=g_dev.contiguous())
-        return None, None, None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw']
+        return None, dX, None, None, out['Z'], out['raw_ls'], out['raw_os'], out['m'], out['L_raw']
 
 
 def qf_marginals(engine, X, Z, raw_ls, raw_os, m, L_raw, check_status=True, jitter=(0.0, None), with_kl=False):
@@ -408,6 +411,7 @@ class _FlowMlp(torch.autograd.Function):
         if owner is not None:
             owner.last_dropout_masks = used                  # exported keep-mask of this call (None when dropout is off)
         ctx.m, ctx.Xc, ctx.Wp, ctx.mask, ctx.shapes, ctx.dtypes = m, Xc, Wp, used, [w.shape for w in weights], [w.dtype for w in weights]
+        ctx.x_dtype = X.dtype
         return out
 
     @staticmethod
@@ -416,12 +420,17 @@ class _FlowMlp(torch.autograd.Function):
         lib = _lib.load()
         dev = ctx.Xc.device
         dW = torch.zeros_like(ctx.Wp)
+        dX = torch.zeros_like(ctx.Xc) if ctx.needs_input_grad[0] else None
         d = dout.to(torch.float64).contiguous()
         with torch.cuda.device(dev):
             st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(lib.tgp_flow_mlp_backward(ctx.m, ctx.Wp.data_ptr(), ctx.Xc.data_ptr(), ctx.Xc.shape[0],
-                                                 None if ctx.mask is None else ctx.mask.data_ptr(), d.data_ptr(), dW.data_ptr(), st),
-                       'tgp_flow_mlp_backward')
+            mask = None if ctx.mask is None else ctx.mask.data_ptr()
+            if dX is None:
+                _lib.check(lib.tgp_flow_mlp_backward(ctx.m, ctx.Wp.data_ptr(), ctx.Xc.data_ptr(), ctx.Xc.shape[0], mask, d.data_ptr(),
+                                                     dW.data_ptr(), st), 'tgp_flow_mlp_backward')
+            else:
+                _lib.check(lib.tgp_flow_mlp_backward_dx(ctx.m, ctx.Wp.data_ptr(), ctx.Xc.data_ptr(), ctx.Xc.shape[0], mask,
+                                                        d.data_ptr(), dW.data_ptr(), dX.data_ptr(), st), 'tgp_flow_mlp_backward_dx')
         dist = _world()
         if dist is not None:
             dist.all_reduce(dW)          # each rank saw its own rows only: ONE collective for all MLP weights of the layer
@@ -432,9 +441,9 @@ class _FlowMlp(torch.autograd.Function):
                 n *= k
             grads.append(dW[o:o + n].reshape(shp).to(dt))
             o += n
-        return (None, None, None, None, None) + tuple(grads)
+        return (None if dX is None else dX.to(ctx.x_dtype), None, None, None, None) + tuple(grads)
 
 
 def flow_mlp(owner, nets, spec, X, mask_in=None):
-    """theta(x_n) of `len(nets)` flow MLPs in one kernel: (R, n_nets).  Differentiable w.r.t. the MLP weights."""
+    """theta(x_n) of `len(nets)` flow MLPs in one kernel: (R, n_nets).  Differentiable w.r.t. the MLP weights and X."""
     return _FlowMlp.apply(X, spec, mask_in, owner, len(nets), *_mlp_weights(nets))

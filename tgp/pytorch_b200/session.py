@@ -67,9 +67,10 @@ class ElboSession:
             _lib.check(self.lib.tgp_elbo_fwd(self.handle, p, self._batch, float(jitter), fo, _stream(self.device)), 'tgp_elbo_fwd')
         return out
 
-    def backward(self, g_dev, allreduce=None):
+    def backward(self, g_dev, allreduce=None, input_grad=False):
         """Gradients of g_dev[0] * ELL + g_dev[1] * KL (g_dev: device tensor of 2 doubles).  `allreduce(tensor)` — called
-        once on the tril-packed exchange buffer — makes the step row-sharded (e.g. torch.distributed.all_reduce)."""
+        once on the tril-packed exchange buffer — makes the step row-sharded (e.g. torch.distributed.all_reduce).
+        input_grad=True also returns out['X'], the gradient w.r.t. the rows of X of the last forward (this rank's rows)."""
         eng, dev, f64 = self.eng, self.device, torch.float64
         M, D = eng.M, eng.D
         out = dict(Z=torch.empty(M, D, dtype=f64, device=dev), raw_ls=torch.empty(D, dtype=f64, device=dev),
@@ -80,6 +81,9 @@ class ElboSession:
         g.dZ, g.draw_lengthscale, g.draw_outputscale = out['Z'].data_ptr(), out['raw_ls'].data_ptr(), out['raw_os'].data_ptr()
         g.dm, g.dL_raw, g.dlog_var_noise = out['m'].data_ptr(), out['L_raw'].data_ptr(), out['log_var_noise'].data_ptr()
         g.dtheta = out['theta'].data_ptr() if eng.flow.n_theta else None
+        if input_grad:
+            out['X'] = torch.empty(self._batch.R, D, dtype=f64, device=dev)
+            g.dX = out['X'].data_ptr()
         cb = _lib.ALLREDUCE_FN(0)
         if allreduce is not None:
             n_packed = eng.layout.packed_total
