@@ -100,7 +100,8 @@ typedef struct TgpReduceLayout {
 } TgpReduceLayout;
 
 const char* tgp_last_error(void);
-/* 101: adds tgp_qf_backward_dx, tgp_flow_mlp_backward_dx and TgpGrads.dX (input gradients); 100: the initial interface */
+/* 102: retires library option 1 (tgp_set_option); 101: adds tgp_qf_backward_dx, tgp_flow_mlp_backward_dx and TgpGrads.dX
+ * (input gradients); 100: the initial interface */
 int tgp_version(void);
 
 size_t tgp_step_workspace_bytes(const TgpModel* model);
@@ -309,13 +310,10 @@ int tgp_adam_step(int n_tensors, long n_blocks, const void* const* ptr_table, co
 int tgp_kmeans_iteration(const void* X, long N, int D, void* C, int M, int* assign, double* sums, double* counts,
                          double* inertia, int update, void* stream);
 
-/* Library options.  TGP_OPT_FUSED_FORWARD (tensor-core mode): 1 = tgp_qf_forward is ONE kernel that generates the K_xz
- * tiles inside the tcgen05 contraction and emits mu, v from the TMEM accumulators; 0 = staged planes + separate kernels.
- * The fused kernel generates RBF tiles only: a model with a Matern kernel (or D above the fused kernel's limit) takes the
- * staged path whatever the option says, and its backward reuses the K planes that path kept.
+/* Library options.  Key 1 (the single-kernel tensor-core forward) is retired: it is an unknown option since tgp_version() 102.
  * TGP_OPT_ROW_CHUNK (FP64 mode): rows per launch of the batch contractions (default 32768; a tuning knob — it changes the
  * workspace size, so set it before asking for tgp_batch_workspace_bytes). */
-enum { TGP_OPT_FUSED_FORWARD = 1, TGP_OPT_ROW_CHUNK = 2,
+enum { TGP_OPT_ROW_CHUNK = 2,
        TGP_OPT_OVERLAP_KGEN = 3 };   /* 1 (default): tgp_prepare forks the factorisation onto a library-owned high-priority stream;
                                       * tgp_qf_forward enqueues K_xz generation on the caller's stream and joins afterwards, every
                                       * other consumer of the step workspace joins first; 0: everything on the caller's stream.

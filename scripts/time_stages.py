@@ -26,8 +26,6 @@ from tgp.pytorch_b200 import _lib
 if os.environ.get('TGP_ROW_CHUNK'):
     _lib.load().tgp_set_option(_lib.OPT_ROW_CHUNK, int(os.environ['TGP_ROW_CHUNK']))
 for compute in sys.argv[1:] or ['f64', 'i8crt', 'tf32x3']:
-    _lib.load().tgp_set_option(_lib.OPT_FUSED_FORWARD, 1 if compute.endswith('+fused') else 0)
-    label, compute = compute, compute.split('+')[0]
     eng, theta, _, _ = make_engine(p, WL['likelihood'], 100, dev, compute=compute)
     ei = engine_inputs(p, dev)
     eng.set_params(ei['Z'], ei['raw_ls'], ei['raw_os'], ei['m'], ei['L_raw'], ei['log_var_noise'], theta)
@@ -45,4 +43,4 @@ for compute in sys.argv[1:] or ['f64', 'i8crt', 'tf32x3']:
     bstd = v.std().reshape(1) if WL['likelihood'] == 'bernoulli' else None
     t_test, _ = timed(lambda: eng.test_rows(mu, v, yb, None, 1, 1.0, bstd))
     print('%-13s prepare %.3f  qf_forward %.3f  ell %.3f  qf_backward %.3f  chain %.3f  test_rows %.3f  | sum %.3f ms'
-          % (label, t_prep, t_fwd, t_ell, t_fb - t_fwd, t_chain, t_test, t_prep + t_fwd + t_ell + (t_fb - t_fwd) + t_chain))
+          % (compute, t_prep, t_fwd, t_ell, t_fb - t_fwd, t_chain, t_test, t_prep + t_fwd + t_ell + (t_fb - t_fwd) + t_chain))

@@ -255,19 +255,3 @@ def test_handle_api_matches_the_staged_entry_points():
     for k, n in (('Z', 'Z'), ('raw_ls', 'raw_lengthscale'), ('raw_os', 'raw_outputscale'), ('m', 'm'), ('L_raw', 'L_raw')):
         assert rel_err(grads[k].cpu().reshape(-1), staged[n]) < 1e-12, k
     ses.close()
-
-
-def test_fused_forward_option_leaves_matern_models_on_the_staged_path():
-    from tgp.pytorch_b200 import _lib
-    lib = _lib.load()
-    X, y, p = _problem(1000, 64, 8, seed=29, kernel='matern52')
-    out = {}
-    try:
-        for fused in (0, 1):
-            lib.tgp_set_option(_lib.OPT_FUSED_FORWARD, fused)
-            out[fused], _ = _cuda(X, y, p, 5000.0, 'gauss_nonlinear', 30, 'tf32x3')
-    finally:
-        lib.tgp_set_option(_lib.OPT_FUSED_FORWARD, 0)
-    # same kernels either way; mu and the reduce accumulators are FP64 atomics, whose order may differ between runs
-    for k in out[0]:
-        assert rel_err(out[1][k], out[0][k]) < 1e-9, k

@@ -177,14 +177,14 @@ def test_minibatch_stager_has_no_cpu_path():
         PinnedMinibatchStager(X, Y, 4, 'cpu')
 
 
-def test_library_options_and_workspace_sizing_without_a_gpu():
-    """Option ids in the ctypes binding equal the header's enum; the row-chunk option is validated and changes the batch
-    workspace size it documents (pure host code: no kernel is launched)."""
+def test_library_options_retired_key_and_workspace_sizing_without_a_gpu():
+    """Option ids in the ctypes binding equal the header's enum and the retired key 1 is rejected as unknown; the row-chunk
+    option is validated and changes the batch workspace size it documents (pure host code: no kernel is launched)."""
     from tgp.pytorch_b200 import _lib
     lib = _lib.load()
     header = open(os.path.join(ROOT, 'include', 'tgp_b200.h')).read()
     enum = dict(re.findall(r'(TGP_OPT_[A-Z_]+)\s*=\s*(\d+)', header))
-    assert int(enum['TGP_OPT_FUSED_FORWARD']) == _lib.OPT_FUSED_FORWARD
+    assert '1' not in enum.values()                      # key 1 (the retired single-kernel tensor-core forward) is unknown
     assert int(enum['TGP_OPT_ROW_CHUNK']) == _lib.OPT_ROW_CHUNK
     m = _lib.TgpModel()
     m.dtype, m.M, m.D, m.likelihood, m.n_quad = _lib.TGP_F64, 256, 4, 1, 30
@@ -197,6 +197,7 @@ def test_library_options_and_workspace_sizing_without_a_gpu():
         # [A|B] (2M) and K_xz (M) are per row; the two staging buffers (M each) are per chunk
         assert small >= 8 * (3 * 256 * R + 2 * 256 * 8192) and large - small == 8 * 2 * 256 * (65536 - 8192)
         assert lib.tgp_set_option(_lib.OPT_ROW_CHUNK, 64) != 0 and b'row chunk' in lib.tgp_last_error()
+        assert lib.tgp_set_option(1, 1) != 0 and b'unknown option' in lib.tgp_last_error()
         assert lib.tgp_set_option(99, 1) != 0
     finally:
         assert lib.tgp_set_option(_lib.OPT_ROW_CHUNK, 32768) == 0

@@ -30,14 +30,14 @@ def _mlp(n_in=4):
     return m
 
 
-def test_exports_and_version():
+def test_exports_and_interface_version_102():
     text = open(HEADER).read()
     for name in NEW:
         assert name + '(' in text and name in _lib.SIGNATURES
     lib = _lib_or_skip()
     for name in NEW:
         assert hasattr(lib, name)
-    assert lib.tgp_version() == 101
+    assert lib.tgp_version() == 102
 
 
 def test_grads_struct_layout():

@@ -17,7 +17,6 @@ KERNEL_RBF, KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2, 3
 QU_WHITENED, QU_UNWHITENED = 0, 1
 FLOW_RESTRICT, FLOW_ADD_F0, FLOW_PER_ROW, FLOW_SWITCH = 1, 2, 4, 8
 MAX_LAYERS = 64
-OPT_FUSED_FORWARD = 1
 OPT_ROW_CHUNK = 2
 OPT_OVERLAP_KGEN = 3
 

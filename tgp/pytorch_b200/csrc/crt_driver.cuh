@@ -141,15 +141,14 @@ inline int combine(const uint8_t* R, long ldr, long plane_stride, long rows, int
     return check_launch("k_crt_combine");
 }
 
-// K_xz of a row chunk in one pass: FP64 values and residue planes (i8::k_rbf_residues)
+// residue planes of K_xz (i8::k_rbf_residues)
 template <int KIND>
-inline int rbf_residues(const double* X, const double* Zs, const double* ls, const double* os, long R, int M, int D, double* Kout,
-                        int T, uint8_t* planes, long ldp, long plane_stride, cudaStream_t st, int ctas_per_sm = 3) {
-    const long n_tiles = cdiv(M, i8::RS_TC) * cdiv(R, i8::RS_TR);
-    // ctas_per_sm = 0: one CTA per tile (short CTAs: a concurrent high-priority stream gets slots every few microseconds)
-    const unsigned grid = (unsigned)((ctas_per_sm <= 0 || n_tiles < 148L * ctas_per_sm) ? n_tiles : 148L * ctas_per_sm);
+inline int rbf_residues(const double* X, const double* Zs, const double* ls, const double* os, long R, int M, int D, int T,
+                        uint8_t* planes, long ldp, long plane_stride, cudaStream_t st) {
+    // one CTA per tile (short CTAs: a concurrent high-priority stream gets slots every few microseconds)
+    const unsigned grid = (unsigned)(cdiv(M, i8::RS_TC) * cdiv(R, i8::RS_TR));
     const i8::CrtTable& tab = i8::crt_table(T);
-#define TGP_RR(MD) i8::k_rbf_residues<MD, KIND><<<grid, 256, 0, st>>>(X, Zs, ls, os, R, M, D, Kout, M, 53, tab, planes, ldp, plane_stride)
+#define TGP_RR(MD) i8::k_rbf_residues<MD, KIND><<<grid, 256, 0, st>>>(X, Zs, ls, os, R, M, D, 53, tab, planes, ldp, plane_stride)
     if (D <= 4) TGP_RR(4);
     else if (D <= 8) TGP_RR(8);
     else if (D <= 16) TGP_RR(16);
@@ -285,12 +284,12 @@ inline int qf_forward_k(const StepView& s, const StepPlanes& sp, const BatchView
                         cudaStream_t st) {
     const int M = s.M, D = s.D;
     const int Tf = fwd_T(M), bits = fwd_bits_w(M);
-    // K_xz (FP64 values + residue planes) of all rows in one launch.  It depends on Zs / ls / os only, not on the factorisation:
+    // K_xz residue planes of all rows in one launch.  It depends on Zs / ls / os only, not on the factorisation:
     // it is enqueued BEFORE the join with the factorisation, which may still be running on the library's high-priority stream
     // (TGP_OPT_OVERLAP_KGEN, common.cuh), and runs under it.  K residues: one scale for the whole matrix (0 <= k <= outputscale),
     // shared by the forward and the weight contraction.
     {
-        const int rr = rbf_residues<KIND>(X, s.Zs, s.ls, s.os, R, M, D, nullptr, T_ALL, b.Kp, b.ldk, R * b.ldk, st, 0);
+        const int rr = rbf_residues<KIND>(X, s.Zs, s.ls, s.os, R, M, D, T_ALL, b.Kp, b.ldk, R * b.ldk, st);
         if (rr != 0 && rr != -7) return rr;
         if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
         if (rr == -7) {

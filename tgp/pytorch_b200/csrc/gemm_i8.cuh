@@ -247,15 +247,14 @@ __global__ void __launch_bounds__(256) k_to_residues(const double* __restrict__ 
 }
 
 // ARD K tile generated in registers (same arithmetic as k_rbf_tile_reg: x / ls differences, FMA chain, Cov<KIND>::phi) and
-// converted on the spot: FP64 K (kept for the kernel gradients) and its residue planes in ONE pass.  The same planes serve
+// converted on the spot to residue planes; K itself is never stored (the backward recomputes its tiles).  The same planes serve
 // the forward (reduction over the inducing index: K-major) and the weight contraction (reduction over the rows: MN-major).
 // One scale for the whole matrix, for every kind: 0 <= k <= outputscale < 2^kexp, kexp derived from the outputscale in-kernel (the kernel
 // depends on nothing the factorisation produces, so it can run on a side stream under it).
 template <int MAXD, int KIND>
 __global__ void __launch_bounds__(256) k_rbf_residues(const double* __restrict__ X, const double* __restrict__ Zs,
                                                       const double* __restrict__ ls, const double* __restrict__ os, long R, int M, int D,
-                                                      double* __restrict__ Kout, long ldk_out, int bits,
-                                                      CrtTable tab, uint8_t* __restrict__ planes, long ldp, long plane_stride) {
+                                                      int bits, CrtTable tab, uint8_t* __restrict__ planes, long ldp, long plane_stride) {
     // inducing rows of the tile, dimension-major with a skew of one column per 16: the eight column groups of a warp (stride 16
     // columns) read eight different bank pairs (a [column][dimension] layout puts them all on one: an 8-way conflict per load)
     __shared__ __align__(16) double zs[MAXD][RS_TC + RS_TC / 16];
@@ -263,9 +262,9 @@ __global__ void __launch_bounds__(256) k_rbf_residues(const double* __restrict__
     const int tr = tid >> 3, tcb = (tid & 7) * 16;
     const double s = os[0];
     const int sh = bits - exp_above(s);            // the same exponent tgp_prepare stores for the reconstruction (k_exp)
-    // A bounded, persistent grid (the launcher caps it at a few CTAs per SM): when this kernel runs on the side stream under the
-    // factorisation it must leave CTA slots free, or the factorisation's small kernels would queue behind thousands of tiles.
-    // Tiles are walked column-block-major so that a CTA reloads its inducing rows rarely.
+    // The launcher starts one CTA per tile: when this kernel runs on the side stream under the factorisation, its short CTAs
+    // free slots often enough that the factorisation's small kernels do not queue behind thousands of tiles.  A CTA given
+    // several tiles walks them column-block-major, so that it reloads its inducing rows rarely.
     const long row_tiles = cdiv(R, RS_TR);
     const long n_tiles = row_tiles * cdiv(M, RS_TC);
     int c0_loaded = -1;
@@ -295,7 +294,6 @@ __global__ void __launch_bounds__(256) k_rbf_residues(const double* __restrict__
 #pragma unroll
                 for (int d = 0; d < MAXD; ++d) { const double df = xr[d] - zs[d][tcb + i + (tid & 7)]; acc = fma(df, df, acc); }
                 val = s * Cov<KIND>::phi(acc);
-                if (Kout) Kout[r * ldk_out + c] = val;
             }
             xi[i] = __double2ll_rn(mul_pow2(val, sh));
         }

@@ -3,17 +3,11 @@
 #include "step_kernels.cuh"
 #include "backward_kernels.cuh"
 #include "tc_path.cuh"
-#include "tc_fused.cuh"
 
 namespace tgp {
 namespace tc {
 
 constexpr long TC_ROW_CHUNK = 16384;
-extern int g_fused_forward;      // 1: forward = ONE kernel (K tiles generated inside the tcgen05 contraction); 0: staged planes
-
-// The fused forward generates RBF tiles only (D <= FUSED_MAX_D): other models take the staged path under either option.  The
-// backward asks the same question to know whether the forward left K planes behind.
-inline bool fused_forward(const StepView& s) { return g_fused_forward && s.D <= FUSED_MAX_D && s.kind == TGP_KERNEL_RBF; }
 
 struct StepPlanes { float *Whi, *Wlo, *Wthi, *Wtlo; double* u; long ldk, ld2m; };      // u = L^-T m (FP64, M)
 struct BatchPlanes {
@@ -72,13 +66,6 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes
                       cudaStream_t st) {
     const int M = s.M, D = s.D;
     if (join_factor(st)) return set_error(-100, "join with the factorisation failed");
-    if (fused_forward(s)) {
-        FusedFwdParams fp;
-        fp.X = X; fp.Zs = s.Zs; fp.ls = s.ls; fp.os = s.os; fp.mvec = s.mvec;
-        fp.R = (int)R; fp.M = M; fp.D = D; fp.AB = b.AB; fp.ldab = b.ld2m; fp.mu = mu; fp.v = v; fp.u = sp.u;
-        Operand W{sp.Whi, sp.Wlo, 2L * M, M, sp.ldk};
-        return fwd_fused(W, fp, st);
-    }
     // mu = K_xz (L^-T m) is accumulated in FP64 by the K generation
     cudaMemsetAsync(mu, 0, (size_t)R * sizeof(double), st);
     TGP_TRY(with_kernel(s.kind, [&](auto k) {
@@ -98,7 +85,7 @@ inline int qf_forward(const StepView& s, const StepPlanes& sp, const BatchPlanes
         }
         return 0;
     }));
-    k_row_stats_f32<<<row_grid128(R), 128, 0, st>>>(b.AB, b.ld2m, s.mvec, s.os, (int)R, M, nullptr, v);
+    k_row_stats_f32<<<row_grid128(R), 128, 0, st>>>(b.AB, b.ld2m, s.os, (int)R, M, v);
     return check_launch("k_row_stats_f32");
 }
 
@@ -118,9 +105,6 @@ inline int qf_backward_k(const StepView& s, const StepPlanes& sp, const BatchPla
         }
         const long kt_off = (r0 / b.Rc) * (long)M * b.ldt;          // K^T planes of this chunk, kept by the forward
         float *KThi = b.KThi + kt_off, *KTlo = b.KTlo + kt_off;
-        if (fused_forward(s))                                        // the fused forward never wrote K: generate it here
-            TGP_TRY(launch_rbf_planes<KIND>(X + r0 * D, s.Zs, s.ls, s.os, rc, M, D, b.Khi + r0 * b.ldk, b.Klo + r0 * b.ldk, b.ldk, KThi,
-                                      KTlo, b.ldt, st));
         {   // Kbar (rc x M) = ABbar (rc x 2M) * Wt (M x 2M)^T ; for k < M only k >= n contributes
             Params p{};
             p.Mrows = rc; p.Ncols = M; p.K = 2 * M;

@@ -3,7 +3,7 @@
 // Per-step work (K_zz, Cholesky, L^-1, C, KL, the backward chain) and the row epilogue stay in FP64; only the three
 // O(rows * M^2) contractions run on tcgen05 as 3xTF32 products with FP32 accumulation in TMEM (gemm_tc.cuh).
 // Operands are staged as (value, value - tf32_trunc(value)) plane pairs, K-major:
-//   K      (rows x M)   generated on the fly per row chunk (never the full K_xz)         forward  A-operand
+//   K      (rows x M)   generated per row chunk, kept for all rows for the backward        forward  A-operand
 //   W      (2M x M)   = [L^-1 ; C]                                                        forward  B-operand
 //   ABbar  (rows x 2M) = [g_mu m - 2 g_v A | 2 g_v B]                                     backward-data A-operand
 //   Wt     (M x 2M)   = [L^-T | C^T]                                                      backward-data B-operand
@@ -30,11 +30,11 @@ __device__ __forceinline__ void put_planes(float* __restrict__ hi, float* __rest
 
 inline long pad4(long x) { return (x + 3) / 4 * 4; }
 
-// K tile (distance in FP64, as k_rbf_tile; exponential in FP32: Cov<KIND>::kf, common.cuh), written as FP32 planes: row-major (rows x ldk) and/or
+// K tile (distance in FP64, as k_rbf_tile; exponential in FP32: Cov<KIND>::kf, common.cuh), written as FP32 planes: row-major (rows x ldk) and
 // transposed (M x ldt).  32 x 64 tile per CTA staged through shared memory so that both writes are coalesced.
 constexpr int RP_TR = 32, RP_TC = 64, RP_THREADS = 256;
 template <int KIND>
-// If u != NULL (u = L^-T m, FP64, one per step) the marginal mean is accumulated here as well: mu[n] += sum_j K[n,j] u[j] in FP64 —
+// The marginal mean is accumulated here as well (u = L^-T m, FP64, one per step): mu[n] += sum_j K[n,j] u[j] in FP64 —
 // the reference's own evaluation order mu = K_xz (L^-T m) (sparse_MF_SP.py:354-355).  Taking mu from the FP32 rows a = L^-1 k
 // instead lets the conditioning of L^-1 amplify the FP32 rounding of a (measured at cfg4: max |dmu| 3.3e-4 against 2.3e-5, ELBO
 // 3.6e-5 against 2.4e-6 from FP64; scripts/tf32_error_terms.py).
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(RP_THREADS) k_rbf_planes(const double* __restr
     __syncthreads();
     const double s = os[0];
     const int c = tid % RP_TC, j = c0 + c;
-    const double uj = (u && j < M) ? u[j] : 0.0;
+    const double uj = j < M ? u[j] : 0.0;
     for (int r = tid / RP_TC; r < RP_TR; r += RP_THREADS / RP_TC) {
         const int n = r0 + r;
         float val = 0.f;
@@ -71,21 +71,18 @@ __global__ void __launch_bounds__(RP_THREADS) k_rbf_planes(const double* __restr
             val = Cov<KIND>::kf(acc, (float)s);
         }
         tile[r * (RP_TC + 1) + c] = val;
-        if (Khi && n < R && j < M) { put_planes(Khi, Klo, (long)n * ldk + j, val); }
-        if (u) {                               // the 32 lanes of a warp hold 32 columns of the SAME row (RP_TC = 64)
-            const double part = warp_sum((double)val * uj);
-            if ((tid & 31) == 0 && n < R) atomicAdd(mu + n, part);
-        }
+        if (n < R && j < M) put_planes(Khi, Klo, (long)n * ldk + j, val);
+        // the 32 lanes of a warp hold 32 columns of the SAME row (RP_TC = 64)
+        const double part = warp_sum((double)val * uj);
+        if ((tid & 31) == 0 && n < R) atomicAdd(mu + n, part);
     }
-    if (KThi) {
-        __syncthreads();
-        const int rr = tid % RP_TR;
-        for (int cc = tid / RP_TR; cc < RP_TC; cc += RP_THREADS / RP_TR) {
-            const int n = r0 + rr, jj = c0 + cc;
-            if (n < R && jj < M) {
-                const float val = tile[rr * (RP_TC + 1) + cc];
-                put_planes(KThi, KTlo, (long)jj * ldt + n, val);
-            }
+    __syncthreads();
+    const int rr = tid % RP_TR;
+    for (int cc = tid / RP_TR; cc < RP_TC; cc += RP_THREADS / RP_TR) {
+        const int n = r0 + rr, jj = c0 + cc;
+        if (n < R && jj < M) {
+            const float val = tile[rr * (RP_TC + 1) + cc];
+            put_planes(KThi, KTlo, (long)jj * ldt + n, val);
         }
     }
 }
@@ -93,7 +90,7 @@ __global__ void __launch_bounds__(RP_THREADS) k_rbf_planes(const double* __restr
 template <int KIND>
 inline int launch_rbf_planes(const double* X, const double* Zs, const double* ls, const double* os, int R, int M, int D,
                              float* Khi, float* Klo, long ldk, float* KThi, float* KTlo, long ldt, cudaStream_t st,
-                             const double* u = nullptr, double* mu = nullptr) {
+                             const double* u, double* mu) {
     const size_t smem = (size_t)(RP_TR + RP_TC) * (D + 1) * sizeof(double) + (size_t)RP_TR * (RP_TC + 1) * sizeof(float);
     if (smem > 48 * 1024) return set_error(-2, "input dimension too large for the plane-generating RBF kernel");
     dim3 grid((unsigned)cdiv(M, RP_TC), (unsigned)cdiv(R, RP_TR));
@@ -128,23 +125,21 @@ __global__ void k_make_w_planes(const double* __restrict__ Linv, const double* _
     }
 }
 
-// mu, v from the FP32 [A | B] rows (sums accumulated in FP64)
-__global__ void __launch_bounds__(128) k_row_stats_f32(const float* __restrict__ AB, long ldab, const double* __restrict__ m,
-                                                       const double* __restrict__ os, int R, int M,
-                                                       double* __restrict__ mu, double* __restrict__ v) {
+// v from the FP32 [A | B] rows (sums accumulated in FP64); mu is accumulated by k_rbf_planes
+__global__ void __launch_bounds__(128) k_row_stats_f32(const float* __restrict__ AB, long ldab, const double* __restrict__ os, int R,
+                                                       int M, double* __restrict__ v) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     for (long n = (long)blockIdx.x * wpb + wid; n < R; n += (long)gridDim.x * wpb) {
         const float* a = AB + n * ldab;
         const float* b = a + M;
-        double sm = 0.0, sa = 0.0, sb = 0.0;
+        double sa = 0.0, sb = 0.0;
         for (int j = lane; j < M; j += 32) {
             const double aj = a[j], bj = b[j];
-            sm = fma(aj, __ldg(m + j), sm);
             sa = fma(aj, aj, sa);
             sb = fma(bj, bj, sb);
         }
-        sm = warp_sum(sm); sa = warp_sum(sa); sb = warp_sum(sb);
-        if (lane == 0) { if (mu) mu[n] = sm; v[n] = os[0] - sa + sb; }        // mu == NULL: already accumulated by k_rbf_planes
+        sa = warp_sum(sa); sb = warp_sum(sb);
+        if (lane == 0) v[n] = os[0] - sa + sb;
     }
 }
 

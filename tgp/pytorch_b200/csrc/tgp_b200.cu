@@ -19,7 +19,6 @@ namespace tgp {
 char g_last_error[512] = "";
 long g_launch_count = 0;
 GemmTimer g_gemm_timer;
-namespace tc { int g_fused_forward = 0; }
 int g_overlap_kgen = 1;
 
 inline long even(long x) { return (x + 1) / 2 * 2; }
@@ -141,7 +140,7 @@ using namespace tgp;
 extern "C" {
 
 const char* tgp_last_error(void) { return g_last_error; }
-int tgp_version(void) { return 101; }
+int tgp_version(void) { return 102; }
 
 size_t tgp_step_workspace_bytes(const TgpModel* md) {
     if (validate(md)) return 0;
@@ -781,7 +780,6 @@ int tgp_kmeans_iteration(const void* X, long N, int D, void* Cc, int M, int* ass
 long tgp_launch_count(void) { return g_launch_count; }
 
 int tgp_set_option(int key, int value) {
-    if (key == TGP_OPT_FUSED_FORWARD) { tc::g_fused_forward = value != 0; return 0; }
     if (key == TGP_OPT_OVERLAP_KGEN) { g_overlap_kgen = value != 0; return 0; }
     if (key == TGP_OPT_ROW_CHUNK) {
         if (value < 128) return set_error(-1, "row chunk must be >= 128");
