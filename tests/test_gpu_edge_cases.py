@@ -6,6 +6,7 @@ import torch
 
 from oracle import tgp_oracle as O
 from tests.golden_util import rel_err
+from tests.test_gpu_matern import _to
 
 pytestmark = pytest.mark.gpu
 EDGE_TOL = 1e-10      # north_star's FP64 tolerance, values and gradients alike (measured: see profiles/r02_parity_residuals.json)
@@ -15,8 +16,20 @@ def _tol(p):
     """1e-10, widened only where the problem itself cannot carry it: a = L^-1 k and the gradients through L^-T carry
     ~eps * cond(L) = eps * sqrt(cond(K_zz)) of forward error in ANY FP64 evaluation; one of the random tiny problems
     below (D = 1, five inducing points on a line) has cond(K_zz) = 2e12."""
-    Kzz = O.rbf_ard(p['Z'], p['Z'], p['raw_lengthscale'], p['raw_outputscale'])
-    return max(EDGE_TOL, 100.0 * 2.2e-16 * float(torch.linalg.cond(Kzz)) ** 0.5)
+    return max(EDGE_TOL, 100.0 * 2.2e-16 * _cond(p) ** 0.5)
+
+
+def _cond(p):
+    with torch.no_grad():
+        return float(torch.linalg.cond(O.rbf_ard(p['Z'], p['Z'], p['raw_lengthscale'], p['raw_outputscale'])))
+
+
+def _tol32(p, e32):
+    """'tf32x3': the FP32 bound of tests/test_gpu_matern.py, 1e-5 + 4 x e32 (e32: the oracle's own float32 evaluation against
+    its float64 one), widened as _tol where the problem cannot carry it.  The FP32 planes of L^-1 leave ~eps32 * sqrt(cond(K_zz))
+    of error in a = L^-1 k; at cond(K_zz) = 2e12 (the D = 1 problem) that is 0.17, and K_zz is singular in float32, so the
+    oracle's float32 run adds jitter and no longer evaluates the same problem (measured: 5.5e-2 on dm against e32 = 6e-5)."""
+    return max(1e-5 + 4.0 * e32, 1.19e-7 * _cond(p) ** 0.5)
 DEV = 'cuda:0'
 
 
@@ -40,7 +53,8 @@ def _problem(R, M, D, seed, flow=True):
     return X, y, p
 
 
-def _cuda_vs_oracle(X, y, p, N, lik='gauss_nonlinear', nq=30, compute='f64'):
+def _cuda(X, y, p, N, lik, nq, compute):
+    """(ELBO, rows and every gradient of the CUDA path, flow-parameter names)."""
     from tests.gpu_util import engine_inputs, make_engine
     from tgp.pytorch_b200 import functional as Fn
     eng, theta, rowp, names = make_engine(p, lik, nq, DEV, compute=compute)
@@ -51,28 +65,48 @@ def _cuda_vs_oracle(X, y, p, N, lik='gauss_nonlinear', nq=30, compute='f64'):
     scale = N / X.shape[0]
     ELL, KLD, rows, mu, v = Fn.elbo_terms(eng, X.to(DEV).contiguous(), y.to(DEV).contiguous(), scale, *leaves[:6], theta, None)
     (ELL - KLD).backward()
-    E, _, _, rows_o, gr = O.elbo_and_grads(X, y, p, N, lik, nq)
-    out = {'ELBO': rel_err((ELL - KLD).detach().cpu(), E), 'rows': rel_err(rows.cpu(), rows_o),
-           'Z': rel_err(ei['Z'].grad.cpu(), gr['Z']), 'ls': rel_err(ei['raw_ls'].grad.cpu(), gr['raw_lengthscale']),
-           'os': rel_err(ei['raw_os'].grad.cpu().view(()), gr['raw_outputscale']), 'm': rel_err(ei['m'].grad.cpu(), gr['m']),
-           'L': rel_err(ei['L_raw'].grad.cpu(), gr['L_raw']), 'noise': rel_err(ei['log_var_noise'].grad.cpu().view(()), gr['log_var_noise'])}
+    out = {'ELBO': (ELL - KLD).detach().cpu(), 'rows': rows.cpu(), 'Z': ei['Z'].grad.cpu(), 'ls': ei['raw_ls'].grad.cpu(),
+           'os': ei['raw_os'].grad.cpu().view(()), 'm': ei['m'].grad.cpu(), 'L': ei['L_raw'].grad.cpu(),
+           'noise': ei['log_var_noise'].grad.cpu().view(())}
     if theta.numel():
-        ref_theta = torch.stack([gr[n].reshape(()) for n in names])
-        out['theta'] = rel_err(theta.grad.cpu(), ref_theta)
+        out['theta'] = theta.grad.cpu()
+    return out, names
+
+
+def _oracle(X, y, p, N, lik, nq, names):
+    """The oracle's values under the keys of _cuda (in the dtype of X and p)."""
+    E, _, _, rows_o, gr = O.elbo_and_grads(X, y, p, N, lik, nq)
+    out = {'ELBO': E, 'rows': rows_o, 'Z': gr['Z'], 'ls': gr['raw_lengthscale'], 'os': gr['raw_outputscale'], 'm': gr['m'],
+           'L': gr['L_raw'], 'noise': gr['log_var_noise']}
+    if names:
+        out['theta'] = torch.stack([gr[n].reshape(()) for n in names])
     return out
+
+
+def _cuda_vs_oracle(X, y, p, N, lik='gauss_nonlinear', nq=30, compute='f64'):
+    got, names = _cuda(X, y, p, N, lik, nq, compute)
+    ref = _oracle(X, y, p, N, lik, nq, names)
+    return {k: rel_err(got[k], ref[k]) for k in got}
 
 
 @pytest.mark.parametrize('R,M,D', [(1, 5, 1), (3, 1, 2), (130, 63, 3), (257, 65, 4), (64, 128, 8), (300, 129, 5),
                                      (1000, 200, 13), (77, 257, 16), (50, 40, 33), (40, 30, 64)])
-@pytest.mark.parametrize('compute', ['f64', 'i8crt'])
+@pytest.mark.parametrize('compute', ['f64', 'i8crt', 'tf32x3'])
 def test_shapes_around_tile_and_block_boundaries(R, M, D, compute):
-    """Both FP64-accurate modes: ragged row counts, M around the 64 / 128 / 256 tile and block sizes, D beyond the register-resident
-    K generators (D > 32: 'i8crt' falls back to staged K generation and keeps an FP64 K_xz for the kernel gradients)."""
+    """Every mode: ragged row counts, M around the 64 / 128 / 256 tile and block sizes, D beyond the register-resident K
+    generators (D > 32: 'i8crt' falls back to staged K generation and keeps an FP64 K_xz for the kernel gradients; D >= 53:
+    the K generation of 'tf32x3' needs more than 48 KiB of shared memory).  'tf32x3' is held to the FP32 bound _tol32."""
     X, y, p = _problem(R, M, D, seed=R * 7 + M * 3 + D)
-    err = _cuda_vs_oracle(X, y, p, N=10.0 * R, compute=compute)
+    got, names = _cuda(X, y, p, 10.0 * R, 'gauss_nonlinear', 30, compute)
+    ref = _oracle(X, y, p, 10.0 * R, 'gauss_nonlinear', 30, names)
+    err = {k: rel_err(got[k], ref[k]) for k in got}
     from tests.conftest import record_residuals
     record_residuals('edge_shapes[%s]' % compute, err)
-    bad = {k: e for k, e in err.items() if not e < _tol(p)}
+    if compute == 'tf32x3':
+        ref32 = _oracle(X.float(), y.float(), _to(p, torch.float32), 10.0 * R, 'gauss_nonlinear', 30, names)
+        bad = {k: (e, rel_err(ref32[k], ref[k])) for k, e in err.items() if not e < _tol32(p, rel_err(ref32[k], ref[k]))}
+    else:
+        bad = {k: e for k, e in err.items() if not e < _tol(p)}
     assert not bad, (bad, err)
 
 

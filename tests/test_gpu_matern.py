@@ -50,18 +50,21 @@ def _engine(p, lik, nq, compute):
     return eng, theta, names
 
 
-def _cuda(X, y, p, N, lik, nq, compute):
+def _cuda(X, y, p, N, lik, nq, compute, want_dx=False):
+    """ELBO terms, rows, mu, v and every parameter gradient; with want_dx also out['X'] = dELBO/dX."""
     from tgp.pytorch_b200 import functional as Fn
     eng, theta, names = _engine(p, lik, nq, compute)
     ei = engine_inputs(p, DEV)
     leaves = [ei['Z'], ei['raw_ls'], ei['raw_os'], ei['m'], ei['L_raw'], ei['log_var_noise'], theta]
     for t in leaves:
         t.requires_grad_(True)
-    ELL, KLD, rows, mu, v = Fn.elbo_terms(eng, X.to(DEV).contiguous(), y.to(DEV).contiguous(), N / X.shape[0], *leaves[:6],
-                                          theta, None)
+    Xd = X.to(DEV).contiguous().requires_grad_(want_dx)
+    ELL, KLD, rows, mu, v = Fn.elbo_terms(eng, Xd, y.to(DEV).contiguous(), N / X.shape[0], *leaves[:6], theta, None)
     (ELL - KLD).backward()
     out = dict(ELBO=(ELL - KLD).detach().cpu(), ELL=ELL.detach().cpu(), KLD=KLD.detach().cpu(), rows=rows.cpu(), mu=mu.cpu(),
                v=v.cpu())
+    if want_dx:
+        out['X'] = Xd.grad.detach().cpu()
     for k, t in zip(GRAD_KEYS, leaves):
         out[k] = (t.grad if t.grad is not None else torch.zeros_like(t)).detach().cpu().reshape(-1)
     for i, n in enumerate(names):

@@ -92,7 +92,12 @@ inline int launch_rbf_planes(const double* X, const double* Zs, const double* ls
                              float* Khi, float* Klo, long ldk, float* KThi, float* KTlo, long ldt, cudaStream_t st,
                              const double* u, double* mu) {
     const size_t smem = (size_t)(RP_TR + RP_TC) * (D + 1) * sizeof(double) + (size_t)RP_TR * (RP_TC + 1) * sizeof(float);
-    if (smem > 48 * 1024) return set_error(-2, "input dimension too large for the plane-generating RBF kernel");
+    if (smem > 200 * 1024) return set_error(-2, "input dimension too large for the plane-generating RBF kernel");
+    // above 48 KiB (D >= 53) the kernel needs the opt-in to large dynamic shared memory, set once per device to the bound above
+    if (smem > 48 * 1024) {
+        static PerDeviceOnce once;
+        if (once.first()) cudaFuncSetAttribute(k_rbf_planes<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    }
     dim3 grid((unsigned)cdiv(M, RP_TC), (unsigned)cdiv(R, RP_TR));
     k_rbf_planes<KIND><<<grid, RP_THREADS, smem, st>>>(X, Zs, ls, os, R, M, D, Khi, Klo, ldk, KThi, KTlo, ldt, u, mu);
     return check_launch("k_rbf_planes");
