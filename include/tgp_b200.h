@@ -197,7 +197,8 @@ int tgp_coverage_rows(const TgpModel* model, const TgpParams* params, const void
 /* Monte-Carlo expected log-likelihood of the multiclass softmax likelihood — replaces
  * MulticlassCategorical.expected_log_prob (likelihoods/MulticlassCategorical.py:51-105) and, with probs != NULL,
  * marginal_moments (:109-151).  One GP per class: mu, v are (C, R); eps (S, C, R) is the N(0,1) noise of td.Normal.rsample,
- * drawn by the caller (the reference's generator stream); the C flows share model->layers (global parameters only) and own
+ * drawn by the caller (the reference's generator stream); the C flows share model->layers (global parameters only; per-row
+ * flows go through tgp_mc_softmax_rows_rowp) and own
  * one row each of theta (C, n_theta); Y holds the labels 0..C-1 as doubles.
  *   ell_rows[n] = 1/S sum_s log softmax(G(mu + sqrt(v) eps_s))[y_n]
  * want_grad: g_mu, g_v (C, R) = d ell_rows[n] / d mu[c,n], d v[c,n] (unscaled); dtheta (C, n_theta) += d sum_n ell_rows[n] / d theta
@@ -205,6 +206,16 @@ int tgp_coverage_rows(const TgpModel* model, const TgpParams* params, const void
 int tgp_mc_softmax_rows(const TgpModel* model, int C, int S, long R, const void* mu, const void* v, const void* Y, const void* eps,
                         const void* theta, int want_grad, void* ell_rows, void* g_mu, void* g_v, void* dtheta, void* probs,
                         void* stream);
+/* tgp_mc_softmax_rows for input-dependent flows (ID_TGP): the layers flagged TGP_FLOW_PER_ROW take their raw parameters from
+ * rowparams (C, R, n_rowparams), row-major: rowparams[(c R + n) n_rowparams + k] is parameter k of class c's flow at row n, the
+ * class-stacked MLP outputs evaluated once on X for the call and shared by all S samples.  The C flows share model->layers (one
+ * architecture; TgpFlowLayer.p0 indexes theta for global layers and the row vector for per-row ones).  want_grad: drowparams
+ * (C, R, n_rowparams) = d ell_rows[n] / d rowparams[c,n,k], WRITTEN (not accumulated) and unscaled like g_mu / g_v; dtheta as in
+ * tgp_mc_softmax_rows.  n_rowparams <= 16 and C * n_rowparams <= 256.  With model->n_rowparams = 0 (rowparams, drowparams
+ * ignored) this is tgp_mc_softmax_rows, bit for bit. */
+int tgp_mc_softmax_rows_rowp(const TgpModel* model, int C, int S, long R, const void* mu, const void* v, const void* Y,
+                             const void* eps, const void* theta, int want_grad, void* ell_rows, void* g_mu, void* g_v, void* dtheta,
+                             void* probs, const void* rowparams, void* drowparams, void* stream);
 
 /* The exchange format of the one collective per step (SURVEY.md 8e).  The reduce buffer holds two (padded) M x M blocks
  * of which only the lower triangles are populated in TGP_F64 mode (Gbar and dL_S; in TGP_F32 mode the second block, Cbar,

@@ -91,6 +91,7 @@ SIGNATURES = {
     'tgp_coverage_rows': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _I, _I, C.c_ulonglong, _P, _D, _D, _P, _P,
                               _P, _P, _P, _P]),
     'tgp_mc_softmax_rows': (_I, [C.POINTER(TgpModel), _I, _I, _L, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P]),
+    'tgp_mc_softmax_rows_rowp': (_I, [C.POINTER(TgpModel), _I, _I, _L, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     'tgp_reduce_pack': (_I, [C.POINTER(TgpModel), _P, _P, _P]),
     'tgp_reduce_unpack': (_I, [C.POINTER(TgpModel), _P, _P, _P]),
     'tgp_workspace_bytes': (C.c_size_t, [C.POINTER(TgpModel), _L]),

@@ -497,6 +497,38 @@ int tgp_coverage_rows(const TgpModel* md, const TgpParams* p, const void* mu, co
     return 0;
 }
 
+static int mc_softmax_launch(const TgpModel* md, int C, int S, long R, const void* mu, const void* v, const void* Y, const void* eps,
+                             const void* theta, const void* rowparams, int want_grad, void* ell_rows, void* g_mu, void* g_v,
+                             void* dtheta, void* drowparams, void* probs, void* stream) {
+    McSoftmaxArgs a;
+    a.R = (int)R; a.C = C; a.S = S; a.n_theta = md->n_theta; a.want_grad = want_grad;
+    a.mu = (const double*)mu; a.v = (const double*)v; a.y = (const double*)Y; a.eps = (const double*)eps;
+    a.theta = (const double*)theta;
+    a.ell_rows = (double*)ell_rows; a.g_mu = (double*)g_mu; a.g_v = (double*)g_v; a.dtheta = (double*)dtheta; a.probs = (double*)probs;
+    fill_flow(a.flow, md);
+    a.n_rowp = md->n_rowparams; a.rowp = (const double*)rowparams; a.drowp = (double*)drowparams;
+    const unsigned grid = (unsigned)((R + MC_THREADS - 1) / MC_THREADS);
+    if (md->n_rowparams == 0) {
+        const size_t smem = (size_t)C * 3 * (md->n_theta > 0 ? md->n_theta : 1) * sizeof(double);
+        k_row_mc_softmax<false><<<grid, MC_THREADS, smem, (cudaStream_t)stream>>>(a);
+    } else {
+        // flow_prepare indexes its table by parameter slot over all layers, per-row ones included
+        const size_t smem = (size_t)C * 3 * (md->n_theta + md->n_rowparams) * sizeof(double);
+        k_row_mc_softmax<true><<<grid, MC_THREADS, smem, (cudaStream_t)stream>>>(a);
+    }
+    return check_launch("k_row_mc_softmax");
+}
+
+// the checks both Monte-Carlo softmax entry points share, after their class-count and sample-count checks
+static int mc_softmax_check(const TgpModel* md, int C, const void* mu, const void* v, const void* Y, const void* eps,
+                            const void* theta, int want_grad, void* ell_rows, void* g_mu, void* g_v, void* dtheta) {
+    if ((long)C * md->n_theta > MC_MAX_ACC) return set_error(-1, "C * n_theta exceeds the per-thread gradient accumulator (256)");
+    if (!mu || !v || !Y || !eps || !ell_rows || (md->n_theta > 0 && !theta))
+        return set_error(-1, "NULL argument to tgp_mc_softmax_rows");
+    if (want_grad && (!g_mu || !g_v || (md->n_theta > 0 && !dtheta))) return set_error(-1, "gradient outputs required");
+    return 0;
+}
+
 int tgp_mc_softmax_rows(const TgpModel* md, int C, int S, long R, const void* mu, const void* v, const void* Y, const void* eps,
                         const void* theta, int want_grad, void* ell_rows, void* g_mu, void* g_v, void* dtheta, void* probs,
                         void* stream) {
@@ -505,21 +537,28 @@ int tgp_mc_softmax_rows(const TgpModel* md, int C, int S, long R, const void* mu
     if (C < 2 || C > MC_MAX_CLASSES) return set_error(-1, "number of classes out of range (2..32)");
     if (S < 1) return set_error(-1, "S must be positive");
     if (md->n_rowparams > 0) return set_error(-1, "the Monte-Carlo softmax likelihood takes flows with global parameters");
-    if ((long)C * md->n_theta > MC_MAX_ACC) return set_error(-1, "C * n_theta exceeds the per-thread gradient accumulator (256)");
-    if (!mu || !v || !Y || !eps || !ell_rows || (md->n_theta > 0 && !theta))
-        return set_error(-1, "NULL argument to tgp_mc_softmax_rows");
-    if (want_grad && (!g_mu || !g_v || (md->n_theta > 0 && !dtheta))) return set_error(-1, "gradient outputs required");
+    TGP_TRY(mc_softmax_check(md, C, mu, v, Y, eps, theta, want_grad, ell_rows, g_mu, g_v, dtheta));
     for (int i = 0; i < md->n_layers; ++i)
         if (md->layers[i].flags & TGP_FLOW_PER_ROW) return set_error(-1, "per-row flow parameters are not supported here");
-    McSoftmaxArgs a;
-    a.R = (int)R; a.C = C; a.S = S; a.n_theta = md->n_theta; a.want_grad = want_grad;
-    a.mu = (const double*)mu; a.v = (const double*)v; a.y = (const double*)Y; a.eps = (const double*)eps;
-    a.theta = (const double*)theta;
-    a.ell_rows = (double*)ell_rows; a.g_mu = (double*)g_mu; a.g_v = (double*)g_v; a.dtheta = (double*)dtheta; a.probs = (double*)probs;
-    fill_flow(a.flow, md);
-    const size_t smem = (size_t)C * 3 * (md->n_theta > 0 ? md->n_theta : 1) * sizeof(double);
-    k_row_mc_softmax<<<(unsigned)((R + MC_THREADS - 1) / MC_THREADS), MC_THREADS, smem, (cudaStream_t)stream>>>(a);
-    return check_launch("k_row_mc_softmax");
+    return mc_softmax_launch(md, C, S, R, mu, v, Y, eps, theta, nullptr, want_grad, ell_rows, g_mu, g_v, dtheta, nullptr, probs, stream);
+}
+
+int tgp_mc_softmax_rows_rowp(const TgpModel* md, int C, int S, long R, const void* mu, const void* v, const void* Y, const void* eps,
+                             const void* theta, int want_grad, void* ell_rows, void* g_mu, void* g_v, void* dtheta, void* probs,
+                             const void* rowparams, void* drowparams, void* stream) {
+    TGP_TRY(validate(md));
+    if (R <= 0) return 0;
+    if (C < 2 || C > MC_MAX_CLASSES) return set_error(-1, "number of classes out of range (2..32)");
+    if (S < 1) return set_error(-1, "S must be positive");
+    TGP_TRY(mc_softmax_check(md, C, mu, v, Y, eps, theta, want_grad, ell_rows, g_mu, g_v, dtheta));
+    const int nr = md->n_rowparams;
+    if (nr > MAX_ROWP) return set_error(-1, "too many per-row flow parameters (n_rowparams <= 16)");
+    if ((long)C * nr > MC_MAX_ACC)
+        return set_error(-1, "C * n_rowparams exceeds the per-thread per-row gradient accumulator (256)");
+    if (nr > 0 && !rowparams) return set_error(-1, "rowparams required for input-dependent flows");
+    if (want_grad && nr > 0 && !drowparams) return set_error(-1, "drowparams required for the gradient of input-dependent flows");
+    return mc_softmax_launch(md, C, S, R, mu, v, Y, eps, theta, rowparams, want_grad, ell_rows, g_mu, g_v, dtheta, drowparams, probs,
+                             stream);
 }
 
 int tgp_reduce_pack(const TgpModel* md, const double* reduce_buf, double* packed, void* stream) {

@@ -4,7 +4,8 @@
 Same constructor and method signatures as the reference.  The S x C x MB noise of `td.Normal(mean, std).rsample([S])` is drawn
 here with the framework's generator exactly as rsample draws it (`torch.empty(shape).normal_()`), so a seeded run consumes the
 same stream as the reference on the same device; setting `mc_noise` to a (S, C, MB) tensor replaces the draw (parity tests).
-Sampling, flows, log-softmax, the mean over samples and all gradients run in ONE kernel (tgp_mc_softmax_rows)."""
+Sampling, flows, log-softmax, the mean over samples and all gradients run in ONE kernel (tgp_mc_softmax_rows, or
+tgp_mc_softmax_rows_rowp for input-dependent flows, whose MLPs are evaluated on X[c] once per call)."""
 import torch
 import torch.nn as nn
 import torch.distributions as td

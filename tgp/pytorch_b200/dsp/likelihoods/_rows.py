@@ -115,21 +115,21 @@ def _mc_model(layout):
 
 
 def mc_flow_pack(flows, X):
-    """C flow modules of one architecture -> (FlowLayout, theta (C, n_theta) or None)."""
+    """C flow modules of one architecture -> (FlowLayout, theta (C, n_theta) or None, rowp (C, R, n_rowparams) or None).
+    Input-dependent layers evaluate each class's MLPs on X[c]; their outputs are stacked class-major."""
     packs = [flow_pack(fl, X[c] if X is not None else None) for c, fl in enumerate(flows)]
     first = packs[0][0]
-    for lay, _th, rowp in packs:
-        if rowp is not None:
-            raise NotImplementedError('input-dependent flows under the Monte-Carlo softmax likelihood')
-        if lay.layers != first.layers:
+    for lay, _th, _rp in packs:
+        if lay.layers != first.layers:          # kinds, flags, per_row and p0 of every layer
             raise NotImplementedError('the Monte-Carlo softmax kernel takes one flow architecture for all classes')
     theta = torch.stack([p[1] for p in packs]) if first.n_theta > 0 else None
-    return first, theta
+    rowp = torch.stack([p[2] for p in packs]) if first.n_rowparams > 0 else None
+    return first, theta, rowp
 
 
 class _McSoftmax(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, layout, y, eps, want_probs, mu, v, theta):
+    def forward(ctx, layout, y, eps, want_probs, mu, v, theta, rowp):
         import ctypes as C
         from ... import _lib
         lib = _lib.load()
@@ -142,36 +142,44 @@ class _McSoftmax(torch.autograd.Function):
         d = torch.float64
         mu_d, v_d = mu.detach().to(d).contiguous(), v.detach().to(d).contiguous()
         th = None if theta is None else theta.detach().to(d).contiguous()
+        rp = None if rowp is None else rowp.detach().to(d).contiguous()
+        assert rp is None or tuple(rp.shape) == (Cn, R, layout.n_rowparams), 'rowp must be (C, R, n_rowparams)'
         grad = any(ctx.needs_input_grad)
         rows = torch.empty(R, dtype=d, device=dev)
         g_mu = torch.empty(Cn, R, dtype=d, device=dev) if grad else None
         g_v = torch.empty(Cn, R, dtype=d, device=dev) if grad else None
         dth = torch.zeros_like(th) if (grad and th is not None) else None
+        drp = torch.empty_like(rp) if (grad and rp is not None) else None
         probs = torch.empty(R, Cn, dtype=d, device=dev) if want_probs else None
         ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        args = (_mc_model(layout), Cn, S, R, ptr(mu_d), ptr(v_d), ptr(y.to(d).contiguous()), ptr(eps.to(d).contiguous()), ptr(th),
+                1 if grad else 0, ptr(rows), ptr(g_mu), ptr(g_v), ptr(dth), ptr(probs))
         with torch.cuda.device(dev):
             st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(lib.tgp_mc_softmax_rows(_mc_model(layout), Cn, S, R, ptr(mu_d), ptr(v_d), ptr(y.to(d).contiguous()),
-                                               ptr(eps.to(d).contiguous()), ptr(th), 1 if grad else 0, ptr(rows), ptr(g_mu), ptr(g_v),
-                                               ptr(dth), ptr(probs), st), 'tgp_mc_softmax_rows')
+            if rp is None:
+                _lib.check(lib.tgp_mc_softmax_rows(*args, st), 'tgp_mc_softmax_rows')
+            else:
+                _lib.check(lib.tgp_mc_softmax_rows_rowp(*args, ptr(rp), ptr(drp), st), 'tgp_mc_softmax_rows_rowp')
         if grad:
-            ctx.save_for_backward(g_mu, g_v, dth if dth is not None else rows.new_zeros(1))
-        ctx.has_theta, ctx.io_dtype = th is not None, mu.dtype
+            ctx.save_for_backward(g_mu, g_v, dth if dth is not None else rows.new_zeros(1),
+                                  drp if drp is not None else rows.new_zeros(1))
+        ctx.has_theta, ctx.has_rowp, ctx.io_dtype = th is not None, rp is not None, mu.dtype
         out_p = probs if want_probs else rows.new_zeros(0)
         ctx.mark_non_differentiable(rows, out_p)
         return rows.sum(), rows, out_p
 
     @staticmethod
     def backward(ctx, g_sum, _g_rows, _g_probs):
-        g_mu, g_v, dth = ctx.saved_tensors
+        g_mu, g_v, dth, drp = ctx.saved_tensors
         return (None, None, None, None, (g_mu * g_sum).to(ctx.io_dtype), (g_v * g_sum).to(ctx.io_dtype),
-                dth * g_sum if ctx.has_theta else None)
+                dth * g_sum if ctx.has_theta else None, drp * g_sum if ctx.has_rowp else None)
 
 
 def mc_softmax(flows, X, y, eps, mu, v, want_probs=False):
     """(sum over rows of the MC expected log-likelihood, per-row terms, class probabilities or empty)."""
     from ... import functional as Fn
-    layout, theta = mc_flow_pack(flows, X)
+    layout, theta, rowp = mc_flow_pack(flows, X)
     if theta is not None and theta.requires_grad and Fn._world() is not None:
         theta = Fn._SumGradAcrossRanks.apply(theta)          # the flow scalars see rank-local rows only
-    return _McSoftmax.apply(layout, y, eps, bool(want_probs), mu, v, theta)
+    # rowp is row-local; the MLP weights behind it are summed across ranks by the fused MLP backward / synced_module_call
+    return _McSoftmax.apply(layout, y, eps, bool(want_probs), mu, v, theta, rowp)

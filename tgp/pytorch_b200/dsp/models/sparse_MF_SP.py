@@ -418,7 +418,16 @@ class sparse_MF_SP(nn.Module):
                     P = lik.marginal_moments(mean_q_f.squeeze(2), cov_q_f.squeeze(2), self.G_matrix, X)
                 m1, m2 = P, None
             elif isinstance(lik, MulticlassCategorical):
-                m1, m2 = lik.marginal_moments(mean_q_f.squeeze(2), cov_q_f.squeeze(2), self.G_matrix, X), None
+                mq, vq = mean_q_f.squeeze(2), cov_q_f.squeeze(2)
+                if n_mc > 1:
+                    # the n_mc dropout replicas as repeated rows of one kernel call (each replica draws its own masks and
+                    # noise), then the class probabilities averaged over the replicas
+                    MB = mq.shape[1]
+                    P = lik.marginal_moments(mq.repeat(1, n_mc), vq.repeat(1, n_mc), self.G_matrix, X.repeat(1, n_mc, 1))
+                    m1 = P.view(n_mc, MB, -1).mean(0)
+                else:
+                    m1 = lik.marginal_moments(mq, vq, self.G_matrix, X)
+                m2 = None
             else:
                 raise ValueError('Unsupported likelihood [{}]'.format(type(lik)))
         self.train()
