@@ -24,7 +24,14 @@ extern "C" {
 enum { TGP_F64 = 0, TGP_F32 = 1, TGP_F64_I8 = 2 };
 enum { TGP_LIK_GAUSS_LINEAR = 0,     /* likelihoods/GaussianLinearMean.py:60-87   (SVGP, closed form)      */
        TGP_LIK_GAUSS_NONLINEAR = 1,  /* likelihoods/GaussianNonLinearMean.py:113-150 (Gauss-Hermite)       */
-       TGP_LIK_BERNOULLI = 2 };      /* likelihoods/Bernoulli.py:50-95                                      */
+       TGP_LIK_BERNOULLI = 2,        /* likelihoods/Bernoulli.py:50-95                                      */
+       TGP_LIK_GAUSS_WARPED = 3 };   /* likelihoods/WarpedGaussianLinearMean.py:25-168, the warped GP: z = G(y) = f + eps,
+                                      * eps ~ N(0, s2), G = model->layers applied to Y (global parameters only: a
+                                      * TGP_FLOW_PER_ROW layer is refused), the identity on f.  Training row (closed form,
+                                      * no quadrature): log N(G(y) | mu, s2) - v / (2 s2) + log|G'(y)|.  Test row:
+                                      * log N(G(y) | mu, v + s2) + log|G'(y)| - log y_std; moments E[G^-1(z)], Var[G^-1(z)]
+                                      * for z ~ N(mu, v + s2) by Gauss-Hermite (n_quad >= 1) and a Newton inverse per node.
+                                      * tgp_coverage_rows refuses it                                            */
 enum { TGP_FLOW_IDENTITY = 0,        /* models/flow.py:296-307                                              */
        TGP_FLOW_AFFINE = 1,          /* models/flow.py:330-340   params [a, b]                              */
        TGP_FLOW_TANH_STEP = 2,       /* models/flow.py:1096-1103 over :755-773   params n_steps x [a,b,c,d] */
@@ -151,6 +158,7 @@ int tgp_cov_sample(long R, int S, const void* mu, const void* L, long ldl, const
 /* Expected log-likelihood of R rows given (mu, v): flow o Gauss-Hermite o likelihood, with analytic gradients.
  * Replaces likelihood.expected_log_prob (GaussianNonLinearMean.py:113-150, GaussianLinearMean.py:60-87,
  * Bernoulli.py:50-95) and sparse_MF_SP.ELL's N/MB scaling (sparse_MF_SP.py:601-626; `scale` = N/MB_global).
+ * TGP_LIK_GAUSS_WARPED takes no quadrature (quad_t / quad_w may be NULL); dtheta is then the gradient w.r.t. the warp.
  * Outputs: ell_rows (R, unscaled), g_mu / g_v (R, scaled), drowparams (R, n_rowparams, scaled) and, ACCUMULATED
  * into the caller-zeroed reduce buffer: ell_sum (unscaled), dlogvar, dtheta (scaled).  want_grad = 0 skips grads. */
 int tgp_ell_forward(const TgpModel* model, const TgpParams* params, const void* mu, const void* v, const void* Y,
@@ -183,6 +191,13 @@ int tgp_qf_backward_dx(const TgpModel* model, const TgpParams* params, const voi
 int tgp_chain_backward(const TgpModel* model, const TgpParams* params, void* step_ws, const double* reduce_buf,
                        double gE, double gK, const double* g_dev, void* dZ, void* draw_lengthscale, void* draw_outputscale, void* dm,
                        void* dL_raw, void* dlog_var_noise, void* dtheta, void* stream);
+
+/* G^-1(z) elementwise for the global flow of `model->layers` (theta: n_theta device doubles), e.g. to map samples f + s eps of
+ * the warped likelihood to the units of y: out[i] = G^-1(z[i]) by a safeguarded Newton iteration (a bracket expanded from
+ * h = z[i], Newton steps that leave it or do not halve the step before last become bisections, |dh| <= 4 eps max(1, |h|), at most 200 steps), or NaN when the
+ * iteration finds no inverse — no bracket, no convergence, or a point where G' has the opposite sign of G'(z[i]) (G not
+ * monotone).  *n_fail (device int) += the number of NaNs.  No host synchronisation.  Per-row flows are refused. */
+int tgp_flow_inverse(const TgpModel* model, const void* theta, const void* z, long R, void* out, int* n_fail, void* stream);
 
 /* Posterior-predictive samples and 95 % interval coverage per row, from the marginals (mu, v) of the test-NLL pass — replaces
  * sample_from_predictive_distribution (sparse_MF_SP.py:886-992: S x the cost of q(f)) + numpy.quantile + the coverage count of
@@ -226,7 +241,8 @@ int tgp_reduce_pack(const TgpModel* model, const double* reduce_buf, double* pac
 int tgp_reduce_unpack(const TgpModel* model, const double* packed, double* reduce_buf, void* stream);
 
 /* Test log-likelihood rows and predictive moments given (mu, v) (sparse_MF_SP.py:637-825; marginal_moments of the
- * three likelihoods).  rowparams: (R, n_mc, n_rowparams) for MC-dropout flows, n_mc = 1 otherwise.
+ * likelihoods; TGP_LIK_GAUSS_WARPED: n_mc = 1 and NaN moments for a row whose inverse warp fails).
+ * rowparams: (R, n_mc, n_rowparams) for MC-dropout flows, n_mc = 1 otherwise.
  * bern_std: device scalar, batch-wide std of v (Bernoulli.py:120 defect, kept for parity). */
 int tgp_test_rows(const TgpModel* model, const TgpParams* params, const void* mu, const void* v, const void* Y,
                   const void* rowparams, long R, int n_mc, double y_std, const void* quad_t, const void* quad_w,

@@ -10,7 +10,7 @@ LIB_PATH = os.environ.get('TGP_B200_LIB', os.path.join(_HERE, 'libtgp_b200.so'))
 LIB_PATH = os.environ.get('TGP_B200_LIB', LIB_PATH)      # A/B builds of the same sources (scripts/, profiling)
 
 TGP_F64, TGP_F32, TGP_F64_I8 = 0, 1, 2
-LIK_GAUSS_LINEAR, LIK_GAUSS_NONLINEAR, LIK_BERNOULLI = 0, 1, 2
+LIK_GAUSS_LINEAR, LIK_GAUSS_NONLINEAR, LIK_BERNOULLI, LIK_GAUSS_WARPED = 0, 1, 2, 3
 FLOW_IDENTITY, FLOW_AFFINE, FLOW_TANH_STEP, FLOW_SAL, FLOW_ARCSINH, FLOW_BOXCOX, FLOW_INV_BOXCOX = 0, 1, 2, 3, 4, 5, 6
 FLOW_STEP_GROUP = 7
 KERNEL_RBF, KERNEL_MATERN12, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2, 3
@@ -88,6 +88,7 @@ SIGNATURES = {
                                 _P, _P]),
     'tgp_test_rows': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _I, _D, _P, _P, _P, _P, _P,
                            _P, _P]),
+    'tgp_flow_inverse': (_I, [C.POINTER(TgpModel), _P, _P, _L, _P, _P, _P]),
     'tgp_coverage_rows': (_I, [C.POINTER(TgpModel), C.POINTER(TgpParams), _P, _P, _P, _P, _L, _I, _I, C.c_ulonglong, _P, _D, _D, _P, _P,
                               _P, _P, _P, _P]),
     'tgp_mc_softmax_rows': (_I, [C.POINTER(TgpModel), _I, _I, _L, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P]),

@@ -75,11 +75,17 @@ inline int validate(const TgpModel* md) {
     if (md->n_layers < 0 || md->n_layers > TGP_MAX_LAYERS) return set_error(-1, "too many flow layers");
     if (md->n_theta < 0 || md->n_theta > MAX_THETA) return set_error(-1, "too many global flow parameters");
     if (md->n_rowparams < 0 || md->n_rowparams > MAX_ROWP) return set_error(-1, "too many per-row flow parameters");
-    if (md->likelihood < 0 || md->likelihood > 2) return set_error(-1, "unknown likelihood");
+    if (md->likelihood < 0 || md->likelihood > TGP_LIK_GAUSS_WARPED) return set_error(-1, "unknown likelihood");
     if (md->likelihood == TGP_LIK_GAUSS_LINEAR && md->n_layers != 0)
         return set_error(-1, "the closed-form Gaussian likelihood takes an identity flow");
     if (md->likelihood != TGP_LIK_GAUSS_LINEAR && (md->n_quad < 1 || md->n_quad > 4096))
         return set_error(-1, "n_quad out of range");
+    if (md->likelihood == TGP_LIK_GAUSS_WARPED) {
+        if (md->n_rowparams != 0) return set_error(-1, "the warped likelihood takes a warp with global parameters only");
+        for (int i = 0; i < md->n_layers; ++i)
+            if (md->layers[i].flags & TGP_FLOW_PER_ROW)
+                return set_error(-1, "input-dependent warps (TGP_FLOW_PER_ROW) are outside the warped likelihood");
+    }
     for (int i = 0, left = 0; i < md->n_layers; ++i) {          // step groups: header + exactly n_steps member layers
         const TgpFlowLayer& L = md->layers[i];
         if (L.kind < 0 || L.kind > TGP_FLOW_STEP_GROUP) return set_error(-1, "unknown flow layer kind");
@@ -287,7 +293,9 @@ int tgp_ell_forward(const TgpModel* md, const TgpParams* p, const void* mu, cons
     if (want_grad && (!g_mu || !g_v)) return set_error(-1, "g_mu / g_v required when want_grad");
     if (md->n_rowparams > 0 && (!rowparams || (want_grad && !drowparams)))
         return set_error(-1, "rowparams / drowparams required for input-dependent flows");
-    if (md->likelihood != TGP_LIK_GAUSS_LINEAR && (!quad_t || !quad_w)) return set_error(-1, "quadrature rule missing");
+    const bool warped = md->likelihood == TGP_LIK_GAUSS_WARPED;
+    if (md->likelihood != TGP_LIK_GAUSS_LINEAR && !warped && (!quad_t || !quad_w)) return set_error(-1, "quadrature rule missing");
+    if (warped && md->n_theta > 0 && !p->theta) return set_error(-1, "theta required for the warp");
     const TgpReduceLayout l = reduce_layout(md);
     RowQuadArgs a;
     a.R = (int)R; a.likelihood = md->likelihood; a.n_quad = md->n_quad; a.n_theta = md->n_theta;
@@ -300,6 +308,11 @@ int tgp_ell_forward(const TgpModel* md, const TgpParams* p, const void* mu, cons
     a.ell_sum = reduce_buf + l.ell_sum; a.dlogvar = reduce_buf + l.dlogvar; a.dtheta = reduce_buf + l.dtheta;
     a.drowp = (double*)drowparams;
     fill_flow(a.flow, md);
+    if (warped) {
+        const long blocks = cdiv(R, ROW_THREADS);
+        k_row_warped<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), ROW_THREADS, 0, (cudaStream_t)stream>>>(a);
+        return check_launch("k_row_warped");
+    }
     k_row_quad<<<row_grid(R), ROW_THREADS, 0, (cudaStream_t)stream>>>(a);
     return check_launch("k_row_quad");
 }
@@ -458,6 +471,9 @@ int tgp_test_rows(const TgpModel* md, const TgpParams* p, const void* mu, const 
     if (md->n_rowparams > 0 && !rowparams) return set_error(-1, "rowparams required for input-dependent flows");
     if (md->likelihood == TGP_LIK_BERNOULLI && md->n_layers > 0 && !bern_std)
         return set_error(-1, "bern_std required for Bernoulli with a non-identity flow");
+    const bool warped = md->likelihood == TGP_LIK_GAUSS_WARPED;
+    if (warped && (!quad_t || !quad_w)) return set_error(-1, "quadrature rule missing (the warped predictive moments use it)");
+    if (warped && n_mc != 1) return set_error(-1, "the warped likelihood takes n_mc = 1");
     RowTestArgs a;
     a.R = (int)R; a.likelihood = md->likelihood; a.n_quad = md->n_quad; a.n_rowp = md->n_rowparams; a.n_mc = n_mc;
     a.y_std = y_std;
@@ -467,8 +483,23 @@ int tgp_test_rows(const TgpModel* md, const TgpParams* p, const void* mu, const 
     a.qt = (const double*)quad_t; a.qw = (const double*)quad_w; a.bern_std = bern_std;
     a.logp_rows = (double*)logp_rows; a.m1 = (double*)m1; a.m2 = (double*)m2;
     fill_flow(a.flow, md);
-    k_row_test<<<row_grid(R), ROW_THREADS, 0, (cudaStream_t)stream>>>(a);
+    if (warped) k_row_test<true><<<row_grid(R), ROW_THREADS, 0, (cudaStream_t)stream>>>(a);
+    else k_row_test<false><<<row_grid(R), ROW_THREADS, 0, (cudaStream_t)stream>>>(a);
     return check_launch("k_row_test");
+}
+
+int tgp_flow_inverse(const TgpModel* md, const void* theta, const void* z, long R, void* out, int* n_fail, void* stream) {
+    TGP_TRY(validate(md));
+    for (int i = 0; i < md->n_layers; ++i)
+        if (md->layers[i].flags & TGP_FLOW_PER_ROW) return set_error(-1, "tgp_flow_inverse takes flows with global parameters only");
+    if (R <= 0) return 0;
+    if (!z || !out || !n_fail || (md->n_theta > 0 && !theta)) return set_error(-1, "NULL argument to tgp_flow_inverse");
+    FlowDesc fd;
+    fill_flow(fd, md);
+    const long blocks = cdiv(R, ROW_THREADS);
+    k_flow_inverse<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), ROW_THREADS, 0, (cudaStream_t)stream>>>(
+        fd, (const double*)theta, (const double*)z, R, (double*)out, n_fail);
+    return check_launch("k_flow_inverse");
 }
 
 int tgp_coverage_rows(const TgpModel* md, const TgpParams* p, const void* mu, const void* v, const void* Y, const void* rowparams,
@@ -477,6 +508,8 @@ int tgp_coverage_rows(const TgpModel* md, const TgpParams* p, const void* mu, co
     TGP_TRY(validate(md));
     if (R <= 0) return 0;
     if (md->likelihood == TGP_LIK_BERNOULLI) return set_error(-1, "coverage intervals are defined for the Gaussian likelihoods");
+    if (md->likelihood == TGP_LIK_GAUSS_WARPED)
+        return set_error(-1, "coverage intervals are not implemented for the warped likelihood (its samples need the inverse warp)");
     if (!p || !mu || !v || !Y || !q_lo || !q_hi || !covered || !p->log_var_noise) return set_error(-1, "NULL argument to tgp_coverage_rows");
     if (S < 2 || S > 128) return set_error(-1, "S must be in 2..128");
     if (n_mc != 1 && n_mc != S) return set_error(-1, "n_mc must be 1 or S");

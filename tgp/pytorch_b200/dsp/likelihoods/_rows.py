@@ -87,6 +87,19 @@ def test_rows(likelihood, n_quad, y, mu, v, log_var_noise, flow, X, y_std=1.0, n
                              None if bern_std is None else bern_std.double())
 
 
+def flow_inverse(flow, z):
+    """(G^-1(z) elementwise with NaN where the Newton inverse fails, number of failures) for a flow module with global parameters
+    (tgp_flow_inverse; forward only)."""
+    with torch.no_grad():
+        layout, theta, rowp = flow_pack(flow, None)
+        if rowp is not None or layout.n_rowparams:
+            raise NotImplementedError('the inverse flow takes global parameters only (input-dependent warps are out of scope)')
+        eng = row_engine('gauss_warped', 1, layout, z.device)
+        out, n_fail = eng.flow_inverse(None if theta is None else theta.detach().contiguous(),
+                                       z.detach().to(torch.float64).reshape(-1).contiguous())
+        return out.view(z.shape), int(n_fail.item())
+
+
 def coverage_rows(likelihood, n_quad, y, mu, v, log_var_noise, flow, X, S, n_mc=1, seed=0, want_samples=False):
     """S posterior-predictive samples per row, their 2.5 % / 97.5 % quantiles and the coverage indicator of y (forward only)."""
     with torch.no_grad():

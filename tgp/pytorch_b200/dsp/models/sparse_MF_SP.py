@@ -7,7 +7,8 @@ gathers parameters from the unchanged nn.Module tree and shapes the results like
 
 Scope of the fused path (anything else raises, nothing falls back to the CPU): whitened or non-whitened q(u), zero mean, (Scale)RBF-ARD or
 (Scale)Matern-ARD (nu = 1/2, 3/2, 5/2) kernel, FP64 (what the reference's main.py runs), flows made of affine / tanh-step / sinh-arcsinh
-layers (optionally input-dependent with MC-dropout MLPs).  Multi-output models loop over outputs.  Marginals are differentiable;
+layers (optionally input-dependent with MC-dropout MLPs).  The warped GP (`WarpedGaussianLinearMean`: a flow with global parameters
+on the observations) runs with identity flows on f.  Multi-output models loop over outputs.  Marginals are differentiable;
 the full covariance over a batch (`diagonal=False`) and the joint samples drawn from it are evaluation-only (no backward).
 """
 import numpy
@@ -23,15 +24,24 @@ from ..likelihoods.GaussianLinearMean import GaussianLinearMean
 from ..likelihoods.GaussianNonLinearMean import GaussianNonLinearMean
 from ..likelihoods.Bernoulli import Bernoulli
 from ..likelihoods.MulticlassCategorical import MulticlassCategorical
+from ..likelihoods.WarpedGaussianLinearMean import WarpedGaussianLinearMean
 from ..likelihoods import _rows
 from ..quadrature import GaussHermiteQuadrature1D
 from .config_models import get_init_params
 from .flow import instance_flow
 from .utils_models import return_mean, enable_eval_dropout
 
-_LIK_KIND = {GaussianLinearMean: 'gauss_linear', GaussianNonLinearMean: 'gauss_nonlinear', Bernoulli: 'bernoulli'}
+_LIK_KIND = {GaussianLinearMean: 'gauss_linear', GaussianNonLinearMean: 'gauss_nonlinear', Bernoulli: 'bernoulli',
+             WarpedGaussianLinearMean: 'gauss_warped'}
 _INV_SOFTPLUS_ONE = 0.5413248546129181       # softplus^-1(1): outputscale of a bare (unscaled) kernel
 _MATERN_KIND = {0.5: 'matern12', 1.5: 'matern32', 2.5: 'matern52'}
+
+
+def _check_inverse(m1):
+    """The warped likelihood's moments are NaN in the rows whose inverse warp did not converge: raise, naming how many."""
+    bad = int(torch.isnan(m1).sum())
+    if bad:
+        raise ValueError('the inverse warp G^-1 did not converge for %d of %d rows (is G monotone?)' % (bad, m1.numel()))
 
 
 class sparse_MF_SP(nn.Module):
@@ -53,7 +63,8 @@ class sparse_MF_SP(nn.Module):
         self.init_params = get_init_params(init_params)
         self._standard_sampler = None     # built on first use (the reference builds it eagerly, sparse_MF_SP.py:96-97)
         self.is_training = True
-        self.quad_points = likelihood.quad_points if isinstance(likelihood, GaussianNonLinearMean) else cg.quad_points
+        self.quad_points = likelihood.quad_points if isinstance(likelihood, (GaussianNonLinearMean, WarpedGaussianLinearMean)) \
+            else cg.quad_points
         self.quad = GaussHermiteQuadrature1D(self.quad_points)
 
         self.initialize_inducing(init_Z, add_noise_inducing)
@@ -174,6 +185,17 @@ class sparse_MF_SP(nn.Module):
             return None
         lv = lik.log_var_noise
         return lv[0 if lik.noise_is_shared else dy].reshape(1).to(torch.float64)
+
+    def _warp_pack(self, dy, X):
+        """(FlowLayout, theta) of the warp of output `dy` (WarpedGaussianLinearMean): refuses what the warped likelihood does
+        not cover — a flow on f as well, or an input-dependent warp."""
+        if self.G_matrix[dy].describe(X)[0]:
+            raise NotImplementedError('the warped likelihood takes identity flows on f (G_matrix); a warp combined with a flow '
+                                      'on f is out of scope')
+        layout, theta, rowp = _rows.flow_pack(self.likelihood.flow[dy], X)
+        if rowp is not None or layout.n_rowparams:
+            raise NotImplementedError('input-dependent warps are out of scope of the warped likelihood')
+        return layout, theta
 
     def _engine(self, dy, layout, device):
         kind = _LIK_KIND[type(self.likelihood)]
@@ -320,6 +342,8 @@ class sparse_MF_SP(nn.Module):
             Z, raw_ls, raw_os, m, L_raw = self._gp_params(dy)
             if kind == 'gauss_linear':
                 layout, theta, rowp = FlowLayout([]), None, None
+            elif kind == 'gauss_warped':
+                (layout, theta), rowp = self._warp_pack(dy, Xd), None
             else:
                 layout, theta, rowp = _rows.flow_pack(self.G_matrix[dy], Xd)
             eng = self._engine(dy, layout, Xd.device)
@@ -410,6 +434,16 @@ class sparse_MF_SP(nn.Module):
                     m1.append(a)
                     m2.append(b)
                 m1, m2 = torch.stack(m1), torch.stack(m2)
+            elif isinstance(lik, WarpedGaussianLinearMean):
+                m1, m2 = [], []
+                for dy in range(self.out_dim):
+                    self._warp_pack(dy, X[dy])
+                    _, a, b = _rows.test_rows('gauss_warped', self.quad_points, None, mean_q_f[dy, :, 0], cov_q_f[dy, :, 0],
+                                              self._noise(dy), lik.flow[dy], None)
+                    m1.append(a)
+                    m2.append(b)
+                m1, m2 = torch.stack(m1), torch.stack(m2)
+                _check_inverse(m1)
             elif isinstance(lik, Bernoulli):
                 if n_mc > 1:
                     P = torch.stack([lik.marginal_moments(mean_q_f.squeeze(2), cov_q_f.squeeze(2), self.G_matrix, X)
@@ -444,7 +478,7 @@ class sparse_MF_SP(nn.Module):
         lik = self.likelihood
         predictive_params = None
         with torch.no_grad():
-            if isinstance(lik, (GaussianNonLinearMean, GaussianLinearMean)):
+            if isinstance(lik, (GaussianNonLinearMean, GaussianLinearMean, WarpedGaussianLinearMean)):
                 kind = _LIK_KIND[type(lik)]
                 n_mc = S_MC_NNet if (self.fully_bayesian and kind == 'gauss_nonlinear') else 1
                 mean_q_f, cov_q_f = self.marginal_variational_qf_parameters(X_run, diagonal=True, is_duvenaud=False)
@@ -453,10 +487,13 @@ class sparse_MF_SP(nn.Module):
                 Y_std = Y_std.reshape(-1).to(torch.float64)
                 for dy in range(self.out_dim):
                     Xr = X_run[dy].repeat(n_mc, 1) if n_mc > 1 else X_run[dy]
+                    flow = None if kind == 'gauss_linear' else self.G_matrix[dy]
+                    if kind == 'gauss_warped':
+                        self._warp_pack(dy, Xr)
+                        flow, Xr = lik.flow[dy], None
                     rows, a, b = _rows.test_rows(kind, self.quad_points, Y[:, dy].to(torch.float64), mean_q_f[dy, :, 0],
-                                                 cov_q_f[dy, :, 0], self._noise(dy),
-                                                 None if kind == 'gauss_linear' else self.G_matrix[dy], Xr,
-                                                 y_std=float(Y_std[dy]), n_mc=n_mc)
+                                                 cov_q_f[dy, :, 0], self._noise(dy), flow, Xr, y_std=float(Y_std[dy]),
+                                                 n_mc=n_mc)
                     lp = rows.sum()
                     if kind == 'gauss_nonlinear' and n_mc == 1:
                         # the reference evaluates 0.5*MB*log(pi) entirely in float32 (sparse_MF_SP.py:776)
@@ -465,6 +502,8 @@ class sparse_MF_SP(nn.Module):
                     m1.append(a)
                     m2.append(b)
                 log_p_y = torch.stack(logp)
+                if kind == 'gauss_warped':
+                    _check_inverse(torch.stack(m1))
                 if return_moments:
                     predictive_params = [torch.stack(m1), torch.stack(m2)]
             elif isinstance(lik, (Bernoulli, MulticlassCategorical)):
@@ -496,6 +535,8 @@ class sparse_MF_SP(nn.Module):
         lik = self.likelihood
         if isinstance(lik, Bernoulli):
             raise NotImplementedError('interval coverage is defined for the Gaussian likelihoods (regression)')
+        if isinstance(lik, WarpedGaussianLinearMean):
+            raise NotImplementedError('evaluation_bundle (fused interval coverage) is not implemented for the warped likelihood')
         kind = _LIK_KIND[type(lik)]
         log_p_y, (m1, m2) = self.test_log_likelihood(X, Y, return_moments=True, Y_std=Y_std, S_MC_NNet=S_MC_NNet)
         X_run = self._rows3(X)

@@ -15,7 +15,7 @@ _KIND = {'identity': _lib.FLOW_IDENTITY, 'affine': _lib.FLOW_AFFINE, 'tanh_step'
          'step_group': _lib.FLOW_STEP_GROUP}
 _NPAR = {'affine': 2, 'sal': 2, 'arcsinh': 4, 'boxcox': 1, 'invboxcox': 1, 'step_group': 0}
 _LIK = {'gauss_linear': _lib.LIK_GAUSS_LINEAR, 'gauss_nonlinear': _lib.LIK_GAUSS_NONLINEAR,
-        'bernoulli': _lib.LIK_BERNOULLI}
+        'bernoulli': _lib.LIK_BERNOULLI, 'gauss_warped': _lib.LIK_GAUSS_WARPED}
 
 
 class FlowLayout:
@@ -351,6 +351,19 @@ class Engine:
                                           _ptr(self.qw), _ptr(bern_std), _ptr(logp), _ptr(m1), _ptr(m2), _stream(self.device)),
                    'tgp_test_rows')
         return logp, m1, m2
+
+    @_on_device
+    def flow_inverse(self, theta, z):
+        """(G^-1(z) elementwise, NaN where the Newton inverse fails; device int32 count of the failures) for the engine's
+        flow with global parameters theta (n_theta,).  Forward only."""
+        _chk(theta, 'theta', (self.flow.n_theta,))
+        R = z.numel()
+        _chk(z, 'z', (R,))
+        out = torch.empty(R, dtype=torch.float64, device=self.device)
+        n_fail = torch.zeros(1, dtype=torch.int32, device=self.device)
+        _lib.check(self.lib.tgp_flow_inverse(self.model, _ptr(theta) if self.flow.n_theta else None, _ptr(z), R, _ptr(out),
+                                             _ptr(n_fail), _stream(self.device)), 'tgp_flow_inverse')
+        return out, n_fail
 
     @_on_device
     def coverage_rows(self, mu, v, Y, rowparams, n_mc, S, seed=0, q=(0.025, 0.975), want_samples=False):
